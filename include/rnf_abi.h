@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 9
+#define RNF_ABI_VERSION 10
 
 /* error codes */
 #define RNF_OK 0
@@ -152,6 +152,17 @@ int64_t rnf_flow_inverse_scratch_floats(const rnf_flow* flow, int64_t N);
 int rnf_flow_inverse(rnf_flow* flow, const float* R_in_dev, int64_t N, const float* cond_dev, int64_t B,
                      const int32_t* feat_index_dev, int64_t rows_per_image, float* R_out_dev,
                      float* ldj_out_dev, float* scratch_dev, int mlp_mode, void* stream);
+
+/*
+ * log p and its tangential rotation gradient (eval.py:464-480 nll_grad; the Riemannian gradient of the forward direction), one
+ * launch, FP32 (csrc/flow_grad.cu, one warp per rotation).
+ *   R_in_dev [N,3,3]; cond/B/feat_index/rows_per_image as rnf_flow_forward; fisher_A_dev [B,9], fisher_c_dev [B] or both NULL
+ *   logp_out_dev [N] = ldj [+ sum(A_b * R') - c_b]; grad_out_dev [N,3,3] = R [g]x / 2 (the tangential part of d logp / dR)
+ * K != 64 and ablation layers (kinds RNF_LAYER_SMITH9 .. RNF_LAYER_RIGHT9) return RNF_ESHAPE.
+ */
+int rnf_flow_logprob_grad(rnf_flow* flow, const float* R_in_dev, int64_t N, const float* cond_dev, int64_t B,
+                          const int32_t* feat_index_dev, int64_t rows_per_image, const float* fisher_A_dev,
+                          const float* fisher_c_dev, float* logp_out_dev, float* grad_out_dev, void* stream);
 
 /*
  * Grid evaluation: the inner loops of eval.py:444-462 (gradient()) and agent.py:246-266 fused:

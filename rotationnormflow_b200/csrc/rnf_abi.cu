@@ -249,6 +249,35 @@ int rnf_flow_inverse(rnf_flow* f, const float* R_in, int64_t N, const float* con
   return run_rows(f, true, R_in, N, cond, B, feat_index, rows_per_image, R_out, ldj_out, scratch, mlp_mode, stream);
 }
 
+int rnf_flow_logprob_grad(rnf_flow* f, const float* R_in, int64_t N, const float* cond, int64_t B, const int32_t* feat_index,
+                          int64_t rows_per_image, const float* fisher_A, const float* fisher_c, float* logp_out, float* grad_out,
+                          void* stream) {
+  const char* who = "rnf_flow_logprob_grad";
+  if (!f) return fail(RNF_EINVAL, "%s: null handle", who);
+  if (N < 0) return fail(RNF_EINVAL, "%s: negative N", who);
+  if ((fisher_A == nullptr) != (fisher_c == nullptr)) return fail(RNF_EINVAL, "%s: fisher_A and fisher_c must be given together", who);
+  if (f->model.K != rnf::kK) return fail(RNF_ESHAPE, "%s: the kernel is built for segments=%d (got K=%d)", who, rnf::kK, f->model.K);
+  for (int i = 0; i < f->model.n_layers; ++i) {
+    const int k = f->layers_host[i].kind;
+    if (k != RNF_LAYER_MOBIUS && k != RNF_LAYER_AFFINE)
+      return fail(RNF_ESHAPE, "%s: layer %d is an ablation layer (kind %d), which has no rotation gradient here", who, i, k);
+  }
+  if (N == 0) return RNF_OK;
+  if (!R_in || !logp_out || !grad_out) return fail(RNF_EINVAL, "%s: null buffer", who);
+  const bool per_image = f->cond_floats > 0 || fisher_A != nullptr;
+  if (f->cond_floats > 0 && !cond) return fail(RNF_ESTATE, "%s: conditional flow needs the output of rnf_flow_condition", who);
+  if (per_image) {
+    if (B <= 0) return fail(RNF_EINVAL, "%s: B must be > 0 for a conditional flow or a Fisher base term", who);
+    if (!feat_index && rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
+    if (!feat_index && (N + rows_per_image - 1) / rows_per_image > B)
+      return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N, (long long)rows_per_image,
+                  (long long)B);
+  }
+  cudaError_t e = rnf::launch_flow_grad(f, R_in, N, cond, per_image ? feat_index : nullptr, per_image ? rows_per_image : 1, fisher_A,
+                                        fisher_c, logp_out, grad_out, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
 int64_t rnf_grid_partial_floats(int64_t G, int64_t B) {
   if (G <= 0 || B <= 0) return 0;
   const int64_t tpi = (G + 127) / 128;  // sized for the smaller (tensor-core) tile so either kernel fits

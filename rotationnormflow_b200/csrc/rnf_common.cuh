@@ -109,5 +109,8 @@ cudaError_t launch_healpix(int level, int64_t begin, int64_t end, float* out, cu
 cudaError_t launch_min_geodesic(const float* est, const float* gt, int64_t B, int64_t K, float* out, cudaStream_t st);
 cudaError_t launch_fisher_logprob(const float* A9, const float* c, const float* R, int64_t N, int64_t rows_per_image, float* out,
                                   cudaStream_t st);
+cudaError_t launch_flow_grad(const rnf_flow* f, const float* R_in, int64_t N, const float* cond, const int32_t* feat_index,
+                             int64_t rows_per_image, const float* fisher_A, const float* fisher_c, float* logp_out, float* grad_out,
+                             cudaStream_t st);
 constexpr int kV1Threads = 256;
 }  // namespace rnf

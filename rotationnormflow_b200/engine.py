@@ -486,6 +486,20 @@ class Program:
                                                       self._stream()))
         return R_out, ldj
 
+    def logprob_grad(self, R: torch.Tensor, cond, B: int, feat_index, rows_per_image: int, A9=None, c=None):
+        """(logp [N], G [N,3,3]) of the forward direction in one launch (rnf_flow_logprob_grad): logp = ldj [+ sum(A_b R') - c_b],
+        G = R [g]x / 2 the tangential gradient of logp with respect to R."""
+        N = R.shape[0]
+        logp = torch.empty((N,), device=self.device, dtype=torch.float32)
+        G = torch.empty((N, 3, 3), device=self.device, dtype=torch.float32)
+        if N == 0:
+            return logp, G
+        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.rnf_flow_logprob_grad(self.handle, vp(R), N, vp(cond), B, vp(feat_index), rows_per_image, vp(A9), vp(c),
+                                                       vp(logp), vp(G), self._stream()))
+        return logp, G
+
     def grid_logprob(self, grid: torch.Tensor, g_index0: int, offset, cond, B: int, fisher_A, fisher_c,
                      want_logp: bool, mode: str, gt: torch.Tensor | None = None):
         """-> (max [B], argmax [B], sumexp [B], logp [B,G] | None[, spread_num [B] when gt [B,K,3,3] is given])."""

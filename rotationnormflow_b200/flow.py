@@ -599,6 +599,71 @@ class Flow(_NoProgramState, nn.Module):
     def inverse(self, rotation, feature=None, draw=False, feature_index=None, mlp_mode=None):
         return self.forward(rotation, feature, True, draw, feature_index, mlp_mode)
 
+    # ---- the score d log p / dR of the forward direction (eval.py:464-480 nll_grad) as one call ---------------
+    def log_prob_grad(self, rotation, feature=None, feature_index=None, fisher_A=None):
+        """(logp [N], grad [N,3,3]): log p(R | image) = ldj [+ matrix-Fisher base term] and its tangential gradient R [g]x / 2 with
+        respect to R (what ``rotation.grad`` holds after ``logp.sum().backward()``, projected on the tangent space of SO(3)).
+
+        feature [B,F] one row per image (None for an unconditional flow); row -> image from ``feature_index`` [N], else image-major
+        with N % B == 0.  fisher_A [B,3,3] adds log p of MatrixFisherN(A_b) at the flow's output (utils/fisher.py:217-232).
+        One launch of csrc/flow_grad.cu; the outputs are plain tensors, not autograd graphs.  Flows with segments != 64 or
+        ConditionLU layers run autograd through the per-layer operators of train.py instead (same numbers)."""
+        from .fisher import fisher_constants
+        layers = list(self.layers)
+        ablation = [l.kind for l in layers if l.kind.split("_")[0] in engine.ABLATION_KINDS]
+        if ablation:
+            raise NotImplementedError(f"Flow.log_prob_grad: no rotation gradient for the ablation layers {sorted(set(ablation))}")
+        R = _check_rotation(rotation).detach()
+        N = R.shape[0]
+        dev = R.device
+        conditional = bool(self.condition)
+        if conditional:
+            if feature is None:
+                raise AssertionError("The input feature is needed in this module")
+            feature = feature.detach().to(dev, torch.float32)
+            if feature.dim() != 2:
+                raise ValueError(f"feature must be [B,F] with one row per image, got {tuple(feature.shape)}")
+            B = feature.shape[0]
+        else:
+            feature = None
+            B = fisher_A.shape[0] if fisher_A is not None else 1
+        idx, rpi = None, 1
+        if feature_index is not None:
+            idx = feature_index.to(dev, torch.int32).contiguous()
+            if idx.shape != (N,):
+                raise ValueError("feature_index must have one entry per rotation")
+        elif conditional or fisher_A is not None:
+            if B <= 0 or N % B != 0:
+                raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
+            rpi = N // B
+        A9 = c = None
+        if fisher_A is not None:
+            A9, c = fisher_constants(fisher_A.detach().to(dev))
+            if A9.shape[0] != B:
+                raise ValueError("fisher_A must have one 3x3 matrix per image")
+        if N == 0:
+            return R.new_empty((0,)), R.new_empty((0, 3, 3))
+        if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers):
+            return self._log_prob_grad_composed(R, feature, idx, rpi, A9, c)
+        prog = _program(self, layers, self._perm_rows(), self.feature_dim, dev)
+        cond = prog.condition(feature) if prog.cond_floats else None
+        return prog.logprob_grad(R, cond, B, idx, 0 if idx is not None else rpi, A9, c)
+
+    def _log_prob_grad_composed(self, R, feature, idx, rpi, A9, c):
+        """log_prob_grad by autograd through the differentiable per-layer operators (train.composed_run)."""
+        from . import train
+        N = R.shape[0]
+        img = idx.long() if idx is not None else torch.arange(N, device=R.device) // rpi
+        rows = feature[img] if feature is not None else None
+        with torch.enable_grad():
+            Rg = R.clone().requires_grad_(True)
+            Rout, logp = train.composed_run(list(self.layers), self._perm_rows(), Rg, rows, False)
+            if A9 is not None:
+                logp = logp + (A9[img].reshape(N, 3, 3) * Rout).sum(dim=(1, 2)) - c[img]
+            (G,) = torch.autograd.grad(logp.sum(), Rg)
+        H = R.transpose(1, 2) @ G                      # tangential part R (H - H^T) / 2, the convention of the fused kernel
+        return logp.detach(), R @ (H - H.transpose(1, 2)) / 2
+
     # ---- N1 (SURVEY.md 8f): the loops of eval.py:444-462 / agent.py:246-266 as one call -------------------
     def grid_log_prob(self, grid, feature=None, offset=None, fisher_A=None, return_logp=False, g_index0=0, mlp_mode=None,
                       gt_rotations=None):
