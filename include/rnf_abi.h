@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 10
+#define RNF_ABI_VERSION 11
 
 /* error codes */
 #define RNF_OK 0
@@ -163,6 +163,29 @@ int rnf_flow_inverse(rnf_flow* flow, const float* R_in_dev, int64_t N, const flo
 int rnf_flow_logprob_grad(rnf_flow* flow, const float* R_in_dev, int64_t N, const float* cond_dev, int64_t B,
                           const int32_t* feat_index_dev, int64_t rows_per_image, const float* fisher_A_dev,
                           const float* fisher_c_dev, float* logp_out_dev, float* grad_out_dev, void* stream);
+
+/*
+ * Training (agent.py:49-87: the gradient of a loss on log p with respect to everything log p depends on), FP32, one warp per row
+ * (csrc/flow_grad.cu).  Both calls read the FP32 Mobius images and the unconditional affine blocks from weights_dev, at the
+ * handle's offsets (the packed-image sections of the tensor-core kernels are not read); cond/B/feat_index/rows_per_image as
+ * rnf_flow_forward.  K != 64 and ablation layers return RNF_ESHAPE.
+ *   forward : R_out_dev [N,3,3], ldj_out_dev [N] of the forward direction.
+ *   backward: seeds G_Rout_dev [N,3,3] = dL/dR_out (NULL = 0) and g_ldj_dev [N] = dL/dldj (NULL = 1); writes
+ *             G_R_dev [N,3,3] = dL/dR_in, tangential (R [g]x / 2), and the training records to workspace_dev
+ *             (rnf_flow_train_workspace_floats(N) floats):
+ *               [n_mobius_layers][N][772]: (y, 1) [4], relu(h0), relu(h1), relu(h2), relu(h0 + h3) [4 x 64],
+ *                                          dL/dh0 (residual included), dL/dh1, dL/dh2, dL/dh3 [4 x 64], dL/d(fc_last out) [256]
+ *                                          (fc_last outputs in the packed order: component c at 4c .. 4c+3)
+ *               [n_affine_layers][N][16] : dL/dW of the forward 4x4 of the layer (per-image or unconditional block)
+ *             Layer order is the stack order; the weight gradients are GEMMs over rows of these records and the
+ *             log-det slot of an affine block (has_ldj) receives the sum of g_ldj over its rows.
+ */
+int64_t rnf_flow_train_workspace_floats(const rnf_flow* flow, int64_t N);
+int rnf_flow_train_forward(rnf_flow* flow, const float* weights_dev, const float* R_in_dev, int64_t N, const float* cond_dev, int64_t B,
+                           const int32_t* feat_index_dev, int64_t rows_per_image, float* R_out_dev, float* ldj_out_dev, void* stream);
+int rnf_flow_train_backward(rnf_flow* flow, const float* weights_dev, const float* R_in_dev, int64_t N, const float* cond_dev, int64_t B,
+                            const int32_t* feat_index_dev, int64_t rows_per_image, const float* G_Rout_dev, const float* g_ldj_dev,
+                            float* G_R_dev, float* workspace_dev, int64_t workspace_floats, void* stream);
 
 /*
  * Grid evaluation: the inner loops of eval.py:444-462 (gradient()) and agent.py:246-266 fused:

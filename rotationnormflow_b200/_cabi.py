@@ -11,7 +11,7 @@ import threading
 
 from . import build as _build
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 RNF_LAYER_MOBIUS = 0
 RNF_LAYER_AFFINE = 1
@@ -78,6 +78,9 @@ _SIGNATURES = {
     "rnf_flow_inverse_scratch_floats": (_I64, [_P, _I64]),
     "rnf_flow_inverse": (C.c_int, [_P, _P, _I64, _P, _I64, _P, _I64, _P, _P, _P, C.c_int, _P]),
     "rnf_flow_logprob_grad": (C.c_int, [_P, _P, _I64, _P, _I64, _P, _I64, _P, _P, _P, _P, _P]),
+    "rnf_flow_train_workspace_floats": (_I64, [_P, _I64]),
+    "rnf_flow_train_forward": (C.c_int, [_P, _P, _P, _I64, _P, _I64, _P, _I64, _P, _P, _P]),
+    "rnf_flow_train_backward": (C.c_int, [_P, _P, _P, _I64, _P, _I64, _P, _I64, _P, _P, _P, _P, _I64, _P]),
     "rnf_grid_partial_floats": (_I64, [_I64, _I64]),
     "rnf_grid_logprob": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I64, _P, _P, _P, _P, _P, _P, _P, C.c_int, _P]),
     "rnf_fisher_sample": (C.c_int, [_P, _I64, _I64, C.c_uint64, _P, _P]),

@@ -26,6 +26,12 @@
 //                        flow/rottrans.py:21); W is the forward block of the packed or per-image affine block.
 //           Finally G = gradient_from_tangent(R_0, g).
 // No global scratch, no host synchronisation, one launch: capturable in a CUDA graph.
+//
+// Training (flow_train_kernel, Flow.log_prob): the same layer functions with TRAIN = true.  Forward mode writes R' and ldj.  Backward
+// mode reruns the forward sweep with history and the reverse sweep seeded by the caller's dL/dR' and dL/dldj per row; it writes the
+// tangential dL/dR and, per (layer, row), a training record (kTws* below; dL/dW of the 4x4 for an affine layer).  The weights come
+// from a buffer passed per call, so a training step never re-packs on the host; the weight gradients are GEMMs over the records
+// (engine.TrainProgram.backward).
 #include "mobius_math.cuh"
 #include "rnf_common.cuh"
 
@@ -34,6 +40,14 @@ namespace rnf {
 namespace {
 
 constexpr int kWarpFloats = kH + 4 * kK;            // per-warp activation / gradient vector [64] + conditioner-output gradient [256]
+
+// Training record of one (Mobius layer, row), kTwsFloats floats, rows of a layer contiguous ([layer][row][kTwsFloats]):
+//   kTwsY    (y, 1)                                    input of fc_first's y columns and bias
+//   kTwsAct  relu(h0), relu(h1), relu(h2), relu(h0+h3)  inputs of layers.1, .3, .5 and fc_last
+//   kTwsGrad gh0 (residual included), gp1, gp2, gp3     gradients of the pre-activations h0 .. h3
+//   kTwsGout dL/d(fc_last output) [256]                 packed order (component c at 4c..4c+3)
+constexpr int kTwsY = 0, kTwsAct = 4, kTwsGrad = kTwsAct + 4 * kH, kTwsGout = kTwsGrad + 4 * kH;
+constexpr int kTwsFloats = kTwsGout + 4 * kK;       // 772
 
 struct GradArgs {
   const float* weights;
@@ -97,9 +111,11 @@ __device__ __forceinline__ void set_col(float R[9], int p, const float c[3]) {
 
 // One Mobius layer for the warp's rotation: recomputes the conditioner with the lane's pre-activations kept (units lane, lane+32),
 // the mixture, and -- if BWD -- applies the VJP to the tangent gradient g (at the layer's output) in place.
-template <bool BWD>
+// TRAIN (with BWD): the log-det terms are scaled by gl = dL/dldj of the row, and the row's record of the five linear layers goes
+// to tws (kTws* layout below): their inputs and the gradients of their pre-activations, from which the weight gradients are GEMMs.
+template <bool BWD, bool TRAIN = false>
 __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float* __restrict__ wbuf, const float* cimg, int p0,
-                                             float R[9], float& ldj, float g[3]) {
+                                             float R[9], float& ldj, float g[3], float gl = 1.0f, float* __restrict__ tws = nullptr) {
   const int lane = threadIdx.x & 31;
   const int p1 = (p0 + 1) % 3, p2 = (p0 + 2) % 3;
   float x[3], y[3], z[3], r[3], v[3];
@@ -124,6 +140,11 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
   __syncwarp();
   act[lane] = fmaxf(h0[0], 0.0f);
   act[lane + 32] = fmaxf(h0[1], 0.0f);
+  if (TRAIN) {
+    if (lane < 4) tws[kTwsY + lane] = lane < 3 ? sel3(lane, y[0], y[1], y[2]) : 1.0f;      // (y, 1): fc_first's weights and bias
+    tws[kTwsAct + lane] = act[lane];
+    tws[kTwsAct + lane + 32] = act[lane + 32];
+  }
   __syncwarp();
 #pragma unroll                                               // (static indices keep h1..h3 in registers)
   for (int l = 0; l < 3; ++l) {
@@ -141,6 +162,10 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
     __syncwarp();
     if (l < 2) { act[lane] = fmaxf(a0, 0.0f); act[lane + 32] = fmaxf(a1, 0.0f); }
     else { act[lane] = fmaxf(h0[0] + a0, 0.0f); act[lane + 32] = fmaxf(h0[1] + a1, 0.0f); }      // relu(x0 + x)
+    if (TRAIN) {
+      tws[kTwsAct + kH * (l + 1) + lane] = act[lane];
+      tws[kTwsAct + kH * (l + 1) + lane + 32] = act[lane + 32];
+    }
     __syncwarp();
   }
 
@@ -219,7 +244,7 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
     set_col(Rn, p0, nx);
     set_col(Rn, p2, nz);
   }
-  const float cG = sel3(p1, g[0], g[1], g[2]), cF = 1.0f / Fm;
+  const float cG = sel3(p1, g[0], g[1], g[2]), cF = gl / Fm;
   float sA[3] = {0.f, 0.f, 0.f}, sB[3] = {0.f, 0.f, 0.f};
   __syncwarp();
 #pragma unroll
@@ -244,6 +269,7 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
     go.z = fmaf(B, z[1], -A * x[1]);
     go.w = fmaf(B, z[2], -A * x[2]);
     reinterpret_cast<float4*>(gout)[lane + 32 * u] = go;
+    if (TRAIN) reinterpret_cast<float4*>(tws + kTwsGout)[lane + 32 * u] = go;
 #pragma unroll
     for (int i = 0; i < 3; ++i) { sA[i] = fmaf(A, o[u][1 + i], sA[i]); sB[i] = fmaf(B, o[u][1 + i], sB[i]); }
   }
@@ -292,6 +318,10 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
     __syncwarp();
     act[lane] = gp[0];
     act[lane + 32] = gp[1];
+    if (TRAIN) {                                               // gradient of the output of layers.{2l+1}: h_{l+1}
+      tws[kTwsGrad + kH * (l + 1) + lane] = gp[0];
+      tws[kTwsGrad + kH * (l + 1) + lane + 32] = gp[1];
+    }
     __syncwarp();
     const float* Wt = sW + kMobHid + l * kMobHidStride;        // Wt[k][j] = W[j][k]
     const float* hin0 = l == 2 ? h2 : (l == 1 ? h1 : h0);
@@ -310,6 +340,10 @@ __device__ __forceinline__ void mobius_layer(const float* __restrict__ sW, float
   }
   gh0[0] += gp[0];
   gh0[1] += gp[1];
+  if (TRAIN) {
+    tws[kTwsGrad + lane] = gh0[0];
+    tws[kTwsGrad + lane + 32] = gh0[1];
+  }
   // g_y = W0[:, :3]^T g_h0; the conditioner input y = R[:, p1] adds tangent_of(R, g_y e_p1^T)
   float gy[3] = {0.f, 0.f, 0.f};
 #pragma unroll
@@ -343,9 +377,11 @@ __device__ __forceinline__ void ET_mul(const float q[4], const float d[4], float
   o[2] = -q[3] * d[0] + q[2] * d[1] - q[1] * d[2] + q[0] * d[3];
 }
 
-// calculate_16 (flow/squeezetrans.py:33-38) forward, or its tangent VJP (quat_affine_bwd_kernel) with g_loglen = gL
-template <bool BWD>
-__device__ __forceinline__ void affine_layer(const float* __restrict__ W, bool has_ldj, float R[9], float& ldj, float g[3]) {
+// calculate_16 (flow/squeezetrans.py:33-38) forward, or its tangent VJP (quat_affine_bwd_kernel) with g_loglen = gL.
+// TRAIN (with BWD): gL is scaled by gl = dL/dldj of the row, and lane 0 writes dL/dW = dp q^T (16 floats) to dW.
+template <bool BWD, bool TRAIN = false>
+__device__ __forceinline__ void affine_layer(const float* __restrict__ W, bool has_ldj, float R[9], float& ldj, float g[3],
+                                             float gl = 1.0f, float* __restrict__ dW = nullptr) {
   float Wr[17];
 #pragma unroll
   for (int i = 0; i < 17; ++i) Wr[i] = __ldg(W + i);
@@ -363,9 +399,15 @@ __device__ __forceinline__ void affine_layer(const float* __restrict__ W, bool h
 #pragma unroll
   for (int a = 0; a < 4; ++a) ph[a] = p[a] / len;
   E_mul(ph, g, Eg);
-  const float gL = has_ldj ? -4.0f : 0.0f;                    // d ldj / d log|Wq| (rotation layers: no log-det)
+  const float gL = has_ldj ? -4.0f * gl : 0.0f;               // d ldj / d log|Wq| (rotation layers: no log-det)
 #pragma unroll
   for (int a = 0; a < 4; ++a) dp[a] = (2.0f * Eg[a] + gL * ph[a]) / len;
+  if (TRAIN && (threadIdx.x & 31) == 0) {
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+      for (int b = 0; b < 4; ++b) dW[4 * a + b] = dp[a] * q[b];
+  }
 #pragma unroll
   for (int b = 0; b < 4; ++b) Wt[b] = Wr[b] * dp[0] + Wr[4 + b] * dp[1] + Wr[8 + b] * dp[2] + Wr[12 + b] * dp[3];
   ET_mul(q, Wt, g);
@@ -469,6 +511,144 @@ __global__ void __launch_bounds__(512, 1) flow_grad_kernel(const GradArgs a) {
   }
 }
 
+// ---- training: log p's forward and the full backward (rotation, weight-image and per-image-constant gradients) -----------------
+struct TrainArgs {
+  const float* weights;                             // the packed FP32 image (same offsets as the handle's buffer)
+  const LayerDev* layers;
+  int n_layers;
+  int n_mobius_slots;
+  int n_mob_layers;                                 // Mobius / affine layers in the stack (index of the training records)
+  int n_aff_layers;
+  const float* R_in;
+  int64_t N;
+  const float* cond;
+  int64_t cond_stride;
+  const int32_t* feat_index;
+  int64_t rows_per_image;
+  float* R_out;                                     // forward mode
+  float* ldj_out;
+  const float* G_Rout;                              // backward mode: seeds (null: 0 / 1), outputs
+  const float* g_ldj;
+  float* G_R;
+  float* ws_mob;                                    // [n_mob_layers][N][kTwsFloats]
+  float* ws_aff;                                    // [n_aff_layers][N][16]
+  int64_t n_tiles;
+  int warp_floats;
+};
+
+// Forward mode (BWD = false): R_out, ldj.  Backward mode: the forward sweep with history, then the reverse sweep of flow_grad_kernel
+// seeded with g = tangent_of(R_L, G_Rout[n]) and g_ldj[n], writing G_R (tangential) and the training records of every layer.
+template <bool BWD>
+__global__ void __launch_bounds__(512, 1) flow_train_kernel(const TrainArgs a) {
+  extern __shared__ __align__(16) float smem[];
+  float* sW = smem;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int n_warps = blockDim.x >> 5;
+  float* wbuf = smem + kMobFloats + (size_t)warp * a.warp_floats;
+  float* hist = wbuf + kWarpFloats;                          // backward: R_0 .. R_L, 9 floats each
+  const int L = a.n_layers;
+
+  for (int64_t tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
+    const int64_t row = tile * n_warps + warp;
+    const bool valid = row < a.N;
+    float R[9] = {1.f, 0.f, 0.f, 0.f, 1.f, 0.f, 0.f, 0.f, 1.f};
+    int64_t img = 0;
+    if (valid) {
+#pragma unroll
+      for (int i = 0; i < 9; ++i) R[i] = __ldg(a.R_in + row * 9 + i);
+      img = a.feat_index != nullptr ? (int64_t)__ldg(a.feat_index + row) : row / a.rows_per_image;
+    }
+    const float* cond_img = a.cond != nullptr ? a.cond + img * a.cond_stride : nullptr;
+    float ldj = 0.0f;
+    float g[3] = {0.f, 0.f, 0.f};
+
+    // ---- forward sweep ----
+#pragma unroll 1
+    for (int li = 0; li < L; ++li) {
+      const LayerDev Ld = a.layers[li];
+      if (BWD && valid && lane < 9) hist[9 * li + lane] = R[lane];
+      if (Ld.kind == RNF_LAYER_MOBIUS) {
+        __syncthreads();
+        const float4* src = reinterpret_cast<const float4*>(a.weights + Ld.w_off);
+        float4* dst = reinterpret_cast<float4*>(sW);
+        for (int i = threadIdx.x; i < kMobFloats / 4; i += blockDim.x) dst[i] = __ldg(src + i);
+        __syncthreads();
+        if (valid) {
+          const float* cimg = (Ld.cond_slot >= 0 && cond_img != nullptr) ? cond_img + (int64_t)Ld.cond_slot * kH : nullptr;
+          mobius_layer<false>(sW, wbuf, cimg, Ld.perm, R, ldj, g);
+        }
+      } else if (valid) {
+        const float* W = Ld.cond_slot >= 0 ? cond_img + (int64_t)a.n_mobius_slots * kH + (int64_t)Ld.cond_slot * kAffFloats
+                                           : a.weights + Ld.w_off;
+        affine_layer<false>(W, Ld.has_ldj != 0, R, ldj, g);
+      }
+    }
+    if (!BWD) {
+      if (valid && lane == 0) {
+#pragma unroll
+        for (int i = 0; i < 9; ++i) a.R_out[row * 9 + i] = R[i];
+        a.ldj_out[row] = ldj;
+      }
+      __syncwarp();
+      continue;
+    }
+    float gl = 1.0f;
+    if (valid) {
+      if (a.G_Rout != nullptr) {
+        float G[9];
+#pragma unroll
+        for (int i = 0; i < 9; ++i) G[i] = __ldg(a.G_Rout + row * 9 + i);
+        tangent_of(R, G, g);
+      }
+      if (a.g_ldj != nullptr) gl = __ldg(a.g_ldj + row);
+    }
+
+    // ---- reverse sweep ----
+    int mi = a.n_mob_layers, ai = a.n_aff_layers;
+#pragma unroll 1
+    for (int li = L - 1; li >= 0; --li) {
+      const LayerDev Ld = a.layers[li];
+      __syncwarp();
+      float Rl[9];
+#pragma unroll
+      for (int i = 0; i < 9; ++i) Rl[i] = hist[9 * li + i];
+      float dummy = 0.0f;
+      if (Ld.kind == RNF_LAYER_MOBIUS) {
+        --mi;
+        __syncthreads();
+        const float4* src = reinterpret_cast<const float4*>(a.weights + Ld.w_off);
+        float4* dst = reinterpret_cast<float4*>(sW);
+        for (int i = threadIdx.x; i < kMobFloats / 4; i += blockDim.x) dst[i] = __ldg(src + i);
+        __syncthreads();
+        if (valid) {
+          const float* cimg = (Ld.cond_slot >= 0 && cond_img != nullptr) ? cond_img + (int64_t)Ld.cond_slot * kH : nullptr;
+          mobius_layer<true, true>(sW, wbuf, cimg, Ld.perm, Rl, dummy, g, gl, a.ws_mob + ((int64_t)mi * a.N + row) * kTwsFloats);
+        }
+      } else {
+        --ai;
+        if (valid) {
+          const float* W = Ld.cond_slot >= 0 ? cond_img + (int64_t)a.n_mobius_slots * kH + (int64_t)Ld.cond_slot * kAffFloats
+                                             : a.weights + Ld.w_off;
+          affine_layer<true, true>(W, Ld.has_ldj != 0, Rl, dummy, g, gl, a.ws_aff + ((int64_t)ai * a.N + row) * 16);
+        }
+      }
+    }
+
+    if (valid) {
+      __syncwarp();
+      float R0[9], G[9];
+#pragma unroll
+      for (int i = 0; i < 9; ++i) R0[i] = hist[i];
+      gradient_from_tangent(R0, g, G);
+      if (lane == 0) {
+#pragma unroll
+        for (int i = 0; i < 9; ++i) a.G_R[row * 9 + i] = G[i];
+      }
+    }
+    __syncwarp();
+  }
+}
+
 }  // namespace
 
 size_t flow_grad_smem_bytes(int n_layers, int warps) {
@@ -509,6 +689,62 @@ cudaError_t launch_flow_grad(const rnf_flow* f, const float* R_in, int64_t N, co
   a.warp_floats = (kWarpFloats + 9 * (L + 1) + 3) & ~3;
   const int64_t grid = a.n_tiles < f->sm_count ? a.n_tiles : f->sm_count;
   flow_grad_kernel<<<(unsigned)grid, 32 * warps, smem, st>>>(a);
+  return cudaGetLastError();
+}
+
+}  // namespace rnf
+
+namespace rnf {
+
+int64_t flow_train_workspace_floats(const rnf_flow* f, int64_t N) {
+  int64_t n_mob = 0, n_aff = 0;
+  for (int i = 0; i < f->model.n_layers; ++i) (f->layers_host[i].kind == RNF_LAYER_MOBIUS ? n_mob : n_aff) += 1;
+  return N * (n_mob * kTwsFloats + n_aff * 16);
+}
+
+cudaError_t launch_flow_train(const rnf_flow* f, bool backward, const float* weights, const float* R_in, int64_t N, const float* cond,
+                              const int32_t* feat_index, int64_t rows_per_image, float* R_out, float* ldj_out, const float* G_Rout,
+                              const float* g_ldj, float* G_R, float* workspace, cudaStream_t st) {
+  if (N <= 0) return cudaSuccess;
+  const int L = f->model.n_layers;
+  int n_mob = 0;
+  for (int i = 0; i < L; ++i) n_mob += f->layers_host[i].kind == RNF_LAYER_MOBIUS;
+  // the forward mode keeps no rotation history: its per-warp buffer is the activation / gradient vector alone
+  auto smem_bytes = [&](int warps) {
+    return backward ? flow_grad_smem_bytes(L, warps) : ((size_t)kMobFloats + (size_t)warps * kWarpFloats) * sizeof(float);
+  };
+  int warps = (int)((N + f->sm_count - 1) / f->sm_count);
+  warps = warps < 1 ? 1 : (warps > 16 ? 16 : warps);
+  while (warps > 1 && smem_bytes(warps) > 227 * 1024) --warps;
+  const size_t smem = smem_bytes(warps);
+  if (smem > 227 * 1024) return cudaErrorInvalidConfiguration;
+  TrainArgs a;
+  a.weights = weights;
+  a.layers = f->layers_dev;
+  a.n_layers = L;
+  a.n_mobius_slots = f->model.n_mobius_slots;
+  a.n_mob_layers = n_mob;
+  a.n_aff_layers = L - n_mob;
+  a.R_in = R_in;
+  a.N = N;
+  a.cond = f->cond_floats > 0 ? cond : nullptr;
+  a.cond_stride = f->cond_floats;
+  a.feat_index = feat_index;
+  a.rows_per_image = rows_per_image > 0 ? rows_per_image : 1;
+  a.R_out = R_out;
+  a.ldj_out = ldj_out;
+  a.G_Rout = G_Rout;
+  a.g_ldj = g_ldj;
+  a.G_R = G_R;
+  a.ws_mob = workspace;
+  a.ws_aff = workspace != nullptr ? workspace + N * (int64_t)n_mob * kTwsFloats : nullptr;
+  a.n_tiles = (N + warps - 1) / warps;
+  a.warp_floats = backward ? (kWarpFloats + 9 * (L + 1) + 3) & ~3 : kWarpFloats;
+  const int64_t grid = a.n_tiles < f->sm_count ? a.n_tiles : f->sm_count;
+  auto kern = backward ? flow_train_kernel<true> : flow_train_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  kern<<<(unsigned)grid, 32 * warps, smem, st>>>(a);
   return cudaGetLastError();
 }
 

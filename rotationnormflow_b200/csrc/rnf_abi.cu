@@ -278,6 +278,58 @@ int rnf_flow_logprob_grad(rnf_flow* f, const float* R_in, int64_t N, const float
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
 }
 
+// shared argument checks of the training entry points (those of rnf_flow_logprob_grad, plus the weights pointer)
+static int check_train_args(const rnf_flow* f, const char* who, const float* weights, const float* R_in, int64_t N, const float* cond,
+                            int64_t B, const int32_t* feat_index, int64_t rows_per_image) {
+  if (!f) return fail(RNF_EINVAL, "%s: null handle", who);
+  if (N < 0) return fail(RNF_EINVAL, "%s: negative N", who);
+  if (f->model.K != rnf::kK) return fail(RNF_ESHAPE, "%s: the kernel is built for segments=%d (got K=%d)", who, rnf::kK, f->model.K);
+  for (int i = 0; i < f->model.n_layers; ++i) {
+    const int k = f->layers_host[i].kind;
+    if (k != RNF_LAYER_MOBIUS && k != RNF_LAYER_AFFINE)
+      return fail(RNF_ESHAPE, "%s: layer %d is an ablation layer (kind %d), which has no gradient here", who, i, k);
+  }
+  if (N == 0) return RNF_OK;
+  if (!weights || !R_in) return fail(RNF_EINVAL, "%s: null buffer", who);
+  if (f->cond_floats > 0) {
+    if (!cond) return fail(RNF_ESTATE, "%s: conditional flow needs its per-image constants", who);
+    if (B <= 0) return fail(RNF_EINVAL, "%s: B must be > 0 for a conditional flow", who);
+    if (!feat_index && rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
+    if (!feat_index && (N + rows_per_image - 1) / rows_per_image > B)
+      return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N, (long long)rows_per_image,
+                  (long long)B);
+  }
+  return RNF_OK;
+}
+
+int64_t rnf_flow_train_workspace_floats(const rnf_flow* f, int64_t N) { return f && N > 0 ? rnf::flow_train_workspace_floats(f, N) : 0; }
+
+int rnf_flow_train_forward(rnf_flow* f, const float* weights_dev, const float* R_in, int64_t N, const float* cond, int64_t B,
+                           const int32_t* feat_index, int64_t rows_per_image, float* R_out, float* ldj_out, void* stream) {
+  const char* who = "rnf_flow_train_forward";
+  const int rc = check_train_args(f, who, weights_dev, R_in, N, cond, B, feat_index, rows_per_image);
+  if (rc != RNF_OK || N == 0) return rc;
+  if (!R_out || !ldj_out) return fail(RNF_EINVAL, "%s: null buffer", who);
+  const bool cnd = f->cond_floats > 0;
+  cudaError_t e = rnf::launch_flow_train(f, false, weights_dev, R_in, N, cond, cnd ? feat_index : nullptr, cnd ? rows_per_image : 1,
+                                         R_out, ldj_out, nullptr, nullptr, nullptr, nullptr, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+int rnf_flow_train_backward(rnf_flow* f, const float* weights_dev, const float* R_in, int64_t N, const float* cond, int64_t B,
+                            const int32_t* feat_index, int64_t rows_per_image, const float* G_Rout, const float* g_ldj, float* G_R,
+                            float* workspace, int64_t workspace_floats, void* stream) {
+  const char* who = "rnf_flow_train_backward";
+  const int rc = check_train_args(f, who, weights_dev, R_in, N, cond, B, feat_index, rows_per_image);
+  if (rc != RNF_OK || N == 0) return rc;
+  if (!G_R || !workspace) return fail(RNF_EINVAL, "%s: null buffer", who);
+  if (workspace_floats < rnf::flow_train_workspace_floats(f, N)) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  const bool cnd = f->cond_floats > 0;
+  cudaError_t e = rnf::launch_flow_train(f, true, weights_dev, R_in, N, cond, cnd ? feat_index : nullptr, cnd ? rows_per_image : 1,
+                                         nullptr, nullptr, G_Rout, g_ldj, G_R, workspace, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
 int64_t rnf_grid_partial_floats(int64_t G, int64_t B) {
   if (G <= 0 || B <= 0) return 0;
   const int64_t tpi = (G + 127) / 128;  // sized for the smaller (tensor-core) tile so either kernel fits

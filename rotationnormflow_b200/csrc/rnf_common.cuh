@@ -112,5 +112,9 @@ cudaError_t launch_fisher_logprob(const float* A9, const float* c, const float* 
 cudaError_t launch_flow_grad(const rnf_flow* f, const float* R_in, int64_t N, const float* cond, const int32_t* feat_index,
                              int64_t rows_per_image, const float* fisher_A, const float* fisher_c, float* logp_out, float* grad_out,
                              cudaStream_t st);
+int64_t flow_train_workspace_floats(const rnf_flow* f, int64_t N);
+cudaError_t launch_flow_train(const rnf_flow* f, bool backward, const float* weights, const float* R_in, int64_t N, const float* cond,
+                              const int32_t* feat_index, int64_t rows_per_image, float* R_out, float* ldj_out, const float* G_Rout,
+                              const float* g_ldj, float* G_R, float* workspace, cudaStream_t st);
 constexpr int kV1Threads = 256;
 }  // namespace rnf

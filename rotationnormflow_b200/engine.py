@@ -555,3 +555,228 @@ def dedup_rows(feature: torch.Tensor, cap: int):
         _cabi.check(lib.rnf_dedup_rows(C.c_void_p(feature.data_ptr()), N, F, C.c_void_p(idx.data_ptr()), C.c_void_p(first.data_ptr()), cap,
                                        C.c_void_p(count.data_ptr()), C.c_void_p(ws.data_ptr()), nbytes, st))
     return idx, first, count
+
+
+# ------------------------------------------------------------------------------------------------------
+# training path: the FP32 image and the per-image constants built by differentiable torch ops on the parameters' device
+# (csrc/flow_grad.cu, flow_train_kernel).  The kernel returns gradients with respect to this image and these constants; autograd
+# through the packing below carries them to the parameters, the features and the SVDs.
+# ------------------------------------------------------------------------------------------------------
+TRAIN_RECORD_FLOATS = 772                  # kTwsFloats in csrc/flow_grad.cu: training record of one (Mobius layer, row)
+TRAIN_WORKSPACE_BYTES = 512 << 20          # bound of the backward's training records; larger batches run in chunks of rows
+_PERM_CACHE: dict = {}
+
+
+def _last_layer_perm_on(device) -> torch.Tensor:
+    key = str(device)
+    if key not in _PERM_CACHE:
+        _PERM_CACHE[key] = torch.from_numpy(_last_layer_perm(K_SEGMENTS)).to(device)
+    return _PERM_CACHE[key]
+
+
+def mobius_images(conds: list) -> torch.Tensor:
+    """Conditioner tensors (conditioner_tensors) of Lm Mobius layers -> [Lm, MOB_FLOATS]: the images of pack_mobius, stacked."""
+    Lm = len(conds)
+    st = lambda k: torch.stack([c[k] for c in conds]).to(torch.float32)
+    W0 = st("fc_first.weight")
+    perm = _last_layer_perm_on(W0.device)
+    parts = [torch.cat([W0[:, :, :3], st("fc_first.bias")[:, :, None]], dim=2).reshape(Lm, 4 * HIDDEN)]
+    for j in (1, 3, 5):
+        parts += [st(f"layers.{j}.weight").transpose(1, 2).reshape(Lm, HIDDEN * HIDDEN), st(f"layers.{j}.bias")]
+    parts += [st("fc_last.weight")[:, perm].transpose(1, 2).reshape(Lm, -1), st("fc_last.bias")[:, perm]]
+    return torch.cat(parts, dim=1)
+
+
+def logabsdet4(W: torch.Tensor) -> torch.Tensor:
+    """log|det W| of [...,4,4] by the expansion in 2x2 minors, evaluated in float64 and rounded to float32 (as pack_affine_matrix).
+    Differentiable, batched, and free of the LU factorisation's pivoting and info checks."""
+    a = W.to(torch.float64)
+    e = [[a[..., i, j] for j in range(4)] for i in range(4)]
+    m = lambda r0, r1, c0, c1: e[r0][c0] * e[r1][c1] - e[r1][c0] * e[r0][c1]
+    det = (m(0, 1, 0, 1) * m(2, 3, 2, 3) - m(0, 1, 0, 2) * m(2, 3, 1, 3) + m(0, 1, 0, 3) * m(2, 3, 1, 2)
+           + m(0, 1, 1, 2) * m(2, 3, 0, 3) - m(0, 1, 1, 3) * m(2, 3, 0, 2) + m(0, 1, 2, 3) * m(2, 3, 0, 1))
+    return det.abs().log().to(torch.float32)
+
+
+def affine_blocks(layers: list) -> torch.Tensor:
+    """Unconditional affine layers -> [La, 17]: the forward block (W, log|det W|) of pack_affine_matrix; U^T V and 0 for rot_u."""
+    from . import train
+    Ws, has = [], []
+    for l in layers:
+        W, h = train._affine_matrix(l, None, False)
+        Ws.append(W.reshape(4, 4))
+        has.append(h)
+    W = torch.stack(Ws).to(torch.float32)
+    ld = logabsdet4(W)
+    if not all(has):
+        ld = torch.stack([x if h else torch.zeros_like(x) for x, h in zip(ld.unbind(0), has)])
+    return torch.cat([W.reshape(-1, 16), ld[:, None]], dim=1)
+
+
+def _conditioners_stacked(cts: list, x: torch.Tensor) -> torch.Tensor:
+    """conditioner_torch of S conditioners on the same per-image input x [B,Ni] -> [S,B,No], as batched GEMMs."""
+    sd = [conditioner_tensors(ct) for ct in cts]
+    st = lambda k: torch.stack([d[k] for d in sd])
+    h0 = torch.baddbmm(st("fc_first.bias")[:, None, :], x.expand(len(cts), -1, -1), st("fc_first.weight").transpose(1, 2))
+    h = h0
+    for j in (1, 3, 5):
+        h = torch.baddbmm(st(f"layers.{j}.bias")[:, None, :], torch.relu(h), st(f"layers.{j}.weight").transpose(1, 2))
+    return torch.baddbmm(st("fc_last.bias")[:, None, :], torch.relu(h0 + h), st("fc_last.weight").transpose(1, 2))
+
+
+def condition_torch(layers: list, feature: torch.Tensor) -> torch.Tensor:
+    """feature [B,F] -> [B, cond_floats]: the per-image constants rnf_flow_condition writes (+ the polar factor of ConditionRot),
+    differentiable.  Sections: W_f . feature per conditional Mobius slot; the forward block (W_b, log|det W_b|) per conditional affine
+    slot (U^T V and 0 for rot_c); zeros where the forward kernels read nothing (inverse blocks, first-layer scratch)."""
+    feat = feature.to(torch.float32)
+    B = feat.shape[0]
+    mob = [l for l in layers if l.kind == "mobius" and l.condition]
+    aff = [l for l in layers if l.kind in ("aff_c", "rot_c")]
+    parts = []
+    if mob:
+        Wf = torch.cat([conditioner_tensors(l.conditioner)["fc_first.weight"][:, 3:] for l in mob])     # [Lc*64, F]
+        parts.append(feat @ Wf.t())
+    if aff:
+        S = len(aff)
+        if len({l.kind for l in aff}) > 1:
+            raise NotImplementedError("mixing different families of conditional affine layers in one flow")
+        W = _conditioners_stacked([l.net for l in aff], feat).reshape(S, B, 4, 4) + torch.eye(4, device=feat.device)
+        if aff[0].kind == "rot_c":
+            U, _, V = torch.svd(W)                                  # flow/rottrans.py:43-46 (V, not V^T)
+            W = U.transpose(-1, -2) @ V
+            ld = W.new_zeros((S, B))
+        else:
+            ld = logabsdet4(W)
+        blk = torch.cat([W.reshape(S, B, 16), ld[..., None], W.new_zeros((S, B, AFF_FLOATS - 17))], dim=2)
+        parts += [blk.transpose(0, 1).reshape(B, S * AFF_FLOATS), feat.new_zeros((B, S * HIDDEN))]
+    return torch.cat(parts, dim=1)
+
+
+class TrainProgram:
+    """The training path's Program: packed once for a layer structure (kinds, perms, F, device) and reused whatever the weights are --
+    every call brings its own image (``image``) and per-image constants.  Holds what the gradient reductions need."""
+
+    def __init__(self, layers: list, perms: list, F: int, device: torch.device):
+        self.prog = Program([LayerSpec(l.kind, p, l) for l, p in zip(layers, perms)], F, device)
+        self.device = device
+        descs = self.prog.descs
+        self.mob_layers, mob_off, self.mob_cond = [], [], []
+        self.aff_u_layers, aff_u_off, self.aff_u, self.aff_c = [], [], [], []
+        self.aff_c_has_ldj = False
+        n_aff = 0
+        for i, l in enumerate(layers):
+            d = descs[i]
+            if d.kind == _cabi.RNF_LAYER_MOBIUS:
+                if d.cond_slot >= 0:
+                    self.mob_cond.append(len(self.mob_layers))
+                self.mob_layers.append(l)
+                mob_off.append(d.w_off)
+            elif d.kind == _cabi.RNF_LAYER_AFFINE:
+                if d.cond_slot >= 0:
+                    self.aff_c.append(n_aff)
+                    self.aff_c_has_ldj = bool(d.has_ldj)
+                else:
+                    self.aff_u.append(n_aff)
+                    self.aff_u_layers.append(l)
+                    aff_u_off.append(d.w_off)
+                n_aff += 1
+            else:
+                raise NotImplementedError(f"layer kind {l.kind!r} (ablation) has no differentiable path")
+        self.aff_u_has_ldj = [not l.kind.startswith("rot") for l in self.aff_u_layers]
+        self.n_mob, self.n_aff = len(self.mob_layers), n_aff
+        self.cond_floats = self.prog.cond_floats
+        self.n_mob_slots, self.n_aff_slots = self.prog.n_mob, self.prog.n_aff
+        idx = [torch.arange(o, o + MOB_FLOATS) for o in mob_off] + [torch.arange(o, o + 17) for o in aff_u_off]
+        self.image_index = torch.cat(idx).to(device) if idx else torch.zeros(0, dtype=torch.int64, device=device)
+        self.aff_c_t = torch.tensor(self.aff_c, dtype=torch.int64, device=device)
+        self.aff_u_t = torch.tensor(self.aff_u, dtype=torch.int64, device=device)
+        self.mob_cond_t = torch.tensor(self.mob_cond, dtype=torch.int64, device=device)
+        self.ldj_mask_u = torch.tensor(self.aff_u_has_ldj, dtype=torch.float32, device=device)
+
+    def images(self):
+        """(mob [Lm, MOB_FLOATS], aff [Lu, 17]): the FP32 image sections the kernels read, differentiable in the parameters."""
+        mob = mobius_images([conditioner_tensors(l.conditioner) for l in self.mob_layers]) if self.mob_layers else None
+        aff = affine_blocks(self.aff_u_layers) if self.aff_u_layers else None
+        return mob, aff
+
+    def weights(self, mob, aff) -> torch.Tensor:
+        """A fresh weight buffer with the image sections at the Program's offsets (the tensor-core sections are left unwritten:
+        the FP32 training kernels do not read them)."""
+        buf = torch.empty((int(self.prog.model.n_floats),), device=self.device, dtype=torch.float32)
+        src = [t.reshape(-1) for t in (mob, aff) if t is not None]
+        if src:
+            buf.index_copy_(0, self.image_index, torch.cat(src).detach())
+        return buf
+
+    def _call(self, name, *args):
+        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        with torch.cuda.device(self.device):
+            _cabi.check(getattr(self.prog.lib, name)(self.prog.handle, *[vp(a) if (a is None or torch.is_tensor(a)) else a for a in args],
+                                                     self.prog._stream()))
+
+    def forward(self, weights, R, cond, B: int, idx32):
+        N = R.shape[0]
+        R_out = torch.empty((N, 3, 3), device=self.device, dtype=torch.float32)
+        ldj = torch.empty((N,), device=self.device, dtype=torch.float32)
+        if N:
+            self._call("rnf_flow_train_forward", weights, R, N, cond, B, idx32, 0, R_out, ldj)
+        return R_out, ldj
+
+    def backward(self, weights, R, cond, B: int, idx32, G_Rout, g_ldj):
+        """-> (G_R [N,3,3] tangential, g_mob [Lm, MOB_FLOATS] | None, g_aff [Lu,17] | None, g_cond [B, cond_floats] | None).
+
+        The kernel writes per row the training records (rnf_abi.h); the weight gradients are FP32 GEMMs over rows batched across
+        layers, the per-image sums are index_add over rows.  Rows run in chunks so that the records stay within
+        TRAIN_WORKSPACE_BYTES; the sums accumulate across chunks."""
+        N, dev = R.shape[0], self.device
+        Lm, La, H = self.n_mob, self.n_aff, HIDDEN
+        TF = TRAIN_RECORD_FLOATS
+        G_R = torch.empty((N, 3, 3), device=dev, dtype=torch.float32)
+        g_mob = torch.zeros((Lm, MOB_FLOATS), device=dev, dtype=torch.float32) if Lm else None
+        g_aff = torch.zeros((len(self.aff_u), 17), device=dev, dtype=torch.float32) if self.aff_u else None
+        g_cmob = torch.zeros((B, len(self.mob_cond) * H), device=dev, dtype=torch.float32) if cond is not None and self.mob_cond else None
+        g_caff = torch.zeros((B, len(self.aff_c), 16), device=dev, dtype=torch.float32) if cond is not None and self.aff_c else None
+        img = idx32.long() if idx32 is not None else None
+        per_row = Lm * TF + La * 16
+        chunk = max(1, min(N, TRAIN_WORKSPACE_BYTES // (4 * max(per_row, 1))))
+        ws = torch.empty((max(1, chunk * per_row),), device=dev, dtype=torch.float32)
+        for s in range(0, N, chunk):
+            n = min(chunk, N - s)
+            sl = lambda t: None if t is None else t[s:s + n]
+            self._call("rnf_flow_train_backward", weights, R[s:s + n], n, cond, B, sl(idx32), 0, sl(G_Rout), sl(g_ldj), G_R[s:s + n],
+                       ws, int(ws.numel()))
+            wm = ws[:Lm * n * TF].view(Lm, n, TF)
+            wa = ws[Lm * n * TF: Lm * n * TF + La * n * 16].view(La, n, 16)
+            if Lm:
+                act = lambda i: wm[:, :, 4 + H * i: 4 + H * (i + 1)]
+                grad = lambda i: wm[:, :, 4 + 4 * H + H * i: 4 + 4 * H + H * (i + 1)]
+                gout = wm[:, :, 4 + 8 * H:]
+                bsum = wm[:, :, 4 + 5 * H:].sum(dim=1)                      # biases of layers.1/3/5 and fc_last
+                parts = [torch.bmm(grad(0).transpose(1, 2), wm[:, :, 0:4]).reshape(Lm, 4 * H)]
+                for i in range(3):
+                    parts += [torch.bmm(act(i).transpose(1, 2), grad(i + 1)).reshape(Lm, H * H), bsum[:, H * i: H * (i + 1)]]
+                parts += [torch.bmm(act(3).transpose(1, 2), gout).reshape(Lm, -1), bsum[:, 3 * H:]]
+                g_mob += torch.cat(parts, dim=1)
+                if g_cmob is not None:
+                    gh0 = grad(0) if len(self.mob_cond) == Lm else grad(0).index_select(0, self.mob_cond_t)
+                    g_cmob.index_add_(0, img[s:s + n], gh0.transpose(0, 1).reshape(n, -1))
+            if g_aff is not None:
+                g_aff[:, :16] += wa.index_select(0, self.aff_u_t).sum(dim=1)
+            if g_caff is not None:
+                g_caff.index_add_(0, img[s:s + n], wa.index_select(0, self.aff_c_t).transpose(0, 1))
+        # log-det slots: d ldj / d log|det W| = 1 on every row the block acts on
+        gl = g_ldj if g_ldj is not None else torch.ones((N,), device=dev, dtype=torch.float32)
+        if g_aff is not None:
+            g_aff[:, 16] = gl.sum() * self.ldj_mask_u
+        g_cond = None
+        if cond is not None:
+            parts = [] if g_cmob is None else [g_cmob]
+            if g_caff is not None:
+                Sc = len(self.aff_c)
+                ld = torch.zeros((B,), device=dev, dtype=torch.float32)
+                if self.aff_c_has_ldj:
+                    ld.index_add_(0, img, gl)
+                parts += [torch.cat([g_caff, ld[:, None, None].expand(B, Sc, 1), g_caff.new_zeros((B, Sc, AFF_FLOATS - 17))], dim=2).reshape(B, -1),
+                          g_caff.new_zeros((B, Sc * H))]
+            g_cond = torch.cat(parts, dim=1)
+        return G_R, g_mob, g_aff, g_cond

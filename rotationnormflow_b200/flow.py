@@ -38,10 +38,12 @@ class _NoProgramState:
     def invalidate_cache(self):
         """Forget the packed weights (needed only after writes that bypass autograd versioning, e.g. ``p.data.copy_()``)."""
         self.__dict__.pop("_rnf_programs", None)
+        self.__dict__.pop("_rnf_train_programs", None)
 
     def __getstate__(self):
         state = self.__dict__.copy()
         state.pop("_rnf_programs", None)
+        state.pop("_rnf_train_programs", None)
         return state
 
 
@@ -458,6 +460,18 @@ def _program(owner, layers, perms, F, device) -> engine.Program:
     return prog
 
 
+def _train_program(owner, layers, perms, F, device) -> engine.TrainProgram:
+    """The training path's program, cached on the owning module and keyed on structure only (device, layer modules and kinds, perms,
+    F): it is packed once, and every call brings the current weights as a device image, so optimiser steps cost no re-pack."""
+    cache = owner.__dict__.setdefault("_rnf_train_programs", {})
+    dev = device.index if device.index is not None else torch.cuda.current_device()
+    key = (dev, tuple(perms), tuple((id(l), l.kind) for l in layers), int(F))
+    tp = cache.get(key)
+    if tp is None:
+        tp = cache[key] = engine.TrainProgram(layers, perms, F, torch.device("cuda", dev))
+    return tp
+
+
 def _wants_grad(layers, rotation, feature) -> bool:
     if not torch.is_grad_enabled():
         return False
@@ -648,6 +662,67 @@ class Flow(_NoProgramState, nn.Module):
         prog = _program(self, layers, self._perm_rows(), self.feature_dim, dev)
         cond = prog.condition(feature) if prog.cond_floats else None
         return prog.logprob_grad(R, cond, B, idx, 0 if idx is not None else rpi, A9, c)
+
+    # ---- training: differentiable log p in the fused kernels (agent.py:49-87) ------------------------------------------------
+    def log_prob(self, rotation, feature=None, feature_index=None, fisher_A=None):
+        """log p(R | image) [N] = ldj [+ sum(A_b * R') - c_b with a matrix-Fisher base A_b], differentiable by autograd with respect to
+        every flow parameter, ``feature``, ``fisher_A`` and ``rotation`` (tangential gradient, as the per-layer operators give).
+
+        feature [B,F] one row per image (None for an unconditional flow); row -> image from ``feature_index`` [N], else image-major
+        with N % B == 0.  Forward and backward each run as one kernel launch over the whole stack (csrc/flow_grad.cu) plus batched
+        GEMMs for the weight gradients; the weights reach the kernels as a device-side image built by torch ops, so an optimiser step
+        costs no re-pack and nothing synchronises with the host.  Flows with segments != 64 or ConditionLU run train.composed_run
+        instead (same numbers); ablation layers raise NotImplementedError.
+
+        The loss of agent.py:54-73 (``rotation, ldjs = flow(gt, feature)``, then the Fisher log-prob of ``rotation``) becomes::
+
+            logp = flow.log_prob(gt, feature, feature_index=idx, fisher_A=A)     # A [B,3,3] or None (uniform base)
+            loss = -logp.mean()
+        """
+        from . import train
+        from .fisher import fisher_constants
+        layers = list(self.layers)
+        ablation = [l.kind for l in layers if l.kind.split("_")[0] in engine.ABLATION_KINDS]
+        if ablation:
+            raise NotImplementedError(f"Flow.log_prob: no differentiable path for the ablation layers {sorted(set(ablation))}")
+        R = _check_rotation(rotation)
+        N, dev = R.shape[0], R.device
+        conditional = bool(self.condition)
+        B = 1
+        if conditional:
+            if feature is None:
+                raise AssertionError("The input feature is needed in this module")
+            feature = feature.to(dev, torch.float32)
+            if feature.dim() != 2:
+                raise ValueError(f"feature must be [B,F] with one row per image, got {tuple(feature.shape)}")
+            B = feature.shape[0]
+        else:
+            feature = None
+            if fisher_A is not None:
+                B = fisher_A.shape[0]
+        idx = None
+        if feature_index is not None:
+            idx = feature_index.to(dev, torch.int32).contiguous()
+            if idx.shape != (N,):
+                raise ValueError("feature_index must have one entry per rotation")
+        elif conditional or fisher_A is not None:
+            if B <= 0 or N % B != 0:
+                raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
+            idx = torch.arange(N, device=dev, dtype=torch.int32) // (N // B)
+        perms = self._perm_rows()
+        if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers):
+            rows = feature[idx.long()] if feature is not None else None
+            R_out, logp = train.composed_run(layers, perms, R, rows, False)
+        else:
+            tp = _train_program(self, layers, perms, self.feature_dim, dev)
+            R_out, logp = train.fused_run(tp, layers, R, feature, idx if conditional else None, B)
+        if fisher_A is not None:
+            A9, c = fisher_constants(fisher_A.to(dev))
+            if A9.shape[0] != B:
+                raise ValueError("fisher_A must have one 3x3 matrix per image")
+            img = idx.long()
+            logp = logp + (A9[img].reshape(N, 3, 3) * R_out).sum(dim=(1, 2)) - c[img]
+        return logp
 
     def _log_prob_grad_composed(self, R, feature, idx, rpi, A9, c):
         """log_prob_grad by autograd through the differentiable per-layer operators (train.composed_run)."""

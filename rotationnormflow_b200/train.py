@@ -87,6 +87,38 @@ class QuatAffine(torch.autograd.Function):
         return G_R, G_W
 
 
+class FusedLogDensity(torch.autograd.Function):
+    """(R [N,3,3], Mobius images, unconditional affine blocks, per-image constants) -> (R' [N,3,3], ldj [N]) of the forward direction
+    in the fused training kernels (csrc/flow_grad.cu through rnf_flow_train_forward / rnf_flow_train_backward).  The gradients it
+    returns are with respect to the packed image and constants of engine.TrainProgram; autograd through the packing
+    (engine.mobius_images, engine.affine_blocks, engine.condition_torch) carries them to the parameters and the features."""
+
+    @staticmethod
+    def forward(ctx, tp, R, idx32, B: int, mob, aff, cond):
+        weights = tp.weights(mob, aff)
+        R_out, ldj = tp.forward(weights, R, cond, B, idx32)
+        ctx.tp, ctx.B, ctx.idx32, ctx.weights = tp, B, idx32, weights
+        ctx.save_for_backward(R, cond)
+        return R_out, ldj
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, G_Rout, g_ldj):
+        R, cond = ctx.saved_tensors
+        G_Rout = None if G_Rout is None else G_Rout.contiguous().float()
+        g_ldj = R.new_zeros(R.shape[0]) if g_ldj is None else g_ldj.contiguous().float()
+        G_R, g_mob, g_aff, g_cond = ctx.tp.backward(ctx.weights, R, cond, ctx.B, ctx.idx32, G_Rout, g_ldj)
+        return None, G_R, None, None, g_mob, g_aff, g_cond
+
+
+def fused_run(tp, layers, R, feature, idx32, B: int):
+    """(R', ldj) of the forward direction through FusedLogDensity; feature [B,F] one row per image (None if unconditional),
+    idx32 [N] row -> image."""
+    mob, aff = tp.images()
+    cond = engine.condition_torch(layers, feature) if tp.cond_floats else None
+    return FusedLogDensity.apply(tp, R, idx32, B, mob, aff, cond)
+
+
 def _affine_matrix(layer, rows, inverse: bool):
     """The 4x4 a layer applies in this direction ([1,4,4] or [N,4,4], differentiable torch algebra) and whether it has a log-det."""
     eye = None
