@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 11
+#define RNF_ABI_VERSION 12
 
 /* error codes */
 #define RNF_OK 0
@@ -275,6 +275,20 @@ int rnf_train_mobius_backward(const float* R_dev, const float* out_dev, int64_t 
 int rnf_train_affine_forward(const float* R_dev, const float* W_dev, int64_t N, float* R_out_dev, float* loglen_dev, void* stream);
 int rnf_train_affine_backward(const float* R_dev, const float* W_dev, int64_t N, const float* R_out_dev, const float* G_Rout_dev,
                               const float* g_loglen_dev, float* G_R_dev, float* G_W_dev, void* stream);
+
+/*
+ * Differentiable ablation layers (csrc/ablation_layers.cuh; flow/affineflow.py:27-41,55-70): the same per-row arithmetic as the fused
+ * kernels, forward and vector-Jacobian product, one rotation per thread, FP32.
+ *   kind : RNF_LAYER_SMITH9 .. RNF_LAYER_RIGHT9
+ *   M_dev: [N,n,n] (n = 6 for RNF_LAYER_SMITH36, else 3), the matrix the layer applies IN THIS DIRECTION, one per row: inv(M) of the
+ *          Smith layers and M^T of the SVD layers in the inverse direction, the Gram-Schmidt Q (or Q^T) of calculate_9_r_smith.
+ *   forward : R_out_dev [N,3,3], ldj_dev [N] (log|det| of the Smith layers by tangent propagation; 0 for the others)
+ *   backward: the saved R_dev, M_dev, R_out_dev and the incoming G_Rout_dev [N,3,3], g_ldj_dev [N]; writes the TANGENTIAL rotation
+ *             gradient G_R_dev [N,3,3] (R [g]x / 2) and G_M_dev [N,n,n] per row.
+ */
+int rnf_train_ablation_forward(const float* R_dev, const float* M_dev, int64_t N, int kind, float* R_out_dev, float* ldj_dev, void* stream);
+int rnf_train_ablation_backward(const float* R_dev, const float* M_dev, int64_t N, int kind, const float* R_out_dev, const float* G_Rout_dev,
+                                const float* g_ldj_dev, float* G_R_dev, float* G_M_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -11,7 +11,7 @@ import threading
 
 from . import build as _build
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 
 RNF_LAYER_MOBIUS = 0
 RNF_LAYER_AFFINE = 1
@@ -74,6 +74,8 @@ _SIGNATURES = {
     "rnf_train_mobius_backward": (C.c_int, [_P, _P, _I64, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P]),
     "rnf_train_affine_forward": (C.c_int, [_P, _P, _I64, _P, _P, _P]),
     "rnf_train_affine_backward": (C.c_int, [_P, _P, _I64, _P, _P, _P, _P, _P, _P]),
+    "rnf_train_ablation_forward": (C.c_int, [_P, _P, _I64, C.c_int, _P, _P, _P]),
+    "rnf_train_ablation_backward": (C.c_int, [_P, _P, _I64, C.c_int, _P, _P, _P, _P, _P, _P]),
     "rnf_flow_forward": (C.c_int, [_P, _P, _I64, _P, _I64, _P, _I64, _P, _P, C.c_int, _P]),
     "rnf_flow_inverse_scratch_floats": (_I64, [_P, _I64]),
     "rnf_flow_inverse": (C.c_int, [_P, _P, _I64, _P, _I64, _P, _I64, _P, _P, _P, C.c_int, _P]),

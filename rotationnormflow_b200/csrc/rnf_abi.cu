@@ -482,4 +482,30 @@ int rnf_train_affine_backward(const float* R, const float* W, int64_t N, const f
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, "rnf_train_affine_backward");
 }
 
+// argument checks before the device check, so that a bad call is reported as such on any host; N == 0 is a no-op (the buffers of
+// empty tensors may be null)
+static int ablation_args_ok(const char* who, int64_t N, int kind, bool null_buffer) {
+  if (N < 0) return fail(RNF_EINVAL, "%s: negative N", who);
+  if (kind < RNF_LAYER_SMITH9 || kind > RNF_LAYER_RIGHT9) return fail(RNF_EINVAL, "%s: kind %d is not an ablation layer (%d..%d)", who, kind,
+                                                                     RNF_LAYER_SMITH9, RNF_LAYER_RIGHT9);
+  if (N == 0) return RNF_OK;
+  if (null_buffer) return fail(RNF_EINVAL, "%s: null buffer", who);
+  return rnf_device_check(nullptr);
+}
+
+int rnf_train_ablation_forward(const float* R, const float* M, int64_t N, int kind, float* R_out, float* ldj, void* stream) {
+  int rc = ablation_args_ok("rnf_train_ablation_forward", N, kind, !R || !M || !R_out || !ldj);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_train_ablation_fwd(R, M, N, kind, R_out, ldj, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, "rnf_train_ablation_forward");
+}
+
+int rnf_train_ablation_backward(const float* R, const float* M, int64_t N, int kind, const float* R_out, const float* G_Rout, const float* g_ldj,
+                                float* G_R, float* G_M, void* stream) {
+  int rc = ablation_args_ok("rnf_train_ablation_backward", N, kind, !R || !M || !R_out || !G_Rout || !g_ldj || !G_R || !G_M);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_train_ablation_bwd(R, M, N, kind, R_out, G_Rout, g_ldj, G_R, G_M, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, "rnf_train_ablation_backward");
+}
+
 }  // extern "C"

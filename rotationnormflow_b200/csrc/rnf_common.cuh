@@ -104,6 +104,9 @@ cudaError_t launch_train_mobius_bwd(const float* R, const float* out, int64_t N,
 cudaError_t launch_train_affine_fwd(const float* R, const float* W, int64_t N, float* R_out, float* loglen, cudaStream_t st);
 cudaError_t launch_train_affine_bwd(const float* R, const float* W, int64_t N, const float* R_out, const float* G_Rout, const float* g_loglen,
                                     float* G_R, float* G_W, cudaStream_t st);
+cudaError_t launch_train_ablation_fwd(const float* R, const float* M, int64_t N, int kind, float* R_out, float* ldj, cudaStream_t st);
+cudaError_t launch_train_ablation_bwd(const float* R, const float* M, int64_t N, int kind, const float* R_out, const float* G_Rout,
+                                      const float* g_ldj, float* G_R, float* G_M, cudaStream_t st);
 int train_max_components();
 cudaError_t launch_healpix(int level, int64_t begin, int64_t end, float* out, cudaStream_t st);
 cudaError_t launch_min_geodesic(const float* est, const float* gt, int64_t B, int64_t K, float* out, cudaStream_t st);

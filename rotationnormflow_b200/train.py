@@ -6,7 +6,8 @@ The fused tcgen05 kernels of the inference path keep nothing for a backward pass
   * the conditioner MLP (flow/condition.py:24-30) as library GEMMs -- torch autograd supplies its backward, weight gradients included;
   * everything after it in hand-written CUDA operators with hand-written vector-Jacobian products (csrc/train_ops.cu through the C
     ABI ``rnf_train_*``): the Mobius mixture with its frame, log-det and, in the inverse direction, the 15-halving bisection and the
-    implicit-function gradient of BinFind.backward (flow/mobiusflow.py:248-273); and the quaternion affine map calculate_16.
+    implicit-function gradient of BinFind.backward (flow/mobiusflow.py:248-273); the quaternion affine map calculate_16; and the
+    ablation layers (36Trans, 9Trans*: csrc/ablation_layers.cuh) with their log-det.
 Rotation gradients are carried in the tangent space of SO(3) (see csrc/train_ops.cu): parameter and feature gradients equal the
 reference's; ``rotation.grad`` of the input is the tangential part of the reference's (the normal part of a gradient with respect to
 a rotation matrix has no meaning on the manifold)."""
@@ -87,6 +88,37 @@ class QuatAffine(torch.autograd.Function):
         return G_R, G_W
 
 
+class AblationLayer(torch.autograd.Function):
+    """(R [N,3,3], M [N,n,n], kind) -> (R', ldj) for one ablation layer (csrc/ablation_layers.cuh; rnf_train_ablation_*).  M is the
+    matrix the layer applies in this direction; ldj is the Smith layers' log-det by tangent propagation (0 for the others)."""
+
+    @staticmethod
+    def forward(ctx, R, M, kind: int):
+        lib = _cabi.load()
+        R, M = R.contiguous().float(), M.contiguous().float()
+        N = R.shape[0]
+        R_out, ldj = torch.empty_like(R), R.new_empty(N)
+        with torch.cuda.device(R.device):
+            _cabi.check(lib.rnf_train_ablation_forward(_ptr(R), _ptr(M), N, kind, _ptr(R_out), _ptr(ldj), _stream(R.device)))
+        ctx.save_for_backward(R, M, R_out)
+        ctx.kind = kind
+        return R_out, ldj
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, G_Rout, g_ldj):
+        R, M, R_out = ctx.saved_tensors
+        lib = _cabi.load()
+        N = R.shape[0]
+        G_Rout = torch.zeros_like(R) if G_Rout is None else G_Rout.contiguous().float()
+        g_ldj = R.new_zeros(N) if g_ldj is None else g_ldj.contiguous().float()
+        G_R, G_M = torch.empty_like(R), torch.empty_like(M)
+        with torch.cuda.device(R.device):
+            _cabi.check(lib.rnf_train_ablation_backward(_ptr(R), _ptr(M), N, ctx.kind, _ptr(R_out), _ptr(G_Rout), _ptr(g_ldj), _ptr(G_R),
+                                                        _ptr(G_M), _stream(R.device)))
+        return G_R, G_M, None
+
+
 class FusedLogDensity(torch.autograd.Function):
     """(R [N,3,3], Mobius images, unconditional affine blocks, per-image constants) -> (R' [N,3,3], ldj [N]) of the forward direction
     in the fused training kernels (csrc/flow_grad.cu through rnf_flow_train_forward / rnf_flow_train_backward).  The gradients it
@@ -135,12 +167,31 @@ def _affine_matrix(layer, rows, inverse: bool):
     elif kind == "rot_u":
         W = layer.rot
     else:
-        raise NotImplementedError(f"layer kind {kind!r} has no differentiable / general-segments path (ablation layers run in the fused kernels only)")
+        raise NotImplementedError(f"layer kind {kind!r} has no differentiable / general-segments path")
     if kind.startswith("rot"):
         U, _, V = torch.svd(W)                                # flow/rottrans.py:15-16 (note V, not V^T)
         W = U.transpose(-1, -2) @ V
         return (W.transpose(-1, -2) if inverse else W), False
     return (torch.linalg.inv(W) if inverse else W), True
+
+
+def _ablation_matrix(layer, base: str, rows, inverse: bool):
+    """The n x n matrix an ablation layer applies in this direction ([1,n,n] or [N,n,n], differentiable torch algebra), as
+    engine.ablation_blocks packs it for the fused kernels: inv(M) of the Smith layers and M^T of the SVD layers in the inverse
+    direction, the Gram-Schmidt Q (Q^T inverse) of calculate_9_r_smith."""
+    if layer.kind.endswith("_c"):
+        n = layer.n
+        M = engine.conditioner_torch(layer.net, rows).reshape(-1, n, n) + torch.eye(n, device=rows.device, dtype=rows.dtype)
+    elif isinstance(layer.mat, torch.nn.Module):
+        M = layer.mat()                                       # Uncondition9TransLU: UnconditionLU.forward, [1,3,3]
+    else:
+        M = layer.mat.unsqueeze(0)
+    if base in ("smith9", "smith36"):
+        return torch.linalg.inv(M) if inverse else M
+    if base in ("polar9l", "polar9r"):
+        return M.transpose(-1, -2) if inverse else M
+    Q = engine.gram_schmidt_columns(M)
+    return Q.transpose(-1, -2) if inverse else Q
 
 
 def composed_run(layers, perms, rotation, feature_rows, inverse: bool):
@@ -156,6 +207,10 @@ def composed_run(layers, perms, rotation, feature_rows, inverse: bool):
             inp = torch.cat((y, feature_rows), dim=-1) if layer.condition else y          # flow/mobiusflow.py:52-56
             out = engine.conditioner_torch(layer.conditioner, inp)
             R, ldj = MobiusMixture.apply(R, out, p0, inverse, layer.K)
+        elif layer.kind.split("_")[0] in engine.ABLATION_KINDS:
+            base = layer.kind.split("_")[0]
+            M = _ablation_matrix(layer, base, feature_rows, inverse)
+            R, ldj = AblationLayer.apply(R, M.expand(N, M.shape[-2], M.shape[-1]), engine.ABLATION_KINDS[base])
         else:
             W, has_ldj = _affine_matrix(layer, feature_rows, inverse)
             R, loglen = QuatAffine.apply(R, W.expand(N, 4, 4))
