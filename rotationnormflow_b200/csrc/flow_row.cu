@@ -81,10 +81,11 @@ __device__ __forceinline__ void store_a32(uint8_t* a_hi, uint8_t* a_lo, int r, i
     for (int e = 0; e < 4; ++e) {
 #if RNF_ROW_SPLIT_PACKED
       // as in flow_t4.cu: truncation by mask + packed subtract (5 instructions per pair instead of 6 with two conversions back and
-      // two scalar subtracts); this kernel runs at the per-warp issue cadence, so an instruction less is time less
+      // two scalar subtracts); this kernel runs at the per-warp issue cadence, so an instruction less is time less.  The masked
+      // value converts exactly up to 65504 and to +Inf from 65536 on: overflow is loud, as in flow_t4.cu relu_split_pair.
       const float x0 = v[8 * c + 2 * e], x1 = v[8 * c + 2 * e + 1];
-      asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi[e]) : "f"(x1), "f"(x0));
       const float m0 = __uint_as_float(__float_as_uint(x0) & 0xFFFFE000u), m1 = __uint_as_float(__float_as_uint(x1) & 0xFFFFE000u);
+      asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(hi[e]) : "f"(m1), "f"(m0));
       float d0, d1;
       upk(sub2(pk(x0, x1), pk(m0, m1)), d0, d1);
       asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo[e]) : "f"(d1), "f"(d0));
@@ -575,7 +576,7 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
       for (int o = 16; o > 0; o >>= 1) {
         const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
         const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+        if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
       }
       if (lane == 0) { s_v[w4] = bv; s_i[w4] = bi; }
       named_bar(3 + tile, 128);
@@ -584,10 +585,10 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
       for (int w = 1; w < 4; ++w) {
         const float ov = s_v[w];
         const long long oi = s_i[w];
-        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+        if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
       }
       const float m = bv;
-      float e = (valid && m > -INFINITY) ? expf(lp - m) : 0.0f;
+      float e = (valid && m != -INFINITY) ? expf(lp - m) : 0.0f;
       float ed = e * dgt;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {

@@ -173,11 +173,12 @@ __device__ __forceinline__ void relu_split_pair(float x0, float x1, uint32_t& hi
 #elif RNF_T4_SPLIT_MASK
   // The fp16 truncation of x, back in fp32, is x with its low 13 mantissa bits cleared: two LOP3 on the (half idle) ALU pipe
   // instead of two HADD2.F32 on the FMA pipe, which is the busiest pipe of this kernel (tools/pipe_rate.cu: every one of these
-  // instructions costs 2 cycles per warp on its pipe).  Differs from the converted-back value only where fp16 is subnormal
-  // (x < 6.1e-5: the sum hi + lo is then off by < 6e-8 absolute) and above the fp16 range (x > 65504 saturates at 65504
-  // instead of 2 x 65504); negative x: hi = 0 and x - (x & mask) <= 0 -> lo = 0.
-  asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(x1), "f"(x0));
+  // instructions costs 2 cycles per warp on its pipe).  hi is that masked value converted exactly (cvt.rn without satfinite),
+  // so hi + lo = x to 22 bits for 0.125 <= x < 65536 and to 2^-25 absolute below; x >= 65536 gives hi = +Inf, which the next
+  // GEMM turns into Inf / NaN rows instead of a silently clipped activation (tests/test_weight_scales.py).  Negative x:
+  // hi = 0 (relu) and x - (x & mask) <= 0 -> lo = 0.
   const float m0 = __uint_as_float(__float_as_uint(x0) & 0xFFFFE000u), m1 = __uint_as_float(__float_as_uint(x1) & 0xFFFFE000u);
+  asm("cvt.rn.relu.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(m1), "f"(m0));
   float d0, d1;
   upk(sub2(pk(x0, x1), pk(m0, m1)), d0, d1);
   asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(d1), "f"(d0));
@@ -674,7 +675,7 @@ __global__ void __launch_bounds__(kThreads, 1) flow_t4_kernel(const FlowArgs a) 
         for (int o = 16; o > 0; o >>= 1) {
           const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
           const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-          if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+          if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
         }
         if (lane == 0) { s_v[w4] = bv; s_i[w4] = bi; }
         named_bar(bar_red, 128);
@@ -683,10 +684,10 @@ __global__ void __launch_bounds__(kThreads, 1) flow_t4_kernel(const FlowArgs a) 
         for (int w = 1; w < 4; ++w) {
           const float ov = s_v[w];
           const long long oi = s_i[w];
-          if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+          if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
         }
         const float m = bv;
-        float e = (valid && m > -INFINITY) ? expf(lp - m) : 0.0f;
+        float e = (valid && m != -INFINITY) ? expf(lp - m) : 0.0f;
         float ed = e * dgt;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {

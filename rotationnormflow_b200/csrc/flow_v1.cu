@@ -275,7 +275,7 @@ __global__ void __launch_bounds__(T, 1) flow_v1_kernel(const FlowArgs a) {
       for (int o = 16; o > 0; o >>= 1) {
         const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
         const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-        if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+        if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
       }
       __syncthreads();
       if ((tid & 31) == 0) { s_red_v[tid >> 5] = bv; s_red_i[tid >> 5] = bi; }
@@ -287,14 +287,14 @@ __global__ void __launch_bounds__(T, 1) flow_v1_kernel(const FlowArgs a) {
         for (int o = 16; o > 0; o >>= 1) {
           const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
           const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-          if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+          if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
         }
         if (tid == 0) { s_bcast = bv; s_red_i[0] = bi; }
       }
       __syncthreads();
       const float m = s_bcast;
       const long long mi = s_red_i[0];
-      float e = (valid && m > -INFINITY) ? expf(lp - m) : 0.0f;
+      float e = (valid && m != -INFINITY) ? expf(lp - m) : 0.0f;
       float ed = e * dgt;
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) {
@@ -334,13 +334,13 @@ __global__ void grid_combine_kernel(const float* __restrict__ part, int64_t tile
   for (int64_t t = tid; t < tiles_per_image; t += blockDim.x) {
     const float v = p[t * kPartStride];
     const long long i = ((long long)(unsigned)__float_as_int(p[t * kPartStride + 2])) | ((long long)__float_as_int(p[t * kPartStride + 3]) << 32);
-    if (v > bv || (v == bv && i < bi)) { bv = v; bi = i; }
+    if (grid_red_better(v, i, bv, bi)) { bv = v; bi = i; }
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
     const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
     const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+    if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
   }
   if ((tid & 31) == 0) { s_v[tid >> 5] = bv; s_i[tid >> 5] = bi; }
   __syncthreads();
@@ -352,7 +352,7 @@ __global__ void grid_combine_kernel(const float* __restrict__ part, int64_t tile
     for (int o = 16; o > 0; o >>= 1) {
       const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
       const long long oi = __shfl_xor_sync(0xffffffffu, bi, o);
-      if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
+      if (grid_red_better(ov, oi, bv, bi)) { bv = ov; bi = oi; }
     }
     if (tid == 0) { s_m = bv; s_i[0] = bi; }
   }
@@ -361,7 +361,7 @@ __global__ void grid_combine_kernel(const float* __restrict__ part, int64_t tile
   float s = 0.0f, sd = 0.0f;
   for (int64_t t = tid; t < tiles_per_image; t += blockDim.x) {
     const float v = p[t * kPartStride];
-    if (v > -INFINITY) {
+    if (v != -INFINITY) {                 // a NaN tile maximum makes the sum NaN
       const float w = expf(v - m);
       s += p[t * kPartStride + 1] * w;
       sd += p[t * kPartStride + 4] * w;

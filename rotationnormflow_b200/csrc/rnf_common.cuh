@@ -87,6 +87,13 @@ struct rnf_flow {
 
 // kernel launchers (defined in the .cu files)
 namespace rnf {
+// Order of the grid reductions (max, first arg-max): a NaN log-density ranks above every number, ties and NaN against NaN go
+// to the lower index, so an image with a non-finite row gets a NaN max / sumexp and the index of its first such row instead
+// of a finite result taken over the remaining rows.
+__device__ __forceinline__ bool grid_red_better(float ov, long long oi, float bv, long long bi) {
+  const bool on = ov != ov, bn = bv != bv;
+  return on ? (!bn || oi < bi) : (!bn && (ov > bv || (ov == bv && oi < bi)));
+}
 cudaError_t launch_flow_v1(const FlowArgs& a, bool inverse, int sm_count, cudaStream_t st);
 cudaError_t launch_fisher_sample(const float* usv, int64_t B, int64_t n, unsigned long long seed, float* out, cudaStream_t st);
 cudaError_t launch_grid_combine(const float* part, int64_t tiles_per_image, int64_t B, int64_t g_index0, float* max_out,

@@ -199,8 +199,10 @@ __device__ __forceinline__ bool elect_one_sync() {
 //   hi = cvt.rz.relu.satfinite(t)          (round toward zero: the residual of a non-negative t is non-negative)
 //   lo = cvt.rn.relu.satfinite(t - hi)     (t < 0: hi = 0, residual = t < 0 -> 0)
 // so the ReLU of flow/condition.py:14-20 costs nothing, at one bit of the 22-bit split (hi 11 bits by truncation + lo 11).
-// Returns packed half2 words {x0 in the low half, x1 in the high half}; satfinite keeps huge activations finite
-// (fp16 range: |activation| < 65504, twice that through hi + lo).
+// Returns packed half2 words {x0 in the low half, x1 in the high half}.  Range (tests/test_weight_scales.py emulates it):
+// hi + lo = x to 22 bits only for x < 65536; above, hi saturates at 65504 and lo = x - 65504 keeps 11 bits (relative error up
+// to 2^-12.5), and from 131024 on lo saturates too: finite and clipped, never Inf.  The kernels compile the mask variants
+// (flow_t4.cu relu_split_pair, flow_row.cu store_a32) instead, which turn x >= 65536 into +Inf.
 __device__ __forceinline__ void relu_split2(float x0, float x1, uint32_t& hi, uint32_t& lo) {
   asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(x1), "f"(x0));
   const float2 back = __half22float2(*reinterpret_cast<const __half2*>(&hi));
