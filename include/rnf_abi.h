@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 12
+#define RNF_ABI_VERSION 13
 
 /* error codes */
 #define RNF_OK 0
@@ -289,6 +289,25 @@ int rnf_train_affine_backward(const float* R_dev, const float* W_dev, int64_t N,
 int rnf_train_ablation_forward(const float* R_dev, const float* M_dev, int64_t N, int kind, float* R_out_dev, float* ldj_dev, void* stream);
 int rnf_train_ablation_backward(const float* R_dev, const float* M_dev, int64_t N, int kind, const float* R_out_dev, const float* G_Rout_dev,
                                 const float* g_ldj_dev, float* G_R_dev, float* G_M_dev, void* stream);
+
+/*
+ * Separated posterior modes of a grid log-density (csrc/modes.cu; DESIGN 4.7): per image, M rounds of greedy non-maximum
+ * suppression on SO(3).  Round m takes the best point not yet labelled (NaN first, then larger value, then lower index: the order
+ * of the grid arg-max), reports whether it is a local maximum (no point within neighbour_radius is higher) and labels every
+ * unlabelled point closer than min_separation with m.  Angles are tested on quaternions of the fp32 matrices:
+ * angle < theta <=> |q_g . q_c| > cos(theta / 2), angle <= rho <=> |q_g . q_c| >= cos(rho / 2).
+ *   values_dev [B,G] float32 (e.g. the logp of rnf_grid_logprob); rot_dev [G,3,3] any rotation set (the geodesic angle is
+ *   right-invariant, so the grid without its offset gives the same labels); 1 <= M <= 256; 0 < neighbour_radius <= min_separation <= pi
+ *   workspace_dev  rnf_rotation_modes_workspace_bytes(G, B, M) bytes
+ *   index_out_dev [B,M] int64 global index (g_index0 + local), value_out_dev [B,M], local_max_out_dev [B,M] (0/1),
+ *   mass_out_dev [B,M] = sum over the mode's points of exp(v - v_mode0) / sum over all points of the same, count_out_dev [B] int32.
+ *   Entries at or after count are padding: index -1, value -inf, local_max 0, mass 0.  B == 0 does nothing; G == 0 writes padding.
+ * 2M + 3 launches, no atomics, no host synchronisation: bitwise reproducible and CUDA-graph capturable.
+ */
+int64_t rnf_rotation_modes_workspace_bytes(int64_t G, int64_t B, int M);
+int rnf_rotation_modes(const float* values_dev, int64_t B, int64_t G, int64_t g_index0, const float* rot_dev, int M, float min_separation,
+                       float neighbour_radius, void* workspace_dev, int64_t workspace_bytes, int64_t* index_out_dev, float* value_out_dev,
+                       uint8_t* local_max_out_dev, float* mass_out_dev, int32_t* count_out_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -35,6 +35,11 @@ cudaError_t launch_flow_row(const FlowArgs& a, bool inverse, int sm_count, cudaS
 cudaError_t launch_flow_t4(const FlowArgs& a, int sm_count, cudaStream_t st);
 bool flow_tc_supported(const rnf_flow* f);
 int pick_active_tiles(int64_t n_tiles, int sm_count);
+int64_t modes_workspace_bytes(int64_t G, int64_t B);
+int64_t modes_slices(int64_t G);
+cudaError_t launch_rotation_modes(const float* values, int64_t B, int64_t G, int64_t g_index0, const float* rot, int M, float cos_sep,
+                                  float cos_nb, void* workspace, int64_t* index_out, float* value_out, unsigned char* local_max_out,
+                                  float* mass_out, int32_t* count_out, cudaStream_t st);
 }  // namespace rnf
 
 extern "C" {
@@ -506,6 +511,37 @@ int rnf_train_ablation_backward(const float* R, const float* M, int64_t N, int k
   if (rc != RNF_OK) return rc;
   cudaError_t e = rnf::launch_train_ablation_bwd(R, M, N, kind, R_out, G_Rout, g_ldj, G_R, G_M, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, "rnf_train_ablation_backward");
+}
+
+int64_t rnf_rotation_modes_workspace_bytes(int64_t G, int64_t B, int M) {
+  if (G < 0 || B <= 0 || M < 1) return 0;
+  return rnf::modes_workspace_bytes(G, B);
+}
+
+int rnf_rotation_modes(const float* values, int64_t B, int64_t G, int64_t g_index0, const float* rot, int M, float min_separation,
+                       float neighbour_radius, void* workspace, int64_t workspace_bytes, int64_t* index_out, float* value_out,
+                       uint8_t* local_max_out, float* mass_out, int32_t* count_out, void* stream) {
+  // argument checks before the device check, so that a bad call is reported as such on any host; B == 0 is a no-op and G == 0 reads
+  // no input (the buffers of empty tensors may be null)
+  const char* who = "rnf_rotation_modes";
+  if (B < 0 || G < 0) return fail(RNF_EINVAL, "%s: negative size", who);
+  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
+  const float pi = 3.14159265358979323846f;
+  if (!(neighbour_radius > 0.f) || !(neighbour_radius <= min_separation) || !(min_separation <= pi))
+    return fail(RNF_EINVAL, "%s: need 0 < neighbour_radius <= min_separation <= pi (got %g, %g)", who, (double)neighbour_radius,
+                (double)min_separation);
+  if (rnf::modes_slices(G) > 65535) return fail(RNF_EINVAL, "%s: G=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G);
+  if (B == 0) return RNF_OK;
+  if (!workspace || !index_out || !value_out || !local_max_out || !mass_out || !count_out || (G > 0 && (!values || !rot)))
+    return fail(RNF_EINVAL, "%s: null pointer", who);
+  if (workspace_bytes < rnf_rotation_modes_workspace_bytes(G, B, M)) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  const int rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  // the thresholds in double, rounded once: |q_g . q_c| > cos(theta / 2) and >= cos(rho / 2)
+  const float cos_sep = (float)cos(0.5 * (double)min_separation), cos_nb = (float)cos(0.5 * (double)neighbour_radius);
+  cudaError_t e = rnf::launch_rotation_modes(values, B, G, g_index0, rot, M, cos_sep, cos_nb, workspace, index_out, value_out, local_max_out,
+                                             mass_out, count_out, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
 }
 
 }  // extern "C"

@@ -3,15 +3,27 @@
     estimate_rotation_grid      eval.py:437-462  (gradient(): grid log-pdf + arg-max per image)
     estimate_rotation_sampling  agent.py:238-266 (eval_acc: inverse-flow samples + arg-max per image), uniform base
     refine_rotation             eval.py:464-480  (nll_grad: Adam on a quaternion per row, climbing log p; one fused launch per step)
+    estimate_rotation_modes     (no reference counterpart) the M best separated modes per image from one grid pass, optionally refined
 
 Both avoid the reference's `feature.repeat` (4 GB per 500 000-row chunk at F = 2080, eval.py:450) and its per-image
 Python loop; all per-rotation arithmetic runs in the fused kernels.
 """
 from __future__ import annotations
 
+import math
+
 import torch
 
 from . import grid as rgrid
+from .modes import rotation_modes
+
+# Default neighbour_radius of estimate_rotation_modes per grid level: 1.5x the largest nearest-neighbour angle of the level-l HEALPix
+# grid, measured once on the CPU by tools/grid_spacing.py (DESIGN 4.7).  From level 2 on the measured angle halves exactly per level
+# (pi / 12 at level 2), so levels past 5 continue the halving.
+NEIGHBOUR_RADIUS = (1.570796, 0.778990, 0.392699, 0.196350, 0.098175, 0.049087)
+# estimate_rotation_modes evaluates the grid in image chunks whose [chunk, G] float32 log-density stays under this many bytes
+# (a level-6 grid is 151 MB per image)
+MODES_LOGP_BYTES = 1 << 30
 
 
 def _random_rotation(device, generator=None):
@@ -42,6 +54,93 @@ def estimate_rotation_grid(flow, feature, number_queries, fisher_A=None, offset=
             raise ValueError("refine_steps > 0 needs refine_lr")
         est, out["refined_logp"] = refine_rotation(flow, feature, est, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
     return est, out
+
+
+@torch.no_grad()
+def default_neighbour_radius(level: int) -> float:
+    """1.5x the largest nearest-neighbour angle (radians) of the level-``level`` HEALPix grid (NEIGHBOUR_RADIUS)."""
+    if level < len(NEIGHBOUR_RADIUS):
+        return NEIGHBOUR_RADIUS[level]
+    return NEIGHBOUR_RADIUS[-1] / 2 ** (level - len(NEIGHBOUR_RADIUS) + 1)
+
+
+@torch.no_grad()
+def estimate_rotation_modes(flow, feature, number_queries, num_modes, *, min_separation, neighbour_radius=None, fisher_A=None, offset=None,
+                            generator=None, mlp_mode=None, refine_steps=0, refine_lr=None):
+    """The ``num_modes`` best separated posterior modes per image from one grid pass (the grid and offset of
+    ``estimate_rotation_grid``): ``modes.rotation_modes`` on the grid log-density with angles ``min_separation`` and
+    ``neighbour_radius`` (default ``default_neighbour_radius(level)``; radians), keeping the local maxima only.
+
+    refine_steps > 0 runs one ``refine_rotation`` (lr = refine_lr) on all [B,M] modes at once, then merges refined modes closer than
+    ``neighbour_radius`` greedily by refined log p (the masses of merged modes add up).
+
+    Returns (rotations [B,M,3,3], dict(logp [B,M], mass [B,M], valid [B,M] bool, count [B], grid_index [B,M] int64, max [B], argmax [B],
+    sumexp [B])): modes sorted by log p (the refined one after refinement), valid ones first; padded entries have NaN rotations, logp
+    -inf, mass 0 and grid_index -1.  ``max`` / ``argmax`` / ``sumexp`` are those of ``Flow.grid_log_prob``; mode 0 of the grid pass is
+    its arg-max.  The grid is evaluated in image chunks of at most MODES_LOGP_BYTES of log-density."""
+    level = rgrid.closest_grid_level(number_queries)
+    rho = default_neighbour_radius(level) if neighbour_radius is None else float(neighbour_radius)
+    if float(min_separation) < rho:
+        raise ValueError(f"min_separation={min_separation} is below neighbour_radius={rho}: a mode's neighbourhood would reach past its "
+                         "own ball")
+    if refine_steps > 0 and refine_lr is None:
+        raise ValueError("refine_steps > 0 needs refine_lr")
+    dev = feature.device if feature is not None else torch.device("cuda", torch.cuda.current_device())
+    grid = rgrid.get_closest_available_grid(number_queries, dev)
+    if offset is None:
+        offset = _random_rotation(dev, generator)
+    offset = offset.to(dev, torch.float32)
+    G, M = grid.shape[0], int(num_modes)
+    B = feature.shape[0] if (feature is not None and flow.condition) else 1
+    chunk = max(1, MODES_LOGP_BYTES // (G * 4))
+    parts = []
+    for s in range(0, B, chunk):
+        f = feature[s:s + chunk] if (feature is not None and flow.condition) else feature
+        A = fisher_A[s:s + chunk] if fisher_A is not None else None
+        out = flow.grid_log_prob(grid, f, offset=offset, fisher_A=A, return_logp=True, mlp_mode=mlp_mode)
+        md = rotation_modes(out.pop("logp"), grid, M, min_separation, rho)
+        parts.append((out, md))
+    out = {k: torch.cat([p[0][k] for p in parts]) for k in ("max", "argmax", "sumexp")}
+    md = {k: torch.cat([p[1][k] for p in parts]) for k in ("index", "value", "local_max", "mass")}
+    # drop the shoulders, keeping the greedy order (non-increasing value) of the local maxima
+    valid = md["local_max"]
+    order = torch.sort((~valid).to(torch.int8), dim=1, stable=True).indices
+    valid = torch.gather(valid, 1, order)
+    index = torch.where(valid, torch.gather(md["index"], 1, order), -1)
+    logp = torch.where(valid, torch.gather(md["value"], 1, order), -math.inf)
+    mass = torch.where(valid, torch.gather(md["mass"], 1, order), 0.0)
+    rot = grid[index.clamp(min=0)] @ offset
+    if refine_steps > 0:
+        seeds = torch.where(valid[..., None, None], rot, (grid[md["index"][:, 0]] @ offset)[:, None])   # padding: mode 0 of the grid
+        rot, lp = refine_rotation(flow, feature, seeds, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
+        rot, logp, mass, valid, index = _merge_modes(rot, torch.where(valid, lp, -math.inf), mass, valid, index, rho)
+    rot = torch.where(valid[..., None, None], rot, math.nan)
+    out.update(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)
+    return rot, out
+
+
+def _merge_modes(rot, logp, mass, valid, index, radius):
+    """Greedy merge of refined modes by log p: a mode within ``radius`` of a better one that is kept adds its mass to the best such
+    one and is dropped.  Returns the kept modes first, sorted by log p, padded as estimate_rotation_modes pads."""
+    B, M = logp.shape
+    order = torch.sort(logp, dim=1, descending=True, stable=True).indices
+    rot = torch.gather(rot, 1, order[..., None, None].expand(B, M, 3, 3))
+    logp, mass, valid, index = (torch.gather(t, 1, order) for t in (logp, mass, valid, index))
+    q = matrix_to_quaternion(rot)
+    close = (q @ q.transpose(1, 2)).abs() >= math.cos(radius / 2)            # [B,M,M], angle <= radius
+    kept = torch.zeros_like(valid)
+    target = torch.arange(M, device=rot.device).expand(B, M).clone()
+    for i in range(M):
+        near = close[:, i, :i] & kept[:, :i]
+        merged = near.any(1)
+        kept[:, i] = valid[:, i] & ~merged
+        if i > 0:
+            target[:, i] = torch.where(valid[:, i] & merged, near.to(torch.int8).argmax(1), i)
+    mass = torch.zeros_like(mass).scatter_add_(1, target, torch.where(valid, mass, 0.0))
+    order = torch.sort((~kept).to(torch.int8), dim=1, stable=True).indices
+    rot = torch.gather(rot, 1, order[..., None, None].expand(B, M, 3, 3))
+    logp, mass, kept, index = (torch.gather(t, 1, order) for t in (logp, mass, kept, index))
+    return rot, torch.where(kept, logp, -math.inf), torch.where(kept, mass, 0.0), kept, torch.where(kept, index, -1)
 
 
 @torch.no_grad()
