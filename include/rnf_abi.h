@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 13
+#define RNF_ABI_VERSION 14
 
 /* error codes */
 #define RNF_OK 0
@@ -308,6 +308,31 @@ int64_t rnf_rotation_modes_workspace_bytes(int64_t G, int64_t B, int M);
 int rnf_rotation_modes(const float* values_dev, int64_t B, int64_t G, int64_t g_index0, const float* rot_dev, int M, float min_separation,
                        float neighbour_radius, void* workspace_dev, int64_t workspace_bytes, int64_t* index_out_dev, float* value_out_dev,
                        uint8_t* local_max_out_dev, float* mass_out_dev, int32_t* count_out_dev, void* stream);
+
+/*
+ * The same modes over a grid split across ranks (csrc/modes.cu; DESIGN 4.7 "Sharded"): rank k holds values [B,G_r] and rotations
+ * [G_r,3,3] of the contiguous global slice [g_index0, g_index0 + G_r); every rank ends with the outputs rnf_rotation_modes gives on
+ * the whole [B,G] (index, value, local_max, count bit for bit; mass up to the order of its sums).  Per rank:
+ *   rnf_rotation_modes_shard_setup  once (quaternions of the slice), then for r = 0 .. M:
+ *     rnf_rotation_modes_shard_round  writes this rank's record of round r, record_out_dev [B] x RNF_MODES_RECORD_BYTES;
+ *     the caller all-gathers the records of the W ranks, rank-major, to records_dev [W][B] x RNF_MODES_RECORD_BYTES;
+ *     rnf_rotation_modes_shard_merge  folds them in rank order and writes mode r-1's mass / local_max and mode r's index / value /
+ *                                     rotation (rot_out_dev [B,M,3,3], the owning rank's matrix; padding NaN) and count_out_dev.
+ *   workspace_dev  rnf_rotation_modes_shard_workspace_bytes(G_r, B) bytes, the same buffer for every call of one rank (the merged
+ *                  state lives in it); record buffers 16-byte aligned.
+ * Argument rules as rnf_rotation_modes, plus 0 <= r <= M, g_index0 >= 0, W >= 1.  B == 0 does nothing; G_r == 0 (an empty slice) reads
+ * no input: setup does nothing and the round writes this rank's empty records, so the rank still takes part in every gather.
+ * 2 launches per round and 1 per merge, no atomics, no host synchronisation: bitwise reproducible and CUDA-graph capturable.
+ */
+#define RNF_MODES_RECORD_BYTES 80
+int64_t rnf_rotation_modes_shard_workspace_bytes(int64_t G_r, int64_t B);
+int rnf_rotation_modes_shard_setup(const float* rot_dev, int64_t G_r, int64_t B, void* workspace_dev, int64_t workspace_bytes, void* stream);
+int rnf_rotation_modes_shard_round(const float* values_dev, int64_t B, int64_t G_r, int64_t g_index0, const float* rot_dev, int r, int M,
+                                   float min_separation, float neighbour_radius, void* workspace_dev, int64_t workspace_bytes,
+                                   void* record_out_dev, void* stream);
+int rnf_rotation_modes_shard_merge(const void* records_dev, int W, int64_t B, int r, int M, void* workspace_dev, int64_t workspace_bytes,
+                                   int64_t* index_out_dev, float* value_out_dev, uint8_t* local_max_out_dev, float* mass_out_dev,
+                                   int32_t* count_out_dev, float* rot_out_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -11,7 +11,7 @@ import threading
 
 from . import build as _build
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 
 RNF_LAYER_MOBIUS = 0
 RNF_LAYER_AFFINE = 1
@@ -92,6 +92,10 @@ _SIGNATURES = {
     "rnf_min_geodesic": (C.c_int, [_P, _P, _I64, _I64, _P, _P]),
     "rnf_rotation_modes_workspace_bytes": (_I64, [_I64, _I64, C.c_int]),
     "rnf_rotation_modes": (C.c_int, [_P, _I64, _I64, _I64, _P, C.c_int, C.c_float, C.c_float, _P, _I64, _P, _P, _P, _P, _P, _P]),
+    "rnf_rotation_modes_shard_workspace_bytes": (_I64, [_I64, _I64]),
+    "rnf_rotation_modes_shard_setup": (C.c_int, [_P, _I64, _I64, _P, _I64, _P]),
+    "rnf_rotation_modes_shard_round": (C.c_int, [_P, _I64, _I64, _I64, _P, C.c_int, C.c_int, C.c_float, C.c_float, _P, _I64, _P, _P]),
+    "rnf_rotation_modes_shard_merge": (C.c_int, [_P, C.c_int, _I64, C.c_int, C.c_int, _P, _I64, _P, _P, _P, _P, _P, _P, _P]),
 }
 
 _lib = None

@@ -40,6 +40,14 @@ int64_t modes_slices(int64_t G);
 cudaError_t launch_rotation_modes(const float* values, int64_t B, int64_t G, int64_t g_index0, const float* rot, int M, float cos_sep,
                                   float cos_nb, void* workspace, int64_t* index_out, float* value_out, unsigned char* local_max_out,
                                   float* mass_out, int32_t* count_out, cudaStream_t st);
+int64_t modes_shard_workspace_bytes(int64_t G, int64_t B);
+int64_t modes_shard_state_bytes(int64_t B);
+cudaError_t launch_modes_shard_setup(const float* rot, int64_t G, int64_t B, void* workspace, cudaStream_t st);
+cudaError_t launch_modes_shard_round(const float* values, int64_t B, int64_t G, int64_t g_index0, const float* rot, int r, int M,
+                                     float cos_sep, float cos_nb, void* workspace, void* rec_out, cudaStream_t st);
+cudaError_t launch_modes_shard_merge(const void* records, int W, int64_t B, int r, int M, void* workspace, int64_t* index_out,
+                                     float* value_out, unsigned char* local_max_out, float* mass_out, int32_t* count_out, float* rot_out,
+                                     cudaStream_t st);
 }  // namespace rnf
 
 extern "C" {
@@ -541,6 +549,77 @@ int rnf_rotation_modes(const float* values, int64_t B, int64_t G, int64_t g_inde
   const float cos_sep = (float)cos(0.5 * (double)min_separation), cos_nb = (float)cos(0.5 * (double)neighbour_radius);
   cudaError_t e = rnf::launch_rotation_modes(values, B, G, g_index0, rot, M, cos_sep, cos_nb, workspace, index_out, value_out, local_max_out,
                                              mass_out, count_out, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+
+// the thresholds of rnf_rotation_modes and its argument checks (the same expressions, so the shards test the same floats)
+static int modes_thresholds_ok(const char* who, int M, float min_separation, float neighbour_radius) {
+  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
+  const float pi = 3.14159265358979323846f;
+  if (!(neighbour_radius > 0.f) || !(neighbour_radius <= min_separation) || !(min_separation <= pi))
+    return fail(RNF_EINVAL, "%s: need 0 < neighbour_radius <= min_separation <= pi (got %g, %g)", who, (double)neighbour_radius,
+                (double)min_separation);
+  return RNF_OK;
+}
+
+int64_t rnf_rotation_modes_shard_workspace_bytes(int64_t G_r, int64_t B) {
+  if (G_r < 0 || B <= 0) return 0;
+  return rnf::modes_shard_workspace_bytes(G_r, B);
+}
+
+int rnf_rotation_modes_shard_setup(const float* rot, int64_t G_r, int64_t B, void* workspace, int64_t workspace_bytes, void* stream) {
+  const char* who = "rnf_rotation_modes_shard_setup";
+  if (B < 0 || G_r < 0) return fail(RNF_EINVAL, "%s: negative size", who);
+  if (rnf::modes_slices(G_r) > 65535) return fail(RNF_EINVAL, "%s: G_r=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G_r);
+  if (B == 0 || G_r == 0) return RNF_OK;
+  if (!rot || !workspace) return fail(RNF_EINVAL, "%s: null pointer", who);
+  if (workspace_bytes < rnf_rotation_modes_shard_workspace_bytes(G_r, B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  const int rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_modes_shard_setup(rot, G_r, B, workspace, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+int rnf_rotation_modes_shard_round(const float* values, int64_t B, int64_t G_r, int64_t g_index0, const float* rot, int r, int M,
+                                   float min_separation, float neighbour_radius, void* workspace, int64_t workspace_bytes, void* record_out,
+                                   void* stream) {
+  const char* who = "rnf_rotation_modes_shard_round";
+  if (B < 0 || G_r < 0) return fail(RNF_EINVAL, "%s: negative size", who);
+  if (g_index0 < 0) return fail(RNF_EINVAL, "%s: negative g_index0", who);
+  int rc = modes_thresholds_ok(who, M, min_separation, neighbour_radius);
+  if (rc != RNF_OK) return rc;
+  if (r < 0 || r > M) return fail(RNF_EINVAL, "%s: round %d outside 0..M=%d", who, r, M);
+  if (rnf::modes_slices(G_r) > 65535) return fail(RNF_EINVAL, "%s: G_r=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G_r);
+  if (B == 0) return RNF_OK;
+  if (!workspace || !record_out || (G_r > 0 && (!values || !rot))) return fail(RNF_EINVAL, "%s: null pointer", who);
+  if (((uintptr_t)record_out & 15) != 0) return fail(RNF_EINVAL, "%s: record buffer not 16-byte aligned", who);
+  if (workspace_bytes < rnf_rotation_modes_shard_workspace_bytes(G_r, B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  const float cos_sep = (float)cos(0.5 * (double)min_separation), cos_nb = (float)cos(0.5 * (double)neighbour_radius);
+  cudaError_t e = rnf::launch_modes_shard_round(values, B, G_r, g_index0, rot, r, M, cos_sep, cos_nb, workspace, record_out,
+                                                (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+int rnf_rotation_modes_shard_merge(const void* records, int W, int64_t B, int r, int M, void* workspace, int64_t workspace_bytes,
+                                   int64_t* index_out, float* value_out, uint8_t* local_max_out, float* mass_out, int32_t* count_out,
+                                   float* rot_out, void* stream) {
+  const char* who = "rnf_rotation_modes_shard_merge";
+  if (B < 0) return fail(RNF_EINVAL, "%s: negative size", who);
+  if (W < 1) return fail(RNF_EINVAL, "%s: W=%d ranks, need at least 1", who, W);
+  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
+  if (r < 0 || r > M) return fail(RNF_EINVAL, "%s: round %d outside 0..M=%d", who, r, M);
+  if (B == 0) return RNF_OK;
+  if (!records || !workspace || !index_out || !value_out || !local_max_out || !mass_out || !count_out || !rot_out)
+    return fail(RNF_EINVAL, "%s: null pointer", who);
+  if (((uintptr_t)records & 15) != 0) return fail(RNF_EINVAL, "%s: record buffer not 16-byte aligned", who);
+  if (workspace_bytes < rnf::modes_shard_state_bytes(B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  const int rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_modes_shard_merge(records, W, B, r, M, workspace, index_out, value_out, local_max_out, mass_out, count_out,
+                                                rot_out, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
 }
 

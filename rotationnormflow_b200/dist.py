@@ -5,6 +5,10 @@ The reference evaluates the grid on a single GPU in 500 000-rotation chunks (eva
 images with the fused kernel and keeps, per image, (max log p, first arg-max index, sum exp(log p - max)); ONE
 all-gather of ``[B,3]`` float64 (24 B per image per rank) merges them.  There is no other data-path collective: the
 per-(rotation, image) evaluations are independent.
+
+Separated modes over a sharded grid (``sharded_rotation_modes``, ``sharded_estimate_rotation_modes``; DESIGN 4.7 "Sharded") are the
+exception: greedy picking needs each image's global best unlabelled point once per mode, so they make M + 1 all-gathers of an
+80-byte record per image per rank, and return on every rank what the single-GPU call returns on the whole grid.
 """
 from __future__ import annotations
 
@@ -12,6 +16,8 @@ import math
 
 import torch
 import torch.distributed as dist
+
+from .modes import RECORD_BYTES, rotation_modes_rank
 
 
 def shard_range(G: int, rank: int, world: int) -> tuple[int, int]:
@@ -68,3 +74,87 @@ def sharded_grid_log_prob(flow, grid_shard: torch.Tensor, g_index0: int, G_total
         return dict(max=mx, argmax=am, sumexp=se, log_norm=log_normaliser(mx, se, G_total), spread=sn / se)
     mx, am, se = all_merge(out["max"], out["argmax"], out["sumexp"], group)
     return dict(max=mx, argmax=am, sumexp=se, log_norm=log_normaliser(mx, se, G_total))
+
+
+def _record_gather(group):
+    """[B, RECORD_BYTES] -> [W, B, RECORD_BYTES], rank-major: one all_gather_into_tensor (the identity on one rank)."""
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return lambda rec: rec[None]
+    world = dist.get_world_size(group)
+
+    def gather(rec):
+        flat = torch.empty((world * rec.shape[0], RECORD_BYTES), dtype=rec.dtype, device=rec.device)
+        dist.all_gather_into_tensor(flat, rec.contiguous(), group=group)
+        return flat.view(world, rec.shape[0], RECORD_BYTES)
+    return gather
+
+
+def sharded_rotation_modes(values_shard: torch.Tensor, grid_shard: torch.Tensor, g_index0: int, G_total: int, num_modes: int,
+                           min_separation: float, neighbour_radius: float, group=None) -> dict:
+    """``modes.rotation_modes`` over a grid whose contiguous slices live on different ranks: this rank holds ``values_shard``
+    [B,G_r] and ``grid_shard`` [G_r,3,3], the global slice [g_index0, g_index0 + G_r) of a G_total-point grid (``shard_range``).
+    Every rank returns the same dict: index (global), value, local_max, mass, count, valid and ``rotations`` [B,M,3,3], each mode's
+    ``grid_shard`` row as held by the rank that owns it (carried in the record, so any rotation set works; NaN padding).  It equals
+    ``rotation_modes`` on the whole grid: index, value, local_max, count and valid bit for bit, mass up to the order of its sums.
+    M + 1 all-gathers of [B, 80] bytes and nothing else; an empty slice (G_r = 0) takes part in each.  No host synchronisation."""
+    G_r = grid_shard.shape[0]
+    if not (0 <= g_index0 and g_index0 + G_r <= G_total):
+        raise ValueError(f"slice [{g_index0}, {g_index0 + G_r}) is not inside the {G_total}-point grid")
+    return rotation_modes_rank(values_shard, grid_shard, g_index0, num_modes, min_separation, neighbour_radius, _record_gather(group))
+
+
+@torch.no_grad()
+def sharded_estimate_rotation_modes(flow, grid_shard: torch.Tensor, g_index0: int, G_total: int, feature, num_modes: int, *,
+                                    min_separation: float, neighbour_radius=None, fisher_A=None, offset=None, refine_steps: int = 0,
+                                    refine_lr=None, group=None):
+    """``evalpath.estimate_rotation_modes`` on a HEALPix grid of G_total points split across ranks: every rank scores its slice
+    (``grid_shard``, starting at global index ``g_index0``) for all images, the modes are ``sharded_rotation_modes`` of the slices,
+    and every rank returns (rotations [B,M,3,3], dict(logp, mass, valid, count, grid_index)) as the single-GPU call returns them for
+    the same grid and offset.  ``offset`` (the same [3,3] on every rank; None = no offset) right-multiplies the grid.  With
+    refine_steps > 0 every rank runs the same ``refine_rotation`` call on all modes (per-row arithmetic, so the ranks stay
+    identical) and the same merge of refined modes.  ``neighbour_radius`` defaults to ``evalpath.default_neighbour_radius`` of the
+    grid's level.  The images go in chunks whose log-density on the largest slice stays under ``evalpath.MODES_LOGP_BYTES``; the
+    chunking depends on G_total and the world size only, so all ranks make the same collectives."""
+    from . import evalpath
+    from . import grid as rgrid
+    level = rgrid.closest_grid_level(G_total)
+    rho = evalpath.default_neighbour_radius(level) if neighbour_radius is None else float(neighbour_radius)
+    if float(min_separation) < rho:
+        raise ValueError(f"min_separation={min_separation} is below neighbour_radius={rho}: a mode's neighbourhood would reach past its "
+                         "own ball")
+    if refine_steps > 0 and refine_lr is None:
+        raise ValueError("refine_steps > 0 needs refine_lr")
+    dev = grid_shard.device
+    world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
+    G_r, M = grid_shard.shape[0], int(num_modes)
+    B = feature.shape[0] if (feature is not None and flow.condition) else 1
+    chunk = max(1, evalpath.MODES_LOGP_BYTES // (-(-G_total // world) * 4))
+    off = None if offset is None else offset.to(dev, torch.float32)
+    parts = []
+    for s in range(0, B, chunk):
+        f = feature[s:s + chunk] if (feature is not None and flow.condition) else feature
+        A = fisher_A[s:s + chunk] if fisher_A is not None else None
+        if G_r > 0:
+            lp = flow.grid_log_prob(grid_shard, f, offset=off, fisher_A=A, return_logp=True, g_index0=g_index0)["logp"]
+        else:
+            lp = torch.empty((min(chunk, B - s), 0), device=dev, dtype=torch.float32)
+        parts.append(sharded_rotation_modes(lp, grid_shard, g_index0, G_total, M, min_separation, rho, group))
+    md = {k: torch.cat([p[k] for p in parts]) for k in ("index", "value", "local_max", "mass", "rotations")}
+    # what evalpath.estimate_rotation_modes does after rotation_modes, with the grid rows taken from the records
+    valid = md["local_max"]
+    order = torch.sort((~valid).to(torch.int8), dim=1, stable=True).indices
+    valid = torch.gather(valid, 1, order)
+    index = torch.where(valid, torch.gather(md["index"], 1, order), -1)
+    logp = torch.where(valid, torch.gather(md["value"], 1, order), -math.inf)
+    mass = torch.where(valid, torch.gather(md["mass"], 1, order), 0.0)
+    rows = torch.gather(md["rotations"], 1, order[..., None, None].expand(-1, -1, 3, 3))
+    rot = torch.where(valid[..., None, None], rows, md["rotations"][:, :1])          # padding: mode 0's row (a real rotation)
+    if off is not None:
+        rot = rot @ off
+    if refine_steps > 0:
+        mode0 = md["rotations"][:, 0] if off is None else md["rotations"][:, 0] @ off
+        seeds = torch.where(valid[..., None, None], rot, mode0[:, None])              # padding: mode 0 of the grid
+        rot, lp = evalpath.refine_rotation(flow, feature, seeds, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
+        rot, logp, mass, valid, index = evalpath._merge_modes(rot, torch.where(valid, lp, -math.inf), mass, valid, index, rho)
+    rot = torch.where(valid[..., None, None], rot, math.nan)
+    return rot, dict(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)

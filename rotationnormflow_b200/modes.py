@@ -13,6 +13,23 @@ import torch
 from . import _cabi
 
 MAX_MODES = 256
+RECORD_BYTES = 80          # RNF_MODES_RECORD_BYTES: one rank's per-image record of a sharded round
+
+
+def _check_args(values, rotations, num_modes, min_separation, neighbour_radius):
+    M = int(num_modes)
+    theta, rho = float(min_separation), float(neighbour_radius)
+    if not 1 <= M <= MAX_MODES:
+        raise ValueError(f"num_modes must be in 1..{MAX_MODES}, got {num_modes}")
+    if not (0.0 < rho <= theta <= math.pi):
+        raise ValueError(f"need 0 < neighbour_radius <= min_separation <= pi, got neighbour_radius={rho}, min_separation={theta}")
+    if values.dim() not in (1, 2):
+        raise ValueError(f"values must be [B,G] or [G], got {tuple(values.shape)}")
+    if rotations.dim() != 3 or tuple(rotations.shape[1:]) != (3, 3) or rotations.shape[0] != values.shape[-1]:
+        raise ValueError(f"rotations must be [G,3,3] with G = values.shape[-1], got {tuple(rotations.shape)} for {tuple(values.shape)}")
+    if not (values.is_cuda and rotations.is_cuda):
+        raise RuntimeError("rotationnormflow_b200 runs on a B200 only: tensors must be CUDA tensors (there is no CPU fallback)")
+    return M, theta, rho
 
 
 def rotation_modes(values: torch.Tensor, rotations: torch.Tensor, num_modes: int, min_separation: float, neighbour_radius: float,
@@ -35,18 +52,7 @@ def rotation_modes(values: torch.Tensor, rotations: torch.Tensor, num_modes: int
     A pick that is not a local maximum is a "shoulder": the rim of an earlier mode's ball.  On a continuous ridge of equal density
     (the cone and cylinder of SYMSOL) the picks sample the ridge about every ``min_separation``, and their ``local_max`` flags are
     decided by fp32 noise along it."""
-    M = int(num_modes)
-    theta, rho = float(min_separation), float(neighbour_radius)
-    if not 1 <= M <= MAX_MODES:
-        raise ValueError(f"num_modes must be in 1..{MAX_MODES}, got {num_modes}")
-    if not (0.0 < rho <= theta <= math.pi):
-        raise ValueError(f"need 0 < neighbour_radius <= min_separation <= pi, got neighbour_radius={rho}, min_separation={theta}")
-    if values.dim() not in (1, 2):
-        raise ValueError(f"values must be [B,G] or [G], got {tuple(values.shape)}")
-    if rotations.dim() != 3 or tuple(rotations.shape[1:]) != (3, 3) or rotations.shape[0] != values.shape[-1]:
-        raise ValueError(f"rotations must be [G,3,3] with G = values.shape[-1], got {tuple(rotations.shape)} for {tuple(values.shape)}")
-    if not (values.is_cuda and rotations.is_cuda):
-        raise RuntimeError("rotationnormflow_b200 runs on a B200 only: tensors must be CUDA tensors (there is no CPU fallback)")
+    M, theta, rho = _check_args(values, rotations, num_modes, min_separation, neighbour_radius)
     squeeze = values.dim() == 1
     v = (values[None] if squeeze else values).to(torch.float32).contiguous()      # (a reshape to [-1, G] is ambiguous when G == 0)
     B, G = v.shape
@@ -69,3 +75,82 @@ def rotation_modes(values: torch.Tensor, rotations: torch.Tensor, num_modes: int
     if squeeze:
         out = {k: t[0] for k, t in out.items()}
     return out
+
+
+def _ptr(t):
+    return C.c_void_p(t.data_ptr())
+
+
+class RankModes:
+    """One rank's part of ``rotation_modes`` over a grid split across ranks (rnf_rotation_modes_shard_*; DESIGN 4.7 "Sharded").
+
+    The rank holds ``values`` [B,G_r] (or [G_r]) and ``rotations`` [G_r,3,3] of the contiguous global slice starting at ``g_index0``.
+    For r = 0 .. num_modes, ``propose(r)`` returns this rank's records of round r ([B, RECORD_BYTES] uint8); the records of all W
+    ranks, stacked rank-major to [W, B, RECORD_BYTES], go to ``merge(r, gathered)`` on every rank.  After the last merge ``result()``
+    on every rank equals ``rotation_modes`` on the concatenated grid (index, value, local_max, count bit for bit; mass up to the
+    order of its sums).  ``rotation_modes_rank`` runs the loop with a gather function; this class is the step-wise form, for callers
+    that drive several simulated ranks in one process or capture a round in a CUDA graph.  No host synchronisation."""
+
+    def __init__(self, values, rotations, g_index0, num_modes, min_separation, neighbour_radius):
+        if int(g_index0) < 0:
+            raise ValueError(f"g_index0 must be >= 0, got {g_index0}")
+        M, self.theta, self.rho = _check_args(values, rotations, num_modes, min_separation, neighbour_radius)
+        self.M, self.g_index0, self.squeeze = M, int(g_index0), values.dim() == 1
+        v = (values[None] if self.squeeze else values).to(torch.float32).contiguous()
+        self.B, self.G = v.shape
+        dev = self.device = v.device
+        self.v, self.rot = v, rotations.to(dev, torch.float32).contiguous()
+        self.lib = _cabi.load()
+        B = self.B
+        self.out = dict(index=torch.empty((B, M), device=dev, dtype=torch.int64), value=torch.empty((B, M), device=dev, dtype=torch.float32),
+                        local_max=torch.empty((B, M), device=dev, dtype=torch.bool), mass=torch.empty((B, M), device=dev, dtype=torch.float32),
+                        count=torch.empty((B,), device=dev, dtype=torch.int32),
+                        rotations=torch.empty((B, M, 3, 3), device=dev, dtype=torch.float32))
+        self.record = torch.empty((B, RECORD_BYTES), device=dev, dtype=torch.uint8)
+        self.nbytes = int(self.lib.rnf_rotation_modes_shard_workspace_bytes(self.G, B))
+        self.ws = torch.empty((self.nbytes,), device=dev, dtype=torch.uint8)
+        with torch.cuda.device(dev):
+            _cabi.check(self.lib.rnf_rotation_modes_shard_setup(_ptr(self.rot), self.G, B, _ptr(self.ws), self.nbytes, self._stream()))
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def propose(self, r: int) -> torch.Tensor:
+        """Round r on this rank's slice: labels mode r-1's points, tests it, proposes mode r.  Returns the record buffer (reused by
+        the next round: gather it before proposing again)."""
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.rnf_rotation_modes_shard_round(_ptr(self.v), self.B, self.G, self.g_index0, _ptr(self.rot), int(r), self.M,
+                                                                self.theta, self.rho, _ptr(self.ws), self.nbytes, _ptr(self.record),
+                                                                self._stream()))
+        return self.record
+
+    def merge(self, r: int, gathered: torch.Tensor) -> None:
+        """Folds the records of round r of every rank, ``gathered`` [W, B, RECORD_BYTES] uint8 in rank order."""
+        if gathered.dim() != 3 or gathered.dtype != torch.uint8 or tuple(gathered.shape[1:]) != (self.B, RECORD_BYTES):
+            raise ValueError(f"gathered records must be uint8 [W,{self.B},{RECORD_BYTES}], got {gathered.dtype} {tuple(gathered.shape)}")
+        g = gathered.to(self.device).contiguous()
+        o = self.out
+        with torch.cuda.device(self.device):
+            _cabi.check(self.lib.rnf_rotation_modes_shard_merge(_ptr(g), g.shape[0], self.B, int(r), self.M, _ptr(self.ws), self.nbytes,
+                                                                _ptr(o["index"]), _ptr(o["value"]), _ptr(o["local_max"]), _ptr(o["mass"]),
+                                                                _ptr(o["count"]), _ptr(o["rotations"]), self._stream()))
+
+    def result(self) -> dict:
+        """The outputs of ``rotation_modes`` plus ``rotations`` [B,M,3,3] (the owning rank's matrix of each mode, NaN padding) and
+        ``valid`` [B,M] (entry < count)."""
+        out = dict(self.out)
+        out["valid"] = torch.arange(self.M, device=self.device)[None, :] < out["count"][:, None]
+        if self.squeeze:
+            out = {k: t[0] for k, t in out.items()}
+        return out
+
+
+def rotation_modes_rank(values: torch.Tensor, rotations: torch.Tensor, g_index0: int, num_modes: int, min_separation: float,
+                        neighbour_radius: float, gather) -> dict:
+    """This rank's call of ``rotation_modes`` over a grid split across W ranks (``RankModes``): M + 1 rounds, each one call of
+    ``gather`` ([B, RECORD_BYTES] uint8 -> [W, B, RECORD_BYTES], rank-major; ``torch.distributed.all_gather_into_tensor`` across
+    processes, ``torch.stack`` over simulated ranks).  Every rank returns the dict of ``RankModes.result``."""
+    rm = RankModes(values, rotations, g_index0, num_modes, min_separation, neighbour_radius)
+    for r in range(rm.M + 1):
+        rm.merge(r, gather(rm.propose(r)))
+    return rm.result()
