@@ -143,9 +143,14 @@ def _wrapped_angles(h, r, v):
 
 
 def _mobius_prep(sd, prefix, x, y, feature, K):
-    """(flow/mobiusflow.py:52-72): MLP, split, project w onto plane orthogonal to y, frame, mixture weights."""
+    """(flow/mobiusflow.py:52-72): MLP, then mobius_params of its output."""
     inp = y if feature is None else torch.cat((y, feature), -1)
-    out = conditioner(sd, prefix + "conditioner.", inp)
+    return mobius_params(conditioner(sd, prefix + "conditioner.", inp), x, y, K)
+
+
+def mobius_params(out, x, y, K):
+    """(flow/mobiusflow.py:58-72): conditioner output out [N,4K] -> frame r, v [N,3], mixture weights pi [N,K] and squashed centres
+    w' [N,K,3]: split, project w onto the plane orthogonal to y, frame, softplus weights, squash."""
     a, w = out[:, :K], out[:, K:].reshape(-1, K, 3)
     w = w - (w * y[:, None, :]).sum(-1, keepdim=True) * y[:, None, :]     # (I - y y^T) w
     r = -x
@@ -182,7 +187,10 @@ def _assemble(p, c0, c1, c2):
 
 def mobius_forward(sd, prefix, R, p, feature, K, explicit_jacobian=False):
     x, y = R[:, :, p[0]], R[:, :, p[1]]
-    r, v, pi, w = _mobius_prep(sd, prefix, x, y, feature, K)
+    return _mobius_forward(x, y, p, *_mobius_prep(sd, prefix, x, y, feature, K), explicit_jacobian)
+
+
+def _mobius_forward(x, y, p, r, v, pi, w, explicit_jacobian=False):
     h, f = _mobius_h(x, w)
     th = (pi * _wrapped_angles(h, r, v)).sum(1, keepdim=True)             # :100
     tx = r * torch.cos(th) + v * torch.sin(th)                            # :102
@@ -225,8 +233,10 @@ class BinFindWithGrad(torch.autograd.Function):
     """BinFind (flow/mobiusflow.py:189-273) including its backward: the implicit-function gradient at the returned root."""
 
     @staticmethod
-    def forward(ctx, y, r, v, pi, w):
-        x0 = bisect(y, r, v, pi, w)
+    def forward(ctx, y, r, v, pi, w, root=None):
+        """``root`` [N,1]: return it instead of bisecting, so that the implicit-function gradient is evaluated at a given point (the
+        root another implementation returned)."""
+        x0 = bisect(y, r, v, pi, w) if root is None else root.detach().to(y.dtype)
         ctx.save_for_backward(x0.detach(), r.detach(), v.detach(), pi.detach(), w.detach())
         return x0
 
@@ -241,16 +251,27 @@ class BinFindWithGrad(torch.autograd.Function):
         v_grad = torch.where(ok, -gv / gx, torch.zeros_like(gv)) * x_grad
         w_grad = torch.where(ok.unsqueeze(-1), -gw / gx.unsqueeze(-1), torch.zeros_like(gw)) * x_grad.unsqueeze(-1)
         pi_grad = torch.where(ok, -gpi / gx, torch.zeros_like(gpi)) * x_grad
-        return y_grad, r_grad, v_grad, pi_grad, w_grad
+        return y_grad, r_grad, v_grad, pi_grad, w_grad, None
 
 
 def mobius_inverse(sd, prefix, R, p, feature, K, explicit_jacobian=False):
     tx, ty = R[:, :, p[0]], R[:, :, p[1]]
-    r, v, pi, w = _mobius_prep(sd, prefix, tx, ty, feature, K)
+    return _mobius_inverse(tx, ty, p, *_mobius_prep(sd, prefix, tx, ty, feature, K), explicit_jacobian)
+
+
+def _target_angle(tx, r, v):
+    """The angle of the given column in its own frame, wrapped to [0, 2 pi) with 2 pi - 1e-4 .. 2 pi mapped to 0 (:157-167)."""
     tt = torch.atan2((tx * v).sum(-1), (tx * r).sum(-1)).reshape(-1, 1)
     tt = torch.where(tt >= 0, tt, tt + 2 * math.pi)
-    tt = torch.where(abs(tt - 2 * math.pi) < 1e-4, torch.zeros_like(tt), tt)   # :163-167
-    th = BinFindWithGrad.apply(tt, r, v, pi, w) if torch.is_grad_enabled() else bisect(tt, r, v, pi, w)
+    return torch.where(abs(tt - 2 * math.pi) < 1e-4, torch.zeros_like(tt), tt)   # :163-167
+
+
+def _mobius_inverse(tx, ty, p, r, v, pi, w, explicit_jacobian=False, root=None):
+    tt = _target_angle(tx, r, v)
+    if torch.is_grad_enabled() or root is not None:
+        th = BinFindWithGrad.apply(tt, r, v, pi, w, root)
+    else:
+        th = bisect(tt, r, v, pi, w)
     x = r * torch.cos(th) + v * torch.sin(th)
     if explicit_jacobian:
         ldj = _explicit_ldj(x, r, v, pi, w)
@@ -260,6 +281,18 @@ def mobius_inverse(sd, prefix, R, p, feature, K, explicit_jacobian=False):
     z = torch.linalg.cross(x, ty, dim=-1)
     z = z / z.norm(dim=-1, keepdim=True)
     return _assemble(p, x, ty, z), -ldj
+
+
+def mobius_layer(R, out, p0, K, inverse, root=None):
+    """One Mobius layer after its conditioner: (R [N,3,3], out [N,4K]) -> (R', ldj), the moving column p0 (the cyclic rows 0-2 of
+    PERMUTE_TABLE).  Inverse direction: ``root`` [N] evaluates the layer and BinFind's implicit-function gradient at that angle
+    instead of the bisection's."""
+    p = PERMUTE_TABLE[p0]
+    x, y = R[:, :, p[0]], R[:, :, p[1]]
+    prm = mobius_params(out, x, y, K)
+    if not inverse:
+        return _mobius_forward(x, y, p, *prm)
+    return _mobius_inverse(x, y, p, *prm, root=None if root is None else root.reshape(-1, 1))
 
 
 # ----------------------------------------------------------------------------------------------

@@ -649,9 +649,13 @@ def test_composed_operators(tag, case, inverse, request):
     """The per-layer differentiable operators (train.composed_run: Flow.forward / Flow.inverse under autograd) against autograd
     through the fp64 oracle, as tests/test_gpu_train.py: values, then parameter / feature / tangential rotation gradients."""
     if (tag, case, inverse) == ("s_symsol", "logits", False):
-        # measured on a B200: the layers.3 fc_first.weight gradient is 4.9e-3 from the fp64 oracle (bound 2e-3), while the
-        # gradient reaching that conditioner's output is within 1.5e-6; the fused Flow.log_prob meets 1e-4 (DESIGN 4.1)
-        request.applymarker(pytest.mark.xfail(strict=True, reason="composed-path fc_first gradient of s_symsol/logits: 4.9e-3"))
+        # measured on a B200: the layers.3 fc_first.weight gradient is 4.9e-3 from the fp64 oracle (bound 2e-3).  One first-layer
+        # pre-activation of that conditioner (row 41, unit 1) is -1.2e-7 in the fp64 oracle and positive in the fp32 forward, so the
+        # two take different sides of the ReLU kink, where the gradient is discontinuous.  With the oracle's ReLU branches, the G_out
+        # the Mobius kernel returns reproduces the oracle's gradient to 1e-6 (tests/test_train_ops.py
+        # test_composed_symsol_logits_localised; DESIGN 4.1).  No bound fits a discontinuity, so this case stays an expected failure.
+        request.applymarker(pytest.mark.xfail(strict=True, reason="s_symsol/logits: a layers.3 fc_first pre-activation -1.2e-7 "
+                                                                  "from zero takes the other ReLU branch in fp32 (gradient 4.9e-3 off)"))
     b = _base(tag)
     sd, _ = stress_case(tag, case)
     cfg = b["cfg"]
