@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define RNF_ABI_VERSION 14
+#define RNF_ABI_VERSION 15
 
 /* error codes */
 #define RNF_OK 0
@@ -333,6 +333,30 @@ int rnf_rotation_modes_shard_round(const float* values_dev, int64_t B, int64_t G
 int rnf_rotation_modes_shard_merge(const void* records_dev, int W, int64_t B, int r, int M, void* workspace_dev, int64_t workspace_bytes,
                                    int64_t* index_out_dev, float* value_out_dev, uint8_t* local_max_out_dev, float* mass_out_dev,
                                    int32_t* count_out_dev, float* rot_out_dev, void* stream);
+
+/*
+ * Coarse-to-fine search on the HEALPix grids (csrc/hgrid.cu; DESIGN 4.8).
+ *
+ * rnf_healpix_children: the 8 level-(level+1) children of level-`level` grid indices (0 <= level <= 7).  For parent idx = t*npix + p
+ * (nside = 2^level, npix = 12 nside^2, p the RING pixel) child k = 4*dt + j (dt = 0, 1; j = 0..3) is
+ *   t' = 2t + dt,  p' = nest2ring(2 nside, 4 ring2nest(nside, p) + j),  index t' * 4 npix + p'
+ * (the NESTED subdivision: the children of all level-l indices partition the level-(l+1) grid).
+ *   parent_dev [n] int64; offset_dev [3,3] or NULL; child_out_dev [n,8] int64; R_out_dev [n,8,3,3] = rnf_healpix_grid's row of the
+ *   child, times the offset by the fmaf chain of rnf_grid_logprob (bit for bit the rotation the grid pass scores at that index).
+ *   A parent outside [0, 72*8^level) (padding -1) gives children -1 and NaN rotations.  n == 0 does nothing; n <= (2^31 - 1) * 32.
+ *
+ * rnf_topk: per image the K best of values_dev [B,C] under the order of the grid arg-max (NaN first, then the larger value, then the
+ * lower index), best first.  index_dev [B,C] int64 gives each entry's index (NULL: the column number); an entry with a negative index
+ * is padding, ranked after every other entry.  1 <= K <= 4096; v_out_dev [B,K], i_out_dev [B,K] int64; places past the real entries
+ * (K > C, or padding) are (-inf, -1).  workspace_dev: rnf_topk_workspace_bytes(B, C, K) bytes (0 is a valid size: no buffer needed).
+ * B == 0 does nothing; C == 0 writes padding.  1 + ceil(log2(ceil(C / max(4096, 2 Kp)))) launches (Kp = K rounded up to a power of
+ * two), no atomics, no host synchronisation: bitwise reproducible and CUDA-graph capturable.
+ */
+int rnf_healpix_children(int level, const int64_t* parent_dev, int64_t n, const float* offset_dev, int64_t* child_out_dev, float* R_out_dev,
+                         void* stream);
+int64_t rnf_topk_workspace_bytes(int64_t B, int64_t C, int K);
+int rnf_topk(const float* values_dev, const int64_t* index_dev, int64_t B, int64_t C, int K, void* workspace_dev, int64_t workspace_bytes,
+             float* v_out_dev, int64_t* i_out_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -11,7 +11,7 @@ import threading
 
 from . import build as _build
 
-ABI_VERSION = 14
+ABI_VERSION = 15
 
 RNF_LAYER_MOBIUS = 0
 RNF_LAYER_AFFINE = 1
@@ -96,6 +96,9 @@ _SIGNATURES = {
     "rnf_rotation_modes_shard_setup": (C.c_int, [_P, _I64, _I64, _P, _I64, _P]),
     "rnf_rotation_modes_shard_round": (C.c_int, [_P, _I64, _I64, _I64, _P, C.c_int, C.c_int, C.c_float, C.c_float, _P, _I64, _P, _P]),
     "rnf_rotation_modes_shard_merge": (C.c_int, [_P, C.c_int, _I64, C.c_int, C.c_int, _P, _I64, _P, _P, _P, _P, _P, _P, _P]),
+    "rnf_healpix_children": (C.c_int, [C.c_int, _P, _I64, _P, _P, _P, _P]),
+    "rnf_topk_workspace_bytes": (_I64, [_I64, _I64, C.c_int]),
+    "rnf_topk": (C.c_int, [_P, _P, _I64, _I64, C.c_int, _P, _I64, _P, _P, _P]),
 }
 
 _lib = None

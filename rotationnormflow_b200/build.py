@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "librnf_b200.so")
 STAMP = os.path.join(HERE, "csrc", ".build_stamp")
-SOURCES = ["rnf_abi.cu", "flow_v1.cu", "flow_row.cu", "flow_t4.cu", "condition.cu", "dedup.cu", "healpix.cu", "fisher_sample.cu", "train_ops.cu", "flow_grad.cu", "modes.cu"]
+SOURCES = ["rnf_abi.cu", "flow_v1.cu", "flow_row.cu", "flow_t4.cu", "condition.cu", "dedup.cu", "healpix.cu", "fisher_sample.cu", "train_ops.cu", "flow_grad.cu", "modes.cu", "hgrid.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-shared", "--expt-relaxed-constexpr", "-Xptxas", "-v", "-lcuda",

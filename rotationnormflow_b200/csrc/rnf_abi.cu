@@ -48,6 +48,12 @@ cudaError_t launch_modes_shard_round(const float* values, int64_t B, int64_t G, 
 cudaError_t launch_modes_shard_merge(const void* records, int W, int64_t B, int r, int M, void* workspace, int64_t* index_out,
                                      float* value_out, unsigned char* local_max_out, float* mass_out, int32_t* count_out, float* rot_out,
                                      cudaStream_t st);
+cudaError_t launch_healpix_children(int level, const int64_t* parent, int64_t n, const float* offset, int64_t* child_out, float* R_out,
+                                    cudaStream_t st);
+int64_t topk_slices(int64_t C, int K);
+int64_t topk_workspace_bytes(int64_t B, int64_t C, int K);
+cudaError_t launch_topk(const float* values, const int64_t* index, int64_t B, int64_t C, int K, void* workspace, float* v_out,
+                        int64_t* i_out, cudaStream_t st);
 }  // namespace rnf
 
 extern "C" {
@@ -620,6 +626,43 @@ int rnf_rotation_modes_shard_merge(const void* records, int W, int64_t B, int r,
   if (rc != RNF_OK) return rc;
   cudaError_t e = rnf::launch_modes_shard_merge(records, W, B, r, M, workspace, index_out, value_out, local_max_out, mass_out, count_out,
                                                 rot_out, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+// argument checks before the device check, so that a bad call is reported as such on any host
+int rnf_healpix_children(int level, const int64_t* parent, int64_t n, const float* offset, int64_t* child_out, float* R_out, void* stream) {
+  const char* who = "rnf_healpix_children";
+  if (level < 0 || level > 7) return fail(RNF_EINVAL, "%s: child level %d outside 1..8", who, level + 1);
+  if (n < 0) return fail(RNF_EINVAL, "%s: negative n", who);
+  if (n == 0) return RNF_OK;
+  if (!parent || !child_out || !R_out) return fail(RNF_EINVAL, "%s: null buffer", who);
+  // one thread per child, 256 per block: gridDim.x = n / 32 blocks must stay within 2^31 - 1
+  if (n > (int64_t)0x7fffffff * 32) return fail(RNF_EINVAL, "%s: n=%lld parents exceed the (2^31 - 1) * 32 of one launch", who, (long long)n);
+  const int rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_healpix_children(level, parent, n, offset, child_out, R_out, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+int64_t rnf_topk_workspace_bytes(int64_t B, int64_t C, int K) {
+  if (B <= 0 || C < 0 || K < 1 || K > 4096) return 0;
+  return rnf::topk_workspace_bytes(B, C, K);
+}
+
+int rnf_topk(const float* values, const int64_t* index, int64_t B, int64_t C, int K, void* workspace, int64_t workspace_bytes, float* v_out,
+             int64_t* i_out, void* stream) {
+  const char* who = "rnf_topk";
+  if (B < 0 || C < 0) return fail(RNF_EINVAL, "%s: negative size", who);
+  if (K < 1 || K > 4096) return fail(RNF_EINVAL, "%s: K=%d outside 1..4096", who, K);
+  if (B > 0x7fffffffLL) return fail(RNF_EINVAL, "%s: B=%lld images exceed one launch", who, (long long)B);
+  if (rnf::topk_slices(C, K) > 65535) return fail(RNF_EINVAL, "%s: C=%lld entries exceed the 65535 slices of one launch", who, (long long)C);
+  if (B == 0) return RNF_OK;
+  const int64_t need = rnf_topk_workspace_bytes(B, C, K);
+  if (!v_out || !i_out || (C > 0 && !values) || (need > 0 && !workspace)) return fail(RNF_EINVAL, "%s: null buffer", who);
+  if (workspace_bytes < need) return fail(RNF_EINVAL, "%s: workspace too small", who);
+  const int rc = rnf_device_check(nullptr);
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_topk(values, index, B, C, K, workspace, v_out, i_out, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
 }
 

@@ -4,6 +4,8 @@
     estimate_rotation_sampling  agent.py:238-266 (eval_acc: inverse-flow samples + arg-max per image), uniform base
     refine_rotation             eval.py:464-480  (nll_grad: Adam on a quaternion per row, climbing log p; one fused launch per step)
     estimate_rotation_modes     (no reference counterpart) the M best separated modes per image from one grid pass, optionally refined
+    estimate_rotation_hierarchical  (no reference counterpart) the grid arg-max of a fine level from a coarse grid pass and a beam of
+                                child cells per level
 
 Both avoid the reference's `feature.repeat` (4 GB per 500 000-row chunk at F = 2080, eval.py:450) and its per-image
 Python loop; all per-rotation arithmetic runs in the fused kernels.
@@ -24,6 +26,9 @@ NEIGHBOUR_RADIUS = (1.570796, 0.778990, 0.392699, 0.196350, 0.098175, 0.049087)
 # estimate_rotation_modes evaluates the grid in image chunks whose [chunk, G] float32 log-density stays under this many bytes
 # (a level-6 grid is 151 MB per image)
 MODES_LOGP_BYTES = 1 << 30
+# estimate_rotation_hierarchical scores flows the fused kernels cannot run in pieces of at most this many bytes of per-row state
+# (a feature row per rotation, F = 2080: about 112 000 rotations)
+HIER_LAYERWISE_BYTES = 1 << 30
 
 
 def _random_rotation(device, generator=None):
@@ -117,6 +122,126 @@ def estimate_rotation_modes(flow, feature, number_queries, num_modes, *, min_sep
     rot = torch.where(valid[..., None, None], rot, math.nan)
     out.update(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)
     return rot, out
+
+
+def _score_rows(flow, rows, feature, per_image, fisher_A, mlp_mode):
+    """log p of image-major ``rows`` [B*per_image,3,3] (or [per_image,3,3], the same rows for every image) through Flow.forward, plus
+    the matrix-Fisher term of ``fisher_A`` [B,3,3]: ldj + (tr(A_b R') - c_b), the arithmetic of the grid kernels' epilogue.
+    Returns [B, per_image].
+
+    Flows the fused kernels run go in one launch.  The others (segments != 64, ConditionLU) run the per-layer operators, which build a
+    feature row per rotation: they go one image at a time, in pieces of at most HIER_LAYERWISE_BYTES of per-row state, so memory does not
+    grow with the number of images, and ConditionLU (batch-coupled: rows 0..3 of a launch decide its diagonal) sees one image's feature
+    in every row of a launch, the reference's own calling convention (eval.py:450)."""
+    from .fisher import MatrixFisherN
+    from .flow import fused_kernels_run
+    conditional = feature is not None and flow.condition
+    B = feature.shape[0] if conditional else (fisher_A.shape[0] if fisher_A is not None else 1)
+    shared = rows.shape[0] == per_image and B > 1
+    if fused_kernels_run(flow.layers):
+        R = rows.unsqueeze(0).expand(B, -1, -1, -1).reshape(-1, 3, 3) if shared else rows
+        idx = torch.arange(B * per_image, device=rows.device, dtype=torch.int32) // per_image if conditional else None
+        R_out, ldj = flow.forward(R, feature, feature_index=idx, mlp_mode=mlp_mode)
+        if fisher_A is not None:
+            ldj = ldj + MatrixFisherN(fisher_A)._log_prob(R_out)
+        return ldj.reshape(B, per_image)
+    K = max([l.K for l in flow.layers if l.kind == "mobius"] + [1])
+    per_row = 4 * (flow.feature_dim + 19 + 4 * K + 2 * 64)          # feature row, R and R', ldj, one conditioner's output and hidden
+    piece = max(1, HIER_LAYERWISE_BYTES // per_row)
+    out = torch.empty((B, per_image), device=rows.device, dtype=torch.float32)
+    for b in range(B):
+        fb = feature[b:b + 1] if conditional else None
+        fisher = MatrixFisherN(fisher_A[b:b + 1]) if fisher_A is not None else None
+        for s in range(0, per_image, piece):
+            n = min(piece, per_image - s)
+            r = rows[s:s + n] if shared or B == 1 else rows[b * per_image + s:b * per_image + s + n]
+            idx = torch.zeros(n, device=rows.device, dtype=torch.int32) if conditional else None
+            R_out, ldj = flow.forward(r, fb, feature_index=idx, mlp_mode=mlp_mode)
+            if fisher is not None:
+                ldj = ldj + fisher._log_prob(R_out)
+            out[b, s:s + n] = ldj
+    return out
+
+
+@torch.no_grad()
+def estimate_rotation_hierarchical(flow, feature, number_queries, *, start_level=3, beam=64, fisher_A=None, offset=None, generator=None,
+                                   mlp_mode=None):
+    """The arg-max of log p over the level-L HEALPix grid (L = closest_grid_level(number_queries), as estimate_rotation_grid) by a
+    coarse-to-fine search, per image (DESIGN 4.8):
+
+    1. score the full level-``start_level`` grid (Flow.grid_log_prob) and keep the ``beam`` best indices in the order of the grid
+       arg-max (NaN first, then the larger value, then the lower index; grid.top_k);
+    2. for each finer level up to L: expand the kept indices to their 8 children each (grid.healpix_children), score them with
+       Flow.forward at exactly the rotation the grid pass scores at that index (grid rotation times the offset, plus the matrix-Fisher
+       term with ``fisher_A``), and keep the ``beam`` best;
+    3. report the best candidate of level L.
+
+    Every candidate is a member of the level-L grid; with beam >= 72 * 8^(L-1) the search scores every level-L rotation.  A peak
+    narrower than the coarse spacing can be missed.  Flow.forward and Flow.grid_log_prob do not round a rotation's log p bit for bit
+    alike (DESIGN 4.8: up to 6e-5 relative measured), so the reported log p can exceed the full grid's maximum by that difference, and
+    an exhaustive search can pick another index whose full-grid log p is within it of the maximum.  A wider beam usually does at least
+    as well, but not always: it can drop the branch a narrower beam follows.
+
+    Flow.forward runs every layer kind (ablation layers, ConditionLU, segments != 64).  Flow.grid_log_prob refuses the last two, so for
+    them the coarse pass scores the level-``start_level`` grid as the children of the level below, through Flow.forward, one image at
+    a time (_score_rows): they need start_level >= 1 and a final level >= 1.  ``offset`` / ``generator`` as in estimate_rotation_grid.
+    start_level >= L is the plain grid arg-max of level L.  Images are searched in chunks whose coarse [chunk, G0] log-density stays
+    under MODES_LOGP_BYTES.
+
+    Returns (est [B,3,3], dict(logp [B], index [B] int64 level-L grid index, level = L, top_logp [B,beam], top_index [B,beam] (the final
+    beam, best first; (-inf, -1) where the level has fewer than beam rotations), evaluated = rotations scored per image))."""
+    L = rgrid.closest_grid_level(number_queries)
+    if isinstance(beam, bool) or int(beam) != beam or not 1 <= int(beam) <= rgrid.MAX_TOP_K:
+        raise ValueError(f"beam must be an integer in 1..{rgrid.MAX_TOP_K}, got {beam}")
+    if isinstance(start_level, bool) or int(start_level) != start_level or not 0 <= int(start_level) <= 8:
+        raise ValueError(f"start_level must be an integer in 0..8, got {start_level}")
+    beam, l0 = int(beam), min(int(start_level), L)
+    from .flow import fused_kernels_run
+    fused = fused_kernels_run(flow.layers)
+    if not fused and l0 == 0:
+        raise ValueError(f"a flow Flow.grid_log_prob cannot run (segments != 64 or ConditionLU) scores its coarse level as the children "
+                         f"of the level below: it needs start_level >= 1 and a final level >= 1, got start_level={start_level}, final "
+                         f"level {L} (number_queries={number_queries})")
+    dev = feature.device if feature is not None else torch.device("cuda", torch.cuda.current_device())
+    if offset is None:
+        offset = _random_rotation(dev, generator)
+    offset = offset.to(dev, torch.float32)
+    conditional = feature is not None and flow.condition
+    B = feature.shape[0] if conditional else 1
+    G0 = rgrid.GRID_SIZES[l0]
+    chunk = max(1, MODES_LOGP_BYTES // (G0 * 4))
+    parts = []
+    for s in range(0, B, chunk):
+        f = feature[s:s + chunk] if conditional else feature
+        A = fisher_A[s:s + chunk] if fisher_A is not None else None
+        nb = min(chunk, B - s)
+        if fused:
+            grid0 = rgrid.get_closest_available_grid(G0, dev)
+            lp = flow.grid_log_prob(grid0, f, offset=offset, fisher_A=A, return_logp=True, mlp_mode=mlp_mode)["logp"]
+            idx0 = None
+        else:
+            idx0, rot0 = rgrid.healpix_children(l0 - 1, torch.arange(G0 // 8, device=dev), offset)
+            lp = _score_rows(flow, rot0.reshape(G0, 3, 3), f, G0, A, mlp_mode)
+            idx0 = idx0.reshape(1, G0).expand(nb, G0)
+        k = beam if l0 == L else min(beam, G0)
+        top_v, top_i = rgrid.top_k(lp, idx0, k)
+        if l0 == L:     # the plain grid arg-max: the grid pass's own rotation (estimate_rotation_grid)
+            est = rgrid.get_closest_available_grid(G0, dev)[top_i[:, 0].clamp(min=0)] @ offset
+        for level in range(l0 + 1, L + 1):
+            child, rot = rgrid.healpix_children(level - 1, top_i.reshape(-1), offset)       # [nb*k, 8], [nb*k, 8, 3, 3]
+            n = 8 * top_i.shape[1]
+            lp = _score_rows(flow, rot.reshape(-1, 3, 3), f, n, A, mlp_mode)
+            child = child.reshape(nb, n)
+            top_v, top_i = rgrid.top_k(lp, child, beam if level == L else min(beam, rgrid.GRID_SIZES[level]))
+            if level == L:
+                pos = (child == top_i[:, :1]).to(torch.int8).argmax(1)
+                est = rot.reshape(nb, n, 3, 3)[torch.arange(nb, device=dev), pos]
+        parts.append((est, top_v, top_i))
+    est = torch.cat([p[0] for p in parts])
+    top_v = torch.cat([p[1] for p in parts])
+    top_i = torch.cat([p[2] for p in parts])
+    evaluated = G0 + sum(8 * min(beam, rgrid.GRID_SIZES[l - 1]) for l in range(l0 + 1, L + 1))
+    return est, dict(logp=top_v[:, 0], index=top_i[:, 0], level=L, top_logp=top_v, top_index=top_i, evaluated=evaluated)
 
 
 def _merge_modes(rot, logp, mass, valid, index, radius):

@@ -494,11 +494,17 @@ def _check_rotation(rotation):
     return rotation.to(torch.float32).contiguous()
 
 
+def fused_kernels_run(layers) -> bool:
+    """True when the fused kernels evaluate this layer stack: they are specialised for Mobius layers of K_SEGMENTS components and have
+    no ConditionLU (batch-coupled in the reference), which run in the per-layer operators of train.py instead."""
+    return not any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers)
+
+
 def _needs_composed(layers, rotation, feature) -> bool:
     """True when the call must run layer by layer in the differentiable operators of train.py: autograd is on and something
     requires grad (the reference builds a graph there: training at agent.py:87, eval.py:468-477), or a Mobius layer has a number of
     mixture components other than the 64 the fused kernels are specialised for."""
-    if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers):
+    if not fused_kernels_run(layers):
         return True
     return _wants_grad(layers, rotation, feature)
 
@@ -657,7 +663,7 @@ class Flow(_NoProgramState, nn.Module):
                 raise ValueError("fisher_A must have one 3x3 matrix per image")
         if N == 0:
             return R.new_empty((0,)), R.new_empty((0, 3, 3))
-        if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers):
+        if not fused_kernels_run(layers):
             return self._log_prob_grad_composed(R, feature, idx, rpi, A9, c)
         prog = _program(self, layers, self._perm_rows(), self.feature_dim, dev)
         cond = prog.condition(feature) if prog.cond_floats else None
@@ -710,7 +716,7 @@ class Flow(_NoProgramState, nn.Module):
                 raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
             idx = torch.arange(N, device=dev, dtype=torch.int32) // (N // B)
         perms = self._perm_rows()
-        if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in layers):
+        if not fused_kernels_run(layers):
             rows = feature[idx.long()] if feature is not None else None
             R_out, logp = train.composed_run(layers, perms, R, rows, False)
         else:
@@ -756,7 +762,7 @@ class Flow(_NoProgramState, nn.Module):
         G_ = _check_rotation(grid)
         if torch.is_grad_enabled() and torch.is_tensor(feature) and feature.requires_grad:
             raise NotImplementedError(_GRAD_MESSAGE.format(what="the feature"))
-        if any((l.kind == "mobius" and l.K != engine.K_SEGMENTS) or l.kind == "aff_clu" for l in self.layers):
+        if not fused_kernels_run(self.layers):
             raise NotImplementedError(f"Flow.grid_log_prob runs in the fused kernels, which are specialised for segments={engine.K_SEGMENTS} and "
                                       "per-image conditional affines; use Flow.forward on the grid rotations for other segment counts / ConditionLU")
         prog = _program(self, list(self.layers), self._perm_rows(), self.feature_dim, G_.device)

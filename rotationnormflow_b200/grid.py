@@ -70,3 +70,68 @@ def generate_queries(number_queries: int, mode: str = "random", device=None) -> 
                      two_s * (i * j + k * r), 1 - two_s * (i * i + k * k), two_s * (j * k - i * r),
                      two_s * (i * k - j * r), two_s * (j * k + i * r), 1 - two_s * (i * i + j * j)), -1)
     return m.reshape(-1, 3, 3)
+
+
+# ---- coarse-to-fine search (csrc/hgrid.cu; DESIGN 4.8) ------------------------------------------------------------------------------
+MAX_TOP_K = 4096
+
+
+def healpix_children(level: int, index: torch.Tensor, offset: torch.Tensor | None = None):
+    """The 8 level-(level+1) children of level-``level`` grid indices ``index`` [n] (rnf_healpix_children; 0 <= level <= 7).
+
+    For idx = t * npix + p (nside = 2^level, npix = 12 nside^2, p the RING pixel) child k = 4 dt + j is the index t' * 4 npix + p' with
+    t' = 2 t + dt and p' = nest2ring(2 nside, 4 ring2nest(nside, p) + j): the children of all level-l indices partition the
+    level-(l+1) grid.  Returns (child [n,8] int64, rotations [n,8,3,3] float32): ``healpix_grid(level + 1)[child]`` times ``offset``
+    [3,3] by the arithmetic of ``Flow.grid_log_prob``, bit for bit the rotation the grid pass scores at that index.  A parent outside
+    the level's grid (padding -1) gives children -1 and NaN rotations.  No host synchronisation."""
+    level = int(level)
+    if not 0 <= level <= 7:
+        raise ValueError(f"level must be in 0..7 (children at levels 1..8), got {level}")
+    if not index.is_cuda:
+        raise RuntimeError("healpix_children runs on a B200 only: `index` must be a CUDA tensor (there is no CPU fallback)")
+    idx = index.reshape(-1).to(torch.int64).contiguous()
+    dev = idx.device
+    n = idx.shape[0]
+    child = torch.empty((n, 8), device=dev, dtype=torch.int64)
+    rot = torch.empty((n, 8, 3, 3), device=dev, dtype=torch.float32)
+    off = None if offset is None else offset.to(dev, torch.float32).reshape(3, 3).contiguous()
+    lib = _cabi.load()
+    with torch.cuda.device(dev):
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _cabi.check(lib.rnf_healpix_children(level, C.c_void_p(idx.data_ptr()), n, C.c_void_p(off.data_ptr()) if off is not None else None,
+                                             C.c_void_p(child.data_ptr()), C.c_void_p(rot.data_ptr()), st))
+    return child, rot
+
+
+def top_k(values: torch.Tensor, index: torch.Tensor | None, k: int):
+    """Per image the ``k`` best of ``values`` [B,C] (or [C]) under the order of the grid arg-max: NaN first, then the larger value,
+    then the lower index; best first (rnf_topk, 1 <= k <= 4096).  ``index`` (same shape, int64) gives each entry's index, None the
+    column number; an entry with a negative index is padding and ranks after every other one.  Returns (values [B,k], index [B,k]
+    int64); places without a real entry (k > C, or padding) are (-inf, -1).  No host synchronisation; bitwise reproducible."""
+    k = int(k)
+    if not 1 <= k <= MAX_TOP_K:
+        raise ValueError(f"k must be in 1..{MAX_TOP_K}, got {k}")
+    if values.dim() not in (1, 2):
+        raise ValueError(f"values must be [B,C] or [C], got {tuple(values.shape)}")
+    if index is not None and tuple(index.shape) != tuple(values.shape):
+        raise ValueError(f"index must have the shape of values {tuple(values.shape)}, got {tuple(index.shape)}")
+    if not values.is_cuda:
+        raise RuntimeError("top_k runs on a B200 only: `values` must be a CUDA tensor (there is no CPU fallback)")
+    squeeze = values.dim() == 1
+    v = (values[None] if squeeze else values).to(torch.float32).contiguous()
+    B, Cn = v.shape
+    dev = v.device
+    ix = None if index is None else (index[None] if squeeze else index).to(dev, torch.int64).contiguous()
+    out_v = torch.empty((B, k), device=dev, dtype=torch.float32)
+    out_i = torch.empty((B, k), device=dev, dtype=torch.int64)
+    lib = _cabi.load()
+    if B > 0:
+        nbytes = int(lib.rnf_topk_workspace_bytes(B, Cn, k))
+        ws = torch.empty((max(nbytes, 1),), device=dev, dtype=torch.uint8)
+        with torch.cuda.device(dev):
+            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            _cabi.check(lib.rnf_topk(C.c_void_p(v.data_ptr()), C.c_void_p(ix.data_ptr()) if ix is not None else None, B, Cn, k,
+                                     C.c_void_p(ws.data_ptr()), nbytes, C.c_void_p(out_v.data_ptr()), C.c_void_p(out_i.data_ptr()), st))
+    if squeeze:
+        return out_v[0], out_i[0]
+    return out_v, out_i
