@@ -9,6 +9,8 @@ import ctypes as C
 import os
 import threading
 
+import torch
+
 from . import build as _build
 
 ABI_VERSION = 15
@@ -140,6 +142,15 @@ def check(code: int) -> None:
     if code != 0:
         msg = load().rnf_last_error()
         raise RnfError(code, msg.decode() if msg else "?")
+
+
+def launch(name: str, device, *args) -> None:
+    """Calls the streamed entry point ``name`` on ``device``: tensors become their data pointers (None a null pointer), other
+    arguments pass through, the device's current stream goes last, and the return code is checked."""
+    fn = getattr(load(), name)
+    with torch.cuda.device(device):
+        ptrs = [C.c_void_p(a.data_ptr()) if isinstance(a, torch.Tensor) else a for a in args]
+        check(fn(*ptrs, C.c_void_p(torch.cuda.current_stream(device).cuda_stream)))
 
 
 def exported_symbols() -> list[str]:

@@ -6,30 +6,6 @@
 
 #include "rnf_common.cuh"
 
-namespace {
-
-thread_local char g_err[512] = "";
-
-int fail(int code, const char* fmt, ...) {
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(g_err, sizeof(g_err), fmt, ap);
-  va_end(ap);
-  return code;
-}
-
-int cuda_fail(cudaError_t e, const char* what) {
-  snprintf(g_err, sizeof(g_err), "%s: %s (%s)", what, cudaGetErrorName(e), cudaGetErrorString(e));
-  return (int)e;
-}
-
-long long* g_trace = nullptr;
-unsigned long long* g_probe_counter = nullptr;
-
-bool valid_mode(int m) { return m == RNF_MLP_FP32 || m == RNF_MLP_TC || m == RNF_MLP_TC_ROW; }
-
-}  // namespace
-
 namespace rnf {
 cudaError_t launch_flow_row(const FlowArgs& a, bool inverse, int sm_count, cudaStream_t st);
 cudaError_t launch_flow_t4(const FlowArgs& a, int sm_count, cudaStream_t st);
@@ -55,6 +31,112 @@ int64_t topk_workspace_bytes(int64_t B, int64_t C, int K);
 cudaError_t launch_topk(const float* values, const int64_t* index, int64_t B, int64_t C, int K, void* workspace, float* v_out,
                         int64_t* i_out, cudaStream_t st);
 }  // namespace rnf
+
+namespace {
+
+thread_local char g_err[512] = "";
+
+int fail(int code, const char* fmt, ...) {
+  va_list ap;
+  va_start(ap, fmt);
+  vsnprintf(g_err, sizeof(g_err), fmt, ap);
+  va_end(ap);
+  return code;
+}
+
+int cuda_fail(cudaError_t e, const char* what) {
+  snprintf(g_err, sizeof(g_err), "%s: %s (%s)", what, cudaGetErrorName(e), cudaGetErrorString(e));
+  return (int)e;
+}
+
+long long* g_trace = nullptr;
+unsigned long long* g_probe_counter = nullptr;
+
+bool valid_mode(int m) { return m == RNF_MLP_FP32 || m == RNF_MLP_TC || m == RNF_MLP_TC_ROW; }
+
+// rows reach their image through feat_index, or image-major at rows_per_image rows per image: N rows must fit in B images
+int row_map_ok(const char* who, int64_t N, int64_t B, const int32_t* feat_index, int64_t rows_per_image) {
+  if (feat_index) return RNF_OK;
+  if (rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
+  if ((N + rows_per_image - 1) / rows_per_image > B)
+    return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N, (long long)rows_per_image,
+                (long long)B);
+  return RNF_OK;
+}
+
+// the gradient kernels (csrc/flow_grad.cu) run Mobius layers of kK components and quaternion affine layers only
+int gradient_stack_ok(const rnf_flow* f, const char* who) {
+  if (f->model.K != rnf::kK) return fail(RNF_ESHAPE, "%s: the kernel is built for segments=%d (got K=%d)", who, rnf::kK, f->model.K);
+  for (int i = 0; i < f->model.n_layers; ++i) {
+    const int k = f->layers_host[i].kind;
+    if (k != RNF_LAYER_MOBIUS && k != RNF_LAYER_AFFINE)
+      return fail(RNF_ESHAPE, "%s: layer %d is an ablation layer (kind %d), which has no gradient here", who, i, k);
+  }
+  return RNF_OK;
+}
+
+// the fields of a launch of the flow kernels that every entry point sets the same way
+rnf::FlowArgs flow_args(const rnf_flow* f, const float* R_in, int64_t N, const float* cond) {
+  rnf::FlowArgs a;
+  memset(&a, 0, sizeof(a));
+  a.weights = f->weights_dev;
+  a.layers = f->layers_dev;
+  a.n_layers = f->model.n_layers;
+  a.n_mobius_slots = f->model.n_mobius_slots;
+  a.R_in = R_in;
+  a.N = N;
+  a.cond = f->cond_floats > 0 ? cond : nullptr;
+  a.cond_stride = f->cond_floats;
+  a.rows_per_image = 1;
+  a.trace = g_trace;
+  a.probe_counter = g_probe_counter;
+  return a;
+}
+
+// Tiles and kernel of an mlp_mode: 128-row tiles on the tensor cores, kV1Threads rows in FP32.  A grid launch (a.G > 0) tiles each
+// of its B images separately.  RNF_MLP_TC runs four tiles per SM in the forward direction (flow_t4.cu); the bisection of the
+// inverse needs its prepared parameters resident in tensor memory and runs in the two-tile kernel (flow_row.cu), as does everything
+// in RNF_MLP_TC_ROW.
+int launch_flow(const rnf_flow* f, rnf::FlowArgs& a, int64_t B, bool inverse, int mlp_mode, void* stream, const char* who) {
+  if (mlp_mode != RNF_MLP_FP32 && !rnf::flow_tc_supported(f))
+    return fail(RNF_ESTATE, "%s: model was packed without the tensor-core weight image", who);
+  const int64_t tile = mlp_mode == RNF_MLP_FP32 ? rnf::kV1Threads : 128;
+  if (a.G > 0) {
+    a.tiles_per_image = (a.G + tile - 1) / tile;
+    a.n_tiles = a.tiles_per_image * B;
+  } else {
+    a.n_tiles = (a.N + tile - 1) / tile;
+  }
+  cudaError_t e;
+  if (mlp_mode == RNF_MLP_FP32) e = rnf::launch_flow_v1(a, inverse, f->sm_count, (cudaStream_t)stream);
+  else if (mlp_mode == RNF_MLP_TC && !inverse) e = rnf::launch_flow_t4(a, f->sm_count, (cudaStream_t)stream);
+  else e = rnf::launch_flow_row(a, inverse, f->sm_count, (cudaStream_t)stream);
+  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+}
+
+int modes_count_ok(const char* who, int M) { return M < 1 || M > 256 ? fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M) : RNF_OK; }
+
+// The checks of num_modes and the two angles, and the thresholds the kernels test, |q_g . q_c| > cos(theta / 2) and
+// >= cos(rho / 2), in double and rounded once: the single-GPU and the sharded calls get them here, so they test the same floats.
+int modes_thresholds(const char* who, int M, float min_separation, float neighbour_radius, float* cos_sep, float* cos_nb) {
+  const int rc = modes_count_ok(who, M);
+  if (rc != RNF_OK) return rc;
+  const float pi = 3.14159265358979323846f;
+  if (!(neighbour_radius > 0.f) || !(neighbour_radius <= min_separation) || !(min_separation <= pi))
+    return fail(RNF_EINVAL, "%s: need 0 < neighbour_radius <= min_separation <= pi (got %g, %g)", who, (double)neighbour_radius,
+                (double)min_separation);
+  *cos_sep = (float)cos(0.5 * (double)min_separation);
+  *cos_nb = (float)cos(0.5 * (double)neighbour_radius);
+  return RNF_OK;
+}
+
+int modes_slices_ok(const char* who, const char* name, int64_t G) {
+  if (rnf::modes_slices(G) > 65535)
+    return fail(RNF_EINVAL, "%s: %s=%lld rotations exceed the 65535 x 4096 points of one launch", who, name, (long long)G);
+  return RNF_OK;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -104,7 +186,7 @@ int rnf_flow_create(const rnf_model_desc* model, const rnf_layer_desc* layers, c
   if (model->K != rnf::kK || model->H != rnf::kH)
     return fail(RNF_ESHAPE, "rnf_flow_create: kernels are built for segments=64, hidden=64 (got K=%d H=%d)", model->K, model->H);
   if (model->n_floats > 0 && !weights_dev) return fail(RNF_EINVAL, "rnf_flow_create: null weights");
-  int n_mob = 0, n_aff = 0;
+  int n_mob = 0, n_aff = 0, total_mobius = 0;
   for (int i = 0; i < model->n_layers; ++i) {
     const rnf_layer_desc& L = layers[i];
     if (L.kind < RNF_LAYER_MOBIUS || L.kind > RNF_LAYER_RIGHT9) return fail(RNF_EINVAL, "layer %d: bad kind %d", i, L.kind);
@@ -115,13 +197,10 @@ int rnf_flow_create(const rnf_model_desc* model, const rnf_layer_desc* layers, c
       if (L.kind == RNF_LAYER_MOBIUS) { if (L.cond_slot != n_mob++) return fail(RNF_EINVAL, "layer %d: Mobius slots must be consecutive", i); }
       else { if (L.cond_slot != n_aff++) return fail(RNF_EINVAL, "layer %d: affine slots must be consecutive", i); }
     }
+    total_mobius += L.kind == RNF_LAYER_MOBIUS;
   }
-  {
-    int total_mobius = 0;
-    for (int i = 0; i < model->n_layers; ++i) total_mobius += layers[i].kind == RNF_LAYER_MOBIUS;
-    if (total_mobius > 64)
-      return fail(RNF_ESHAPE, "rnf_flow_create: %d Mobius layers; the kernels keep their weight-offset table in 64 shared-memory slots", total_mobius);
-  }
+  if (total_mobius > 64)
+    return fail(RNF_ESHAPE, "rnf_flow_create: %d Mobius layers; the kernels keep their weight-offset table in 64 shared-memory slots", total_mobius);
   if (n_mob != model->n_mobius_slots || n_aff != model->n_affine_slots)
     return fail(RNF_EINVAL, "slot counts (%d,%d) do not match the layer table (%d,%d)", model->n_mobius_slots,
                 model->n_affine_slots, n_mob, n_aff);
@@ -211,44 +290,17 @@ static int run_rows(rnf_flow* f, bool inverse, const float* R_in, int64_t N, con
   if (!R_in || !R_out || !ldj_out) return fail(RNF_EINVAL, "%s: null buffer", who);
   if (f->cond_floats > 0) {
     if (!cond || B <= 0) return fail(RNF_ESTATE, "%s: conditional flow needs the output of rnf_flow_condition", who);
-    if (!feat_index && rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
-    if (!feat_index && (N + rows_per_image - 1) / rows_per_image > B)
-      return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N,
-                  (long long)rows_per_image, (long long)B);
-  } else {
-    cond = nullptr;
+    const int rc = row_map_ok(who, N, B, feat_index, rows_per_image);
+    if (rc != RNF_OK) return rc;
   }
   if (inverse && !scratch) return fail(RNF_EINVAL, "%s: null scratch", who);
-  rnf::FlowArgs a;
-  memset(&a, 0, sizeof(a));
-  a.weights = f->weights_dev;
-  a.layers = f->layers_dev;
-  a.n_layers = f->model.n_layers;
-  a.n_mobius_slots = f->model.n_mobius_slots;
-  a.R_in = R_in;
-  a.N = N;
-  a.cond = cond;
-  a.cond_stride = f->cond_floats;
+  rnf::FlowArgs a = flow_args(f, R_in, N, cond);
   a.feat_index = feat_index;
   a.rows_per_image = rows_per_image > 0 ? rows_per_image : 1;
   a.R_out = R_out;
   a.ldj_out = ldj_out;
   a.scratch = scratch;
-  a.trace = g_trace;
-  a.probe_counter = g_probe_counter;
-  cudaError_t e;
-  if (mlp_mode != RNF_MLP_FP32) {
-    if (!rnf::flow_tc_supported(f)) return fail(RNF_ESTATE, "%s: model was packed without the tensor-core weight image", who);
-    a.n_tiles = (N + 127) / 128;
-    // RNF_MLP_TC: four tiles per SM in the forward direction (flow_t4.cu); the bisection of the inverse needs its prepared
-    // parameters resident in tensor memory and runs in the two-tile kernel (flow_row.cu), as does everything in RNF_MLP_TC_ROW
-    if (mlp_mode == RNF_MLP_TC && !inverse) e = rnf::launch_flow_t4(a, f->sm_count, (cudaStream_t)stream);
-    else e = rnf::launch_flow_row(a, inverse, f->sm_count, (cudaStream_t)stream);
-  } else {
-    a.n_tiles = (N + rnf::kV1Threads - 1) / rnf::kV1Threads;
-    e = rnf::launch_flow_v1(a, inverse, f->sm_count, (cudaStream_t)stream);
-  }
-  return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
+  return launch_flow(f, a, 1, inverse, mlp_mode, stream, who);
 }
 
 int rnf_flow_forward(rnf_flow* f, const float* R_in, int64_t N, const float* cond, int64_t B, const int32_t* feat_index,
@@ -275,48 +327,33 @@ int rnf_flow_logprob_grad(rnf_flow* f, const float* R_in, int64_t N, const float
   if (!f) return fail(RNF_EINVAL, "%s: null handle", who);
   if (N < 0) return fail(RNF_EINVAL, "%s: negative N", who);
   if ((fisher_A == nullptr) != (fisher_c == nullptr)) return fail(RNF_EINVAL, "%s: fisher_A and fisher_c must be given together", who);
-  if (f->model.K != rnf::kK) return fail(RNF_ESHAPE, "%s: the kernel is built for segments=%d (got K=%d)", who, rnf::kK, f->model.K);
-  for (int i = 0; i < f->model.n_layers; ++i) {
-    const int k = f->layers_host[i].kind;
-    if (k != RNF_LAYER_MOBIUS && k != RNF_LAYER_AFFINE)
-      return fail(RNF_ESHAPE, "%s: layer %d is an ablation layer (kind %d), which has no rotation gradient here", who, i, k);
-  }
-  if (N == 0) return RNF_OK;
+  int rc = gradient_stack_ok(f, who);
+  if (rc != RNF_OK || N == 0) return rc;
   if (!R_in || !logp_out || !grad_out) return fail(RNF_EINVAL, "%s: null buffer", who);
   const bool per_image = f->cond_floats > 0 || fisher_A != nullptr;
   if (f->cond_floats > 0 && !cond) return fail(RNF_ESTATE, "%s: conditional flow needs the output of rnf_flow_condition", who);
   if (per_image) {
     if (B <= 0) return fail(RNF_EINVAL, "%s: B must be > 0 for a conditional flow or a Fisher base term", who);
-    if (!feat_index && rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
-    if (!feat_index && (N + rows_per_image - 1) / rows_per_image > B)
-      return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N, (long long)rows_per_image,
-                  (long long)B);
+    rc = row_map_ok(who, N, B, feat_index, rows_per_image);
+    if (rc != RNF_OK) return rc;
   }
   cudaError_t e = rnf::launch_flow_grad(f, R_in, N, cond, per_image ? feat_index : nullptr, per_image ? rows_per_image : 1, fisher_A,
                                         fisher_c, logp_out, grad_out, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
 }
 
-// shared argument checks of the training entry points (those of rnf_flow_logprob_grad, plus the weights pointer)
+// shared argument checks of the training entry points
 static int check_train_args(const rnf_flow* f, const char* who, const float* weights, const float* R_in, int64_t N, const float* cond,
                             int64_t B, const int32_t* feat_index, int64_t rows_per_image) {
   if (!f) return fail(RNF_EINVAL, "%s: null handle", who);
   if (N < 0) return fail(RNF_EINVAL, "%s: negative N", who);
-  if (f->model.K != rnf::kK) return fail(RNF_ESHAPE, "%s: the kernel is built for segments=%d (got K=%d)", who, rnf::kK, f->model.K);
-  for (int i = 0; i < f->model.n_layers; ++i) {
-    const int k = f->layers_host[i].kind;
-    if (k != RNF_LAYER_MOBIUS && k != RNF_LAYER_AFFINE)
-      return fail(RNF_ESHAPE, "%s: layer %d is an ablation layer (kind %d), which has no gradient here", who, i, k);
-  }
-  if (N == 0) return RNF_OK;
+  const int rc = gradient_stack_ok(f, who);
+  if (rc != RNF_OK || N == 0) return rc;
   if (!weights || !R_in) return fail(RNF_EINVAL, "%s: null buffer", who);
   if (f->cond_floats > 0) {
     if (!cond) return fail(RNF_ESTATE, "%s: conditional flow needs its per-image constants", who);
     if (B <= 0) return fail(RNF_EINVAL, "%s: B must be > 0 for a conditional flow", who);
-    if (!feat_index && rows_per_image <= 0) return fail(RNF_EINVAL, "%s: need feat_index or rows_per_image > 0", who);
-    if (!feat_index && (N + rows_per_image - 1) / rows_per_image > B)
-      return fail(RNF_EINVAL, "%s: N=%lld rows at %lld rows/image exceed B=%lld images", who, (long long)N, (long long)rows_per_image,
-                  (long long)B);
+    return row_map_ok(who, N, B, feat_index, rows_per_image);
   }
   return RNF_OK;
 }
@@ -379,17 +416,7 @@ int rnf_grid_logprob_spread(rnf_flow* f, const float* grid_dev, int64_t G, int64
   if (f->cond_floats > 0 && !cond_dev) return fail(RNF_ESTATE, "rnf_grid_logprob: conditional flow needs rnf_flow_condition output");
   if ((gt_dev == nullptr) != (spread_num_out_dev == nullptr) || (gt_dev != nullptr && gt_k <= 0))
     return fail(RNF_EINVAL, "rnf_grid_logprob_spread: gt [B,K,3,3] (K >= 1) and spread_num_out go together");
-  rnf::FlowArgs a;
-  memset(&a, 0, sizeof(a));
-  a.weights = f->weights_dev;
-  a.layers = f->layers_dev;
-  a.n_layers = f->model.n_layers;
-  a.n_mobius_slots = f->model.n_mobius_slots;
-  a.R_in = grid_dev;
-  a.N = G * B;
-  a.cond = f->cond_floats > 0 ? cond_dev : nullptr;
-  a.cond_stride = f->cond_floats;
-  a.rows_per_image = 1;
+  rnf::FlowArgs a = flow_args(f, grid_dev, G * B, cond_dev);
   a.G = G;
   a.g_index0 = g_index0;
   a.offset = offset_dev;
@@ -399,22 +426,9 @@ int rnf_grid_logprob_spread(rnf_flow* f, const float* grid_dev, int64_t G, int64
   a.part = part_dev;
   a.gt = gt_dev;
   a.gt_k = gt_k;
-  a.trace = g_trace;
-  a.probe_counter = g_probe_counter;
-  cudaError_t e;
-  if (mlp_mode != RNF_MLP_FP32) {
-    if (!rnf::flow_tc_supported(f)) return fail(RNF_ESTATE, "rnf_grid_logprob: model was packed without the tensor-core weight image");
-    a.tiles_per_image = (G + 127) / 128;
-    a.n_tiles = a.tiles_per_image * B;
-    if (mlp_mode == RNF_MLP_TC) e = rnf::launch_flow_t4(a, f->sm_count, (cudaStream_t)stream);
-    else e = rnf::launch_flow_row(a, false, f->sm_count, (cudaStream_t)stream);
-  } else {
-    a.tiles_per_image = (G + rnf::kV1Threads - 1) / rnf::kV1Threads;
-    a.n_tiles = a.tiles_per_image * B;
-    e = rnf::launch_flow_v1(a, false, f->sm_count, (cudaStream_t)stream);
-  }
-  if (e != cudaSuccess) return cuda_fail(e, "rnf_grid_logprob");
-  e = rnf::launch_grid_combine(part_dev, a.tiles_per_image, B, g_index0, max_out_dev, argmax_out_dev, sumexp_out_dev,
+  const int rc = launch_flow(f, a, B, false, mlp_mode, stream, "rnf_grid_logprob");
+  if (rc != RNF_OK) return rc;
+  cudaError_t e = rnf::launch_grid_combine(part_dev, a.tiles_per_image, B, g_index0, max_out_dev, argmax_out_dev, sumexp_out_dev,
                                spread_num_out_dev, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, "rnf_grid_logprob (combine)");
 }
@@ -539,34 +553,18 @@ int rnf_rotation_modes(const float* values, int64_t B, int64_t G, int64_t g_inde
   // no input (the buffers of empty tensors may be null)
   const char* who = "rnf_rotation_modes";
   if (B < 0 || G < 0) return fail(RNF_EINVAL, "%s: negative size", who);
-  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
-  const float pi = 3.14159265358979323846f;
-  if (!(neighbour_radius > 0.f) || !(neighbour_radius <= min_separation) || !(min_separation <= pi))
-    return fail(RNF_EINVAL, "%s: need 0 < neighbour_radius <= min_separation <= pi (got %g, %g)", who, (double)neighbour_radius,
-                (double)min_separation);
-  if (rnf::modes_slices(G) > 65535) return fail(RNF_EINVAL, "%s: G=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G);
-  if (B == 0) return RNF_OK;
+  float cos_sep, cos_nb;
+  int rc = modes_thresholds(who, M, min_separation, neighbour_radius, &cos_sep, &cos_nb);
+  if (rc == RNF_OK) rc = modes_slices_ok(who, "G", G);
+  if (rc != RNF_OK || B == 0) return rc;
   if (!workspace || !index_out || !value_out || !local_max_out || !mass_out || !count_out || (G > 0 && (!values || !rot)))
     return fail(RNF_EINVAL, "%s: null pointer", who);
   if (workspace_bytes < rnf_rotation_modes_workspace_bytes(G, B, M)) return fail(RNF_EINVAL, "%s: workspace too small", who);
-  const int rc = rnf_device_check(nullptr);
+  rc = rnf_device_check(nullptr);
   if (rc != RNF_OK) return rc;
-  // the thresholds in double, rounded once: |q_g . q_c| > cos(theta / 2) and >= cos(rho / 2)
-  const float cos_sep = (float)cos(0.5 * (double)min_separation), cos_nb = (float)cos(0.5 * (double)neighbour_radius);
   cudaError_t e = rnf::launch_rotation_modes(values, B, G, g_index0, rot, M, cos_sep, cos_nb, workspace, index_out, value_out, local_max_out,
                                              mass_out, count_out, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
-}
-
-
-// the thresholds of rnf_rotation_modes and its argument checks (the same expressions, so the shards test the same floats)
-static int modes_thresholds_ok(const char* who, int M, float min_separation, float neighbour_radius) {
-  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
-  const float pi = 3.14159265358979323846f;
-  if (!(neighbour_radius > 0.f) || !(neighbour_radius <= min_separation) || !(min_separation <= pi))
-    return fail(RNF_EINVAL, "%s: need 0 < neighbour_radius <= min_separation <= pi (got %g, %g)", who, (double)neighbour_radius,
-                (double)min_separation);
-  return RNF_OK;
 }
 
 int64_t rnf_rotation_modes_shard_workspace_bytes(int64_t G_r, int64_t B) {
@@ -577,11 +575,11 @@ int64_t rnf_rotation_modes_shard_workspace_bytes(int64_t G_r, int64_t B) {
 int rnf_rotation_modes_shard_setup(const float* rot, int64_t G_r, int64_t B, void* workspace, int64_t workspace_bytes, void* stream) {
   const char* who = "rnf_rotation_modes_shard_setup";
   if (B < 0 || G_r < 0) return fail(RNF_EINVAL, "%s: negative size", who);
-  if (rnf::modes_slices(G_r) > 65535) return fail(RNF_EINVAL, "%s: G_r=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G_r);
-  if (B == 0 || G_r == 0) return RNF_OK;
+  int rc = modes_slices_ok(who, "G_r", G_r);
+  if (rc != RNF_OK || B == 0 || G_r == 0) return rc;
   if (!rot || !workspace) return fail(RNF_EINVAL, "%s: null pointer", who);
   if (workspace_bytes < rnf_rotation_modes_shard_workspace_bytes(G_r, B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
-  const int rc = rnf_device_check(nullptr);
+  rc = rnf_device_check(nullptr);
   if (rc != RNF_OK) return rc;
   cudaError_t e = rnf::launch_modes_shard_setup(rot, G_r, B, workspace, (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
@@ -593,17 +591,17 @@ int rnf_rotation_modes_shard_round(const float* values, int64_t B, int64_t G_r, 
   const char* who = "rnf_rotation_modes_shard_round";
   if (B < 0 || G_r < 0) return fail(RNF_EINVAL, "%s: negative size", who);
   if (g_index0 < 0) return fail(RNF_EINVAL, "%s: negative g_index0", who);
-  int rc = modes_thresholds_ok(who, M, min_separation, neighbour_radius);
+  float cos_sep, cos_nb;
+  int rc = modes_thresholds(who, M, min_separation, neighbour_radius, &cos_sep, &cos_nb);
   if (rc != RNF_OK) return rc;
   if (r < 0 || r > M) return fail(RNF_EINVAL, "%s: round %d outside 0..M=%d", who, r, M);
-  if (rnf::modes_slices(G_r) > 65535) return fail(RNF_EINVAL, "%s: G_r=%lld rotations exceed the 65535 x 4096 points of one launch", who, (long long)G_r);
-  if (B == 0) return RNF_OK;
+  rc = modes_slices_ok(who, "G_r", G_r);
+  if (rc != RNF_OK || B == 0) return rc;
   if (!workspace || !record_out || (G_r > 0 && (!values || !rot))) return fail(RNF_EINVAL, "%s: null pointer", who);
   if (((uintptr_t)record_out & 15) != 0) return fail(RNF_EINVAL, "%s: record buffer not 16-byte aligned", who);
   if (workspace_bytes < rnf_rotation_modes_shard_workspace_bytes(G_r, B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
   rc = rnf_device_check(nullptr);
   if (rc != RNF_OK) return rc;
-  const float cos_sep = (float)cos(0.5 * (double)min_separation), cos_nb = (float)cos(0.5 * (double)neighbour_radius);
   cudaError_t e = rnf::launch_modes_shard_round(values, B, G_r, g_index0, rot, r, M, cos_sep, cos_nb, workspace, record_out,
                                                 (cudaStream_t)stream);
   return e == cudaSuccess ? RNF_OK : cuda_fail(e, who);
@@ -615,14 +613,15 @@ int rnf_rotation_modes_shard_merge(const void* records, int W, int64_t B, int r,
   const char* who = "rnf_rotation_modes_shard_merge";
   if (B < 0) return fail(RNF_EINVAL, "%s: negative size", who);
   if (W < 1) return fail(RNF_EINVAL, "%s: W=%d ranks, need at least 1", who, W);
-  if (M < 1 || M > 256) return fail(RNF_EINVAL, "%s: M=%d modes outside 1..256", who, M);
+  int rc = modes_count_ok(who, M);
+  if (rc != RNF_OK) return rc;
   if (r < 0 || r > M) return fail(RNF_EINVAL, "%s: round %d outside 0..M=%d", who, r, M);
   if (B == 0) return RNF_OK;
   if (!records || !workspace || !index_out || !value_out || !local_max_out || !mass_out || !count_out || !rot_out)
     return fail(RNF_EINVAL, "%s: null pointer", who);
   if (((uintptr_t)records & 15) != 0) return fail(RNF_EINVAL, "%s: record buffer not 16-byte aligned", who);
   if (workspace_bytes < rnf::modes_shard_state_bytes(B)) return fail(RNF_EINVAL, "%s: workspace too small", who);
-  const int rc = rnf_device_check(nullptr);
+  rc = rnf_device_check(nullptr);
   if (rc != RNF_OK) return rc;
   cudaError_t e = rnf::launch_modes_shard_merge(records, W, B, r, M, workspace, index_out, value_out, local_max_out, mass_out, count_out,
                                                 rot_out, (cudaStream_t)stream);

@@ -17,7 +17,7 @@ import math
 import torch
 import torch.distributed as dist
 
-from .modes import RECORD_BYTES, rotation_modes_rank
+from .modes import rotation_modes_rank
 
 
 def shard_range(G: int, rank: int, world: int) -> tuple[int, int]:
@@ -45,16 +45,26 @@ def merge_partials(mx: torch.Tensor, am: torch.Tensor, se: torch.Tensor, sn: tor
     return m, idx, s.to(se.dtype)
 
 
+def _world_size(group) -> int:
+    return dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
+
+
+def _gather(t: torch.Tensor, group) -> torch.Tensor:
+    """[n, ...] -> [W, n, ...], rank-major: one all_gather_into_tensor (the identity on one rank)."""
+    world = _world_size(group)
+    if world == 1:
+        return t[None]
+    flat = torch.empty((world * t.shape[0],) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+    dist.all_gather_into_tensor(flat, t.contiguous(), group=group)
+    return flat.view(world, *t.shape)
+
+
 def all_merge(mx: torch.Tensor, am: torch.Tensor, se: torch.Tensor, group=None, sn: torch.Tensor | None = None):
     """One all-gather of the packed partials ([B,3] float64, [B,4] with spread numerators), then ``merge_partials`` on every rank."""
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+    if _world_size(group) == 1:
         return (mx, am, se) if sn is None else (mx, am, se, sn)
-    world = dist.get_world_size(group)
     cols = [mx.double(), am.double(), se.double()] + ([] if sn is None else [sn.double()])   # indices < 2^53 are exact
-    packed = torch.stack(cols, dim=1).contiguous()
-    flat = torch.empty((world * packed.shape[0], len(cols)), dtype=packed.dtype, device=packed.device)
-    dist.all_gather_into_tensor(flat, packed, group=group)                                  # rank-major concatenation
-    gathered = flat.view(world, packed.shape[0], len(cols))
+    gathered = _gather(torch.stack(cols, dim=1), group)
     return merge_partials(gathered[:, :, 0].to(mx.dtype), gathered[:, :, 1].to(torch.int64), gathered[:, :, 2].to(se.dtype),
                           None if sn is None else gathered[:, :, 3].to(sn.dtype))
 
@@ -78,15 +88,7 @@ def sharded_grid_log_prob(flow, grid_shard: torch.Tensor, g_index0: int, G_total
 
 def _record_gather(group):
     """[B, RECORD_BYTES] -> [W, B, RECORD_BYTES], rank-major: one all_gather_into_tensor (the identity on one rank)."""
-    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
-        return lambda rec: rec[None]
-    world = dist.get_world_size(group)
-
-    def gather(rec):
-        flat = torch.empty((world * rec.shape[0], RECORD_BYTES), dtype=rec.dtype, device=rec.device)
-        dist.all_gather_into_tensor(flat, rec.contiguous(), group=group)
-        return flat.view(world, rec.shape[0], RECORD_BYTES)
-    return gather
+    return lambda rec: _gather(rec, group)
 
 
 def sharded_rotation_modes(values_shard: torch.Tensor, grid_shard: torch.Tensor, g_index0: int, G_total: int, num_modes: int,
@@ -117,44 +119,16 @@ def sharded_estimate_rotation_modes(flow, grid_shard: torch.Tensor, g_index0: in
     chunking depends on G_total and the world size only, so all ranks make the same collectives."""
     from . import evalpath
     from . import grid as rgrid
-    level = rgrid.closest_grid_level(G_total)
-    rho = evalpath.default_neighbour_radius(level) if neighbour_radius is None else float(neighbour_radius)
-    if float(min_separation) < rho:
-        raise ValueError(f"min_separation={min_separation} is below neighbour_radius={rho}: a mode's neighbourhood would reach past its "
-                         "own ball")
-    if refine_steps > 0 and refine_lr is None:
-        raise ValueError("refine_steps > 0 needs refine_lr")
+    rho = evalpath._modes_radius(rgrid.closest_grid_level(G_total), min_separation, neighbour_radius, refine_steps, refine_lr)
     dev = grid_shard.device
-    world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
-    G_r, M = grid_shard.shape[0], int(num_modes)
-    B = feature.shape[0] if (feature is not None and flow.condition) else 1
-    chunk = max(1, evalpath.MODES_LOGP_BYTES // (-(-G_total // world) * 4))
+    G_r = grid_shard.shape[0]
     off = None if offset is None else offset.to(dev, torch.float32)
     parts = []
-    for s in range(0, B, chunk):
-        f = feature[s:s + chunk] if (feature is not None and flow.condition) else feature
-        A = fisher_A[s:s + chunk] if fisher_A is not None else None
+    for f, A, n in evalpath._image_chunks(flow, feature, fisher_A, -(-G_total // _world_size(group))):
         if G_r > 0:
             lp = flow.grid_log_prob(grid_shard, f, offset=off, fisher_A=A, return_logp=True, g_index0=g_index0)["logp"]
         else:
-            lp = torch.empty((min(chunk, B - s), 0), device=dev, dtype=torch.float32)
-        parts.append(sharded_rotation_modes(lp, grid_shard, g_index0, G_total, M, min_separation, rho, group))
+            lp = torch.empty((n, 0), device=dev, dtype=torch.float32)
+        parts.append(sharded_rotation_modes(lp, grid_shard, g_index0, G_total, int(num_modes), min_separation, rho, group))
     md = {k: torch.cat([p[k] for p in parts]) for k in ("index", "value", "local_max", "mass", "rotations")}
-    # what evalpath.estimate_rotation_modes does after rotation_modes, with the grid rows taken from the records
-    valid = md["local_max"]
-    order = torch.sort((~valid).to(torch.int8), dim=1, stable=True).indices
-    valid = torch.gather(valid, 1, order)
-    index = torch.where(valid, torch.gather(md["index"], 1, order), -1)
-    logp = torch.where(valid, torch.gather(md["value"], 1, order), -math.inf)
-    mass = torch.where(valid, torch.gather(md["mass"], 1, order), 0.0)
-    rows = torch.gather(md["rotations"], 1, order[..., None, None].expand(-1, -1, 3, 3))
-    rot = torch.where(valid[..., None, None], rows, md["rotations"][:, :1])          # padding: mode 0's row (a real rotation)
-    if off is not None:
-        rot = rot @ off
-    if refine_steps > 0:
-        mode0 = md["rotations"][:, 0] if off is None else md["rotations"][:, 0] @ off
-        seeds = torch.where(valid[..., None, None], rot, mode0[:, None])              # padding: mode 0 of the grid
-        rot, lp = evalpath.refine_rotation(flow, feature, seeds, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
-        rot, logp, mass, valid, index = evalpath._merge_modes(rot, torch.where(valid, lp, -math.inf), mass, valid, index, rho)
-    rot = torch.where(valid[..., None, None], rot, math.nan)
-    return rot, dict(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)
+    return evalpath._finish_modes(flow, feature, fisher_A, md, md["rotations"], off, rho, refine_steps, refine_lr)

@@ -67,25 +67,14 @@ def _last_layer_perm_pairs(K: int) -> np.ndarray:
 
 
 def pack_mobius(cond_sd: dict, F: int) -> tuple[np.ndarray, np.ndarray | None]:
-    """ConditionalTransform(3+F, 4K) -> (FP32 kernel image [MOB_FLOATS], W_f [64,F] or None)."""
-    W0, b0 = _np(cond_sd["fc_first.weight"]), _np(cond_sd["fc_first.bias"])
+    """ConditionalTransform(3+F, 4K) -> (FP32 kernel image [MOB_FLOATS] (mobius_images), W_f [64,F] or None)."""
+    W0 = _np(cond_sd["fc_first.weight"])
     if W0.shape != (HIDDEN, 3 + F):
         raise ValueError(f"fc_first.weight has shape {W0.shape}, expected {(HIDDEN, 3 + F)}")
-    blk = np.empty(MOB_FLOATS, dtype=np.float32)
-    first = np.concatenate([W0[:, :3], b0[:, None]], axis=1)            # [64][4]
-    o = 0
-    blk[o:o + 256] = first.reshape(-1); o += 256
-    for j in (1, 3, 5):
-        W, b = _np(cond_sd[f"layers.{j}.weight"]), _np(cond_sd[f"layers.{j}.bias"])
-        blk[o:o + 4096] = W.T.reshape(-1); o += 4096                     # [k][j]
-        blk[o:o + 64] = b; o += 64
-    W4, b4 = _np(cond_sd["fc_last.weight"]), _np(cond_sd["fc_last.bias"])
-    if W4.shape != (4 * K_SEGMENTS, HIDDEN):
-        raise ValueError(f"fc_last.weight has shape {W4.shape}; kernels are built for segments={K_SEGMENTS}")
-    perm = _last_layer_perm(K_SEGMENTS)
-    blk[o:o + 64 * 256] = W4[perm].T.reshape(-1); o += 64 * 256          # [k][j']
-    blk[o:o + 256] = b4[perm]; o += 256
-    assert o == MOB_FLOATS
+    W4_shape = tuple(cond_sd["fc_last.weight"].shape)
+    if W4_shape != (4 * K_SEGMENTS, HIDDEN):
+        raise ValueError(f"fc_last.weight has shape {W4_shape}; kernels are built for segments={K_SEGMENTS}")
+    blk = mobius_images([{k: t.detach().to("cpu", torch.float32) for k, t in cond_sd.items()}])[0].numpy()
     return blk, (np.ascontiguousarray(W0[:, 3:]) if F > 0 else None)
 
 
@@ -395,9 +384,6 @@ class Program:
             self.handle = None
 
     # ------------------------------------------------------------------------------------------
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
-
     def condition(self, feat: torch.Tensor) -> torch.Tensor:
         """feat [B,F] -> per-image constants [B, cond_floats] (rnf_flow_condition)."""
         B = feat.shape[0]
@@ -405,9 +391,7 @@ class Program:
         if feat.dim() != 2 or feat.shape[1] != self.F:
             raise ValueError(f"feature must be [B,{self.F}], got {tuple(feat.shape)}")
         cond = torch.empty((B, self.cond_floats), device=self.device, dtype=torch.float32)
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_flow_condition(self.handle, C.c_void_p(feat.data_ptr()), B,
-                                                    C.c_void_p(cond.data_ptr()), self._stream()))
+        _cabi.launch("rnf_flow_condition", self.device, self.handle, feat, B, cond)
         if self.rot_slots:
             self._polar_factor(cond, B)
         if self.ablation_slots:
@@ -451,9 +435,7 @@ class Program:
         # capacity rows beyond the run count are never indexed; for ConditionRot they still go through the batched SVD: keep them 0
         alloc = torch.zeros if self.rot_slots else torch.empty
         cond = alloc((cap, self.cond_floats), device=self.device, dtype=torch.float32)
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_flow_condition_runs(self.handle, C.c_void_p(feat.data_ptr()), C.c_void_p(first.data_ptr()),
-                                                         C.c_void_p(count.data_ptr()), cap, C.c_void_p(cond.data_ptr()), self._stream()))
+        _cabi.launch("rnf_flow_condition_runs", self.device, self.handle, feat, first, count, cap, cond)
         if self.rot_slots:
             self._polar_factor(cond, cap)
         if self.ablation_slots:
@@ -461,8 +443,7 @@ class Program:
         return cond
 
     def poison_if_overflow(self, count: torch.Tensor, cap: int, ldj: torch.Tensor) -> None:
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_poison_if_overflow(C.c_void_p(count.data_ptr()), cap, C.c_void_p(ldj.data_ptr()), ldj.numel(), self._stream()))
+        _cabi.launch("rnf_poison_if_overflow", self.device, count, cap, ldj, ldj.numel())
 
     def run(self, R: torch.Tensor, cond, B: int, feat_index, rows_per_image: int, inverse: bool, mode: str):
         N = R.shape[0]
@@ -470,20 +451,13 @@ class Program:
         ldj = torch.empty((N,), device=self.device, dtype=torch.float32)
         if N == 0:
             return R_out, ldj
-        cp = C.c_void_p(cond.data_ptr()) if cond is not None else None
-        ip = C.c_void_p(feat_index.data_ptr()) if feat_index is not None else None
-        m = _MODES[mode]
-        with torch.cuda.device(self.device):
-            if inverse:
-                ns = int(self.lib.rnf_flow_inverse_scratch_floats(self.handle, N))
-                scratch = torch.empty((max(ns, 1),), device=self.device, dtype=torch.float32)
-                _cabi.check(self.lib.rnf_flow_inverse(self.handle, C.c_void_p(R.data_ptr()), N, cp, B, ip, rows_per_image,
-                                                      C.c_void_p(R_out.data_ptr()), C.c_void_p(ldj.data_ptr()),
-                                                      C.c_void_p(scratch.data_ptr()), m, self._stream()))
-            else:
-                _cabi.check(self.lib.rnf_flow_forward(self.handle, C.c_void_p(R.data_ptr()), N, cp, B, ip, rows_per_image,
-                                                      C.c_void_p(R_out.data_ptr()), C.c_void_p(ldj.data_ptr()), m,
-                                                      self._stream()))
+        if inverse:
+            ns = int(self.lib.rnf_flow_inverse_scratch_floats(self.handle, N))
+            scratch = torch.empty((max(ns, 1),), device=self.device, dtype=torch.float32)
+            _cabi.launch("rnf_flow_inverse", self.device, self.handle, R, N, cond, B, feat_index, rows_per_image, R_out, ldj, scratch,
+                         _MODES[mode])
+        else:
+            _cabi.launch("rnf_flow_forward", self.device, self.handle, R, N, cond, B, feat_index, rows_per_image, R_out, ldj, _MODES[mode])
         return R_out, ldj
 
     def logprob_grad(self, R: torch.Tensor, cond, B: int, feat_index, rows_per_image: int, A9=None, c=None):
@@ -494,10 +468,7 @@ class Program:
         G = torch.empty((N, 3, 3), device=self.device, dtype=torch.float32)
         if N == 0:
             return logp, G
-        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_flow_logprob_grad(self.handle, vp(R), N, vp(cond), B, vp(feat_index), rows_per_image, vp(A9), vp(c),
-                                                       vp(logp), vp(G), self._stream()))
+        _cabi.launch("rnf_flow_logprob_grad", self.device, self.handle, R, N, cond, B, feat_index, rows_per_image, A9, c, logp, G)
         return logp, G
 
     def grid_logprob(self, grid: torch.Tensor, g_index0: int, offset, cond, B: int, fisher_A, fisher_c,
@@ -510,21 +481,13 @@ class Program:
         se = torch.empty((B,), device=dev, dtype=torch.float32)
         logp = torch.empty((B, G), device=dev, dtype=torch.float32) if want_logp else None
         part = torch.empty((max(1, int(self.lib.rnf_grid_partial_floats(G, B))),), device=dev, dtype=torch.float32)
-        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        sn = None
         if gt is not None:
             gt = gt.to(dev, torch.float32).reshape(B, -1, 9).contiguous()
             sn = torch.empty((B,), device=dev, dtype=torch.float32)
-            with torch.cuda.device(dev):
-                _cabi.check(self.lib.rnf_grid_logprob_spread(self.handle, vp(grid), G, int(g_index0), vp(offset), vp(cond), B,
-                                                             vp(fisher_A), vp(fisher_c), vp(gt), int(gt.shape[1]), vp(logp),
-                                                             vp(part), vp(mx), vp(am), vp(se), vp(sn), _MODES[mode],
-                                                             self._stream()))
-            return mx, am, se, logp, sn
-        with torch.cuda.device(dev):
-            _cabi.check(self.lib.rnf_grid_logprob(self.handle, vp(grid), G, int(g_index0), vp(offset), vp(cond), B,
-                                                  vp(fisher_A), vp(fisher_c), vp(logp), vp(part), vp(mx), vp(am), vp(se),
-                                                  _MODES[mode], self._stream()))
-        return mx, am, se, logp
+        _cabi.launch("rnf_grid_logprob_spread", dev, self.handle, grid, G, int(g_index0), offset, cond, B, fisher_A, fisher_c, gt,
+                     0 if gt is None else int(gt.shape[1]), logp, part, mx, am, se, sn, _MODES[mode])
+        return (mx, am, se, logp) if gt is None else (mx, am, se, logp, sn)
 
 
 DEDUP_CAP = 8192      # optimistic image capacity of the sync-free drop-in path (44 MB of per-image constants at most)
@@ -550,10 +513,7 @@ def dedup_rows(feature: torch.Tensor, cap: int):
     count = torch.empty((1,), dtype=torch.int32, device=dev)
     nbytes = int(lib.rnf_dedup_workspace_bytes(N))
     ws = torch.empty((max(nbytes, 1),), dtype=torch.uint8, device=dev)
-    with torch.cuda.device(dev):
-        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _cabi.check(lib.rnf_dedup_rows(C.c_void_p(feature.data_ptr()), N, F, C.c_void_p(idx.data_ptr()), C.c_void_p(first.data_ptr()), cap,
-                                       C.c_void_p(count.data_ptr()), C.c_void_p(ws.data_ptr()), nbytes, st))
+    _cabi.launch("rnf_dedup_rows", dev, feature, N, F, idx, first, cap, count, ws, nbytes)
     return idx, first, count
 
 
@@ -708,18 +668,12 @@ class TrainProgram:
             buf.index_copy_(0, self.image_index, torch.cat(src).detach())
         return buf
 
-    def _call(self, name, *args):
-        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
-        with torch.cuda.device(self.device):
-            _cabi.check(getattr(self.prog.lib, name)(self.prog.handle, *[vp(a) if (a is None or torch.is_tensor(a)) else a for a in args],
-                                                     self.prog._stream()))
-
     def forward(self, weights, R, cond, B: int, idx32):
         N = R.shape[0]
         R_out = torch.empty((N, 3, 3), device=self.device, dtype=torch.float32)
         ldj = torch.empty((N,), device=self.device, dtype=torch.float32)
         if N:
-            self._call("rnf_flow_train_forward", weights, R, N, cond, B, idx32, 0, R_out, ldj)
+            _cabi.launch("rnf_flow_train_forward", self.device, self.prog.handle, weights, R, N, cond, B, idx32, 0, R_out, ldj)
         return R_out, ldj
 
     def backward(self, weights, R, cond, B: int, idx32, G_Rout, g_ldj):
@@ -743,8 +697,8 @@ class TrainProgram:
         for s in range(0, N, chunk):
             n = min(chunk, N - s)
             sl = lambda t: None if t is None else t[s:s + n]
-            self._call("rnf_flow_train_backward", weights, R[s:s + n], n, cond, B, sl(idx32), 0, sl(G_Rout), sl(g_ldj), G_R[s:s + n],
-                       ws, int(ws.numel()))
+            _cabi.launch("rnf_flow_train_backward", dev, self.prog.handle, weights, R[s:s + n], n, cond, B, sl(idx32), 0, sl(G_Rout), sl(g_ldj),
+                         G_R[s:s + n], ws, int(ws.numel()))
             wm = ws[:Lm * n * TF].view(Lm, n, TF)
             wa = ws[Lm * n * TF: Lm * n * TF + La * n * 16].view(La, n, 16)
             if Lm:

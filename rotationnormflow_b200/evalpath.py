@@ -69,6 +69,52 @@ def default_neighbour_radius(level: int) -> float:
     return NEIGHBOUR_RADIUS[-1] / 2 ** (level - len(NEIGHBOUR_RADIUS) + 1)
 
 
+def _modes_radius(level, min_separation, neighbour_radius, refine_steps, refine_lr) -> float:
+    """The checks of the mode-estimation arguments; returns neighbour_radius (default: default_neighbour_radius(level))."""
+    rho = default_neighbour_radius(level) if neighbour_radius is None else float(neighbour_radius)
+    if float(min_separation) < rho:
+        raise ValueError(f"min_separation={min_separation} is below neighbour_radius={rho}: a mode's neighbourhood would reach past its "
+                         "own ball")
+    if refine_steps > 0 and refine_lr is None:
+        raise ValueError("refine_steps > 0 needs refine_lr")
+    return rho
+
+
+def _image_chunks(flow, feature, fisher_A, G):
+    """(feature, fisher_A, images) of consecutive image chunks whose [images, G] float32 log-density stays under MODES_LOGP_BYTES.
+    An unconditional flow is one image, its feature passed on as given."""
+    conditional = feature is not None and flow.condition
+    B = feature.shape[0] if conditional else 1
+    chunk = max(1, MODES_LOGP_BYTES // (G * 4))
+    for s in range(0, B, chunk):
+        yield (feature[s:s + chunk] if conditional else feature, fisher_A[s:s + chunk] if fisher_A is not None else None,
+               min(chunk, B - s))
+
+
+def _finish_modes(flow, feature, fisher_A, md, rows, offset, rho, refine_steps, refine_lr):
+    """What follows ``rotation_modes`` in estimate_rotation_modes and dist.sharded_estimate_rotation_modes.  ``md`` holds index, value,
+    local_max and mass [B,M] of the greedy picks, ``rows`` [B,M,3,3] their rotations before the ``offset`` [3,3] (None: no offset).
+    Drops the shoulders, keeping the greedy order (non-increasing value) of the local maxima; refine_steps > 0 refines all modes and
+    merges those within ``rho``.  Returns (rotations [B,M,3,3], dict(logp, mass, valid, count, grid_index)), padded with NaN, -inf,
+    0 and -1."""
+    valid = md["local_max"]
+    order = torch.sort((~valid).to(torch.int8), dim=1, stable=True).indices
+    valid = torch.gather(valid, 1, order)
+    index = torch.where(valid, torch.gather(md["index"], 1, order), -1)
+    logp = torch.where(valid, torch.gather(md["value"], 1, order), -math.inf)
+    mass = torch.where(valid, torch.gather(md["mass"], 1, order), 0.0)
+    rot = torch.gather(rows, 1, order[..., None, None].expand(-1, -1, 3, 3))
+    if offset is not None:
+        rot = rot @ offset
+    if refine_steps > 0:
+        mode0 = rows[:, 0] if offset is None else rows[:, 0] @ offset
+        seeds = torch.where(valid[..., None, None], rot, mode0[:, None])          # padding: mode 0 of the grid
+        rot, lp = refine_rotation(flow, feature, seeds, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
+        rot, logp, mass, valid, index = _merge_modes(rot, torch.where(valid, lp, -math.inf), mass, valid, index, rho)
+    rot = torch.where(valid[..., None, None], rot, math.nan)
+    return rot, dict(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)
+
+
 @torch.no_grad()
 def estimate_rotation_modes(flow, feature, number_queries, num_modes, *, min_separation, neighbour_radius=None, fisher_A=None, offset=None,
                             generator=None, mlp_mode=None, refine_steps=0, refine_lr=None):
@@ -83,44 +129,21 @@ def estimate_rotation_modes(flow, feature, number_queries, num_modes, *, min_sep
     sumexp [B])): modes sorted by log p (the refined one after refinement), valid ones first; padded entries have NaN rotations, logp
     -inf, mass 0 and grid_index -1.  ``max`` / ``argmax`` / ``sumexp`` are those of ``Flow.grid_log_prob``; mode 0 of the grid pass is
     its arg-max.  The grid is evaluated in image chunks of at most MODES_LOGP_BYTES of log-density."""
-    level = rgrid.closest_grid_level(number_queries)
-    rho = default_neighbour_radius(level) if neighbour_radius is None else float(neighbour_radius)
-    if float(min_separation) < rho:
-        raise ValueError(f"min_separation={min_separation} is below neighbour_radius={rho}: a mode's neighbourhood would reach past its "
-                         "own ball")
-    if refine_steps > 0 and refine_lr is None:
-        raise ValueError("refine_steps > 0 needs refine_lr")
+    rho = _modes_radius(rgrid.closest_grid_level(number_queries), min_separation, neighbour_radius, refine_steps, refine_lr)
     dev = feature.device if feature is not None else torch.device("cuda", torch.cuda.current_device())
     grid = rgrid.get_closest_available_grid(number_queries, dev)
     if offset is None:
         offset = _random_rotation(dev, generator)
     offset = offset.to(dev, torch.float32)
-    G, M = grid.shape[0], int(num_modes)
-    B = feature.shape[0] if (feature is not None and flow.condition) else 1
-    chunk = max(1, MODES_LOGP_BYTES // (G * 4))
     parts = []
-    for s in range(0, B, chunk):
-        f = feature[s:s + chunk] if (feature is not None and flow.condition) else feature
-        A = fisher_A[s:s + chunk] if fisher_A is not None else None
+    for f, A, _ in _image_chunks(flow, feature, fisher_A, grid.shape[0]):
         out = flow.grid_log_prob(grid, f, offset=offset, fisher_A=A, return_logp=True, mlp_mode=mlp_mode)
-        md = rotation_modes(out.pop("logp"), grid, M, min_separation, rho)
+        md = rotation_modes(out.pop("logp"), grid, int(num_modes), min_separation, rho)
         parts.append((out, md))
     out = {k: torch.cat([p[0][k] for p in parts]) for k in ("max", "argmax", "sumexp")}
     md = {k: torch.cat([p[1][k] for p in parts]) for k in ("index", "value", "local_max", "mass")}
-    # drop the shoulders, keeping the greedy order (non-increasing value) of the local maxima
-    valid = md["local_max"]
-    order = torch.sort((~valid).to(torch.int8), dim=1, stable=True).indices
-    valid = torch.gather(valid, 1, order)
-    index = torch.where(valid, torch.gather(md["index"], 1, order), -1)
-    logp = torch.where(valid, torch.gather(md["value"], 1, order), -math.inf)
-    mass = torch.where(valid, torch.gather(md["mass"], 1, order), 0.0)
-    rot = grid[index.clamp(min=0)] @ offset
-    if refine_steps > 0:
-        seeds = torch.where(valid[..., None, None], rot, (grid[md["index"][:, 0]] @ offset)[:, None])   # padding: mode 0 of the grid
-        rot, lp = refine_rotation(flow, feature, seeds, lr=refine_lr, steps=refine_steps, fisher_A=fisher_A)
-        rot, logp, mass, valid, index = _merge_modes(rot, torch.where(valid, lp, -math.inf), mass, valid, index, rho)
-    rot = torch.where(valid[..., None, None], rot, math.nan)
-    out.update(logp=logp, mass=mass, valid=valid, count=valid.sum(1), grid_index=index)
+    rot, modes = _finish_modes(flow, feature, fisher_A, md, grid[md["index"].clamp(min=0)], offset, rho, refine_steps, refine_lr)
+    out.update(modes)
     return rot, out
 
 
@@ -206,15 +229,9 @@ def estimate_rotation_hierarchical(flow, feature, number_queries, *, start_level
     if offset is None:
         offset = _random_rotation(dev, generator)
     offset = offset.to(dev, torch.float32)
-    conditional = feature is not None and flow.condition
-    B = feature.shape[0] if conditional else 1
     G0 = rgrid.GRID_SIZES[l0]
-    chunk = max(1, MODES_LOGP_BYTES // (G0 * 4))
     parts = []
-    for s in range(0, B, chunk):
-        f = feature[s:s + chunk] if conditional else feature
-        A = fisher_A[s:s + chunk] if fisher_A is not None else None
-        nb = min(chunk, B - s)
+    for f, A, nb in _image_chunks(flow, feature, fisher_A, G0):
         if fused:
             grid0 = rgrid.get_closest_available_grid(G0, dev)
             lp = flow.grid_log_prob(grid0, f, offset=offset, fisher_A=A, return_logp=True, mlp_mode=mlp_mode)["logp"]

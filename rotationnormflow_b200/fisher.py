@@ -39,9 +39,7 @@ class MatrixFisherN(torch.nn.Module):
         self._A9, self._c = fisher_constants(A)
 
     def _log_prob(self, inputs, context=9):
-        import ctypes as C
         from . import _cabi
-        lib = _cabi.load()
         if not inputs.is_cuda:
             raise RuntimeError("rotationnormflow_b200 runs on a B200 only: `inputs` must be a CUDA tensor (there is no CPU fallback)")
         if inputs.shape[-1] != 3 or inputs.shape[-2] != 3:
@@ -51,10 +49,7 @@ class MatrixFisherN(torch.nn.Module):
             self._A9, self._c = self._A9.to(dev), self._c.to(dev)
         R = inputs.reshape(-1, 3, 3).to(torch.float32).contiguous()
         out = torch.empty((R.shape[0],), device=dev, dtype=torch.float32)
-        with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _cabi.check(lib.rnf_fisher_log_prob(C.c_void_p(self._A9.data_ptr()), C.c_void_p(self._c.data_ptr()), self._A9.shape[0],
-                                                C.c_void_p(R.data_ptr()), R.shape[0], C.c_void_p(out.data_ptr()), st))
+        _cabi.launch("rnf_fisher_log_prob", dev, self._A9, self._c, self._A9.shape[0], R, R.shape[0], out)
         return out
 
     log_prob = _log_prob
@@ -71,17 +66,13 @@ class MatrixFisherN(torch.nn.Module):
             raise NotImplementedError("quaternion output: convert with matrix_to_quaternion (utils/fisher.py:244-245)")
         if not self.A.is_cuda:
             raise RuntimeError("rotationnormflow_b200 runs on a B200 only: `A` must be a CUDA tensor (there is no CPU fallback)")
-        lib = _cabi.load()
         dev = self.A.device
         usv = proper_svd_packed(self.A).to(dev)
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         B = usv.shape[0]
         out = torch.empty((B, int(num_samples), 3, 3), device=dev, dtype=torch.float32)
-        with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _cabi.check(lib.rnf_fisher_sample(C.c_void_p(usv.data_ptr()), B, int(num_samples), C.c_uint64(seed),
-                                              C.c_void_p(out.data_ptr()), st))
+        _cabi.launch("rnf_fisher_sample", dev, usv, B, int(num_samples), C.c_uint64(seed), out)
         return out
 
     sample = _sample

@@ -35,16 +35,15 @@ class _NoProgramState:
     """Mixin: the packed-program cache holds device pointers and a ctypes handle; it is rebuilt on demand and must not travel
     through copy.deepcopy / pickle / torch.save of the module."""
 
+    _CACHES = ("_rnf_programs", "_rnf_train_programs")      # set by _program and _train_program
+
     def invalidate_cache(self):
         """Forget the packed weights (needed only after writes that bypass autograd versioning, e.g. ``p.data.copy_()``)."""
-        self.__dict__.pop("_rnf_programs", None)
-        self.__dict__.pop("_rnf_train_programs", None)
+        for k in self._CACHES:
+            self.__dict__.pop(k, None)
 
     def __getstate__(self):
-        state = self.__dict__.copy()
-        state.pop("_rnf_programs", None)
-        state.pop("_rnf_train_programs", None)
-        return state
+        return {k: v for k, v in self.__dict__.items() if k not in self._CACHES}
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -494,6 +493,46 @@ def _check_rotation(rotation):
     return rotation.to(torch.float32).contiguous()
 
 
+def _refuse_ablation(layers, what: str) -> None:
+    ablation = [l.kind for l in layers if l.kind.split("_")[0] in engine.ABLATION_KINDS]
+    if ablation:
+        raise NotImplementedError(f"{what} the ablation layers {sorted(set(ablation))}")
+
+
+def _per_image(conditional, feature, fisher_A, dev, N=None, feature_index=None):
+    """The per-image arguments of a call on N rotations (Flow.log_prob_grad, Flow.log_prob) or on a grid (Flow.grid_log_prob, N None):
+    (feature [B,F] float32 on ``dev`` or None, B, idx int32 [N] or None, rows per image, A9, c).  B is the number of feature rows, else
+    (not on a grid) of fisher_A's matrices, else 1.  Rows reach their image through ``feature_index``, else image-major, N % B == 0."""
+    from .fisher import fisher_constants
+    B = 1
+    if conditional:
+        if feature is None:
+            raise AssertionError("The input feature is needed in this module")
+        feature = feature.to(dev, torch.float32)
+        if N is not None and feature.dim() != 2:
+            raise ValueError(f"feature must be [B,F] with one row per image, got {tuple(feature.shape)}")
+        B = feature.shape[0]
+    else:
+        feature = None
+        if N is not None and fisher_A is not None:
+            B = fisher_A.shape[0]
+    idx, rpi = None, 1
+    if feature_index is not None:
+        idx = feature_index.to(dev, torch.int32).contiguous()
+        if idx.shape != (N,):
+            raise ValueError("feature_index must have one entry per rotation")
+    elif N is not None and (conditional or fisher_A is not None):
+        if B <= 0 or N % B != 0:
+            raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
+        rpi = N // B
+    A9 = c = None
+    if fisher_A is not None:
+        A9, c = fisher_constants(fisher_A.to(dev))
+        if A9.shape[0] != B:
+            raise ValueError("fisher_A must have one 3x3 matrix per image")
+    return feature, B, idx, rpi, A9, c
+
+
 def fused_kernels_run(layers) -> bool:
     """True when the fused kernels evaluate this layer stack: they are specialised for Mobius layers of K_SEGMENTS components and have
     no ConditionLU (batch-coupled in the reference), which run in the per-layer operators of train.py instead."""
@@ -628,39 +667,13 @@ class Flow(_NoProgramState, nn.Module):
         with N % B == 0.  fisher_A [B,3,3] adds log p of MatrixFisherN(A_b) at the flow's output (utils/fisher.py:217-232).
         One launch of csrc/flow_grad.cu; the outputs are plain tensors, not autograd graphs.  Flows with segments != 64 or
         ConditionLU layers run autograd through the per-layer operators of train.py instead (same numbers)."""
-        from .fisher import fisher_constants
         layers = list(self.layers)
-        ablation = [l.kind for l in layers if l.kind.split("_")[0] in engine.ABLATION_KINDS]
-        if ablation:
-            raise NotImplementedError(f"Flow.log_prob_grad: no rotation gradient for the ablation layers {sorted(set(ablation))}")
+        _refuse_ablation(layers, "Flow.log_prob_grad: no rotation gradient for")
         R = _check_rotation(rotation).detach()
         N = R.shape[0]
         dev = R.device
-        conditional = bool(self.condition)
-        if conditional:
-            if feature is None:
-                raise AssertionError("The input feature is needed in this module")
-            feature = feature.detach().to(dev, torch.float32)
-            if feature.dim() != 2:
-                raise ValueError(f"feature must be [B,F] with one row per image, got {tuple(feature.shape)}")
-            B = feature.shape[0]
-        else:
-            feature = None
-            B = fisher_A.shape[0] if fisher_A is not None else 1
-        idx, rpi = None, 1
-        if feature_index is not None:
-            idx = feature_index.to(dev, torch.int32).contiguous()
-            if idx.shape != (N,):
-                raise ValueError("feature_index must have one entry per rotation")
-        elif conditional or fisher_A is not None:
-            if B <= 0 or N % B != 0:
-                raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
-            rpi = N // B
-        A9 = c = None
-        if fisher_A is not None:
-            A9, c = fisher_constants(fisher_A.detach().to(dev))
-            if A9.shape[0] != B:
-                raise ValueError("fisher_A must have one 3x3 matrix per image")
+        feature, B, idx, rpi, A9, c = _per_image(bool(self.condition), None if feature is None else feature.detach(),
+                                                 None if fisher_A is None else fisher_A.detach(), dev, N, feature_index)
         if N == 0:
             return R.new_empty((0,)), R.new_empty((0, 3, 3))
         if not fused_kernels_run(layers):
@@ -686,35 +699,14 @@ class Flow(_NoProgramState, nn.Module):
             loss = -logp.mean()
         """
         from . import train
-        from .fisher import fisher_constants
         layers = list(self.layers)
-        ablation = [l.kind for l in layers if l.kind.split("_")[0] in engine.ABLATION_KINDS]
-        if ablation:
-            raise NotImplementedError(f"Flow.log_prob: no differentiable path for the ablation layers {sorted(set(ablation))}")
+        _refuse_ablation(layers, "Flow.log_prob: no differentiable path for")
         R = _check_rotation(rotation)
         N, dev = R.shape[0], R.device
         conditional = bool(self.condition)
-        B = 1
-        if conditional:
-            if feature is None:
-                raise AssertionError("The input feature is needed in this module")
-            feature = feature.to(dev, torch.float32)
-            if feature.dim() != 2:
-                raise ValueError(f"feature must be [B,F] with one row per image, got {tuple(feature.shape)}")
-            B = feature.shape[0]
-        else:
-            feature = None
-            if fisher_A is not None:
-                B = fisher_A.shape[0]
-        idx = None
-        if feature_index is not None:
-            idx = feature_index.to(dev, torch.int32).contiguous()
-            if idx.shape != (N,):
-                raise ValueError("feature_index must have one entry per rotation")
-        elif conditional or fisher_A is not None:
-            if B <= 0 or N % B != 0:
-                raise ValueError(f"{N} rotations do not split image-major over B={B} images: pass feature_index")
-            idx = torch.arange(N, device=dev, dtype=torch.int32) // (N // B)
+        feature, B, idx, rpi, A9, c = _per_image(conditional, feature, fisher_A, dev, N, feature_index)
+        if idx is None and (conditional or fisher_A is not None):
+            idx = torch.arange(N, device=dev, dtype=torch.int32) // rpi
         perms = self._perm_rows()
         if not fused_kernels_run(layers):
             rows = feature[idx.long()] if feature is not None else None
@@ -723,9 +715,6 @@ class Flow(_NoProgramState, nn.Module):
             tp = _train_program(self, layers, perms, self.feature_dim, dev)
             R_out, logp = train.fused_run(tp, layers, R, feature, idx if conditional else None, B)
         if fisher_A is not None:
-            A9, c = fisher_constants(fisher_A.to(dev))
-            if A9.shape[0] != B:
-                raise ValueError("fisher_A must have one 3x3 matrix per image")
             img = idx.long()
             logp = logp + (A9[img].reshape(N, 3, 3) * R_out).sum(dim=(1, 2)) - c[img]
         return logp
@@ -758,7 +747,6 @@ class Flow(_NoProgramState, nn.Module):
         fused into the same pass: ``spread`` [B] in radians over THIS slice and ``spread_num`` [B] for merging slices.
         Returns dict(max [B], argmax [B] int64 global grid index (first on ties), sumexp [B] = sum_g exp(logp - max),
         logp [B,G] if requested)."""
-        from .fisher import fisher_constants
         G_ = _check_rotation(grid)
         if torch.is_grad_enabled() and torch.is_tensor(feature) and feature.requires_grad:
             raise NotImplementedError(_GRAD_MESSAGE.format(what="the feature"))
@@ -766,17 +754,8 @@ class Flow(_NoProgramState, nn.Module):
             raise NotImplementedError(f"Flow.grid_log_prob runs in the fused kernels, which are specialised for segments={engine.K_SEGMENTS} and "
                                       "per-image conditional affines; use Flow.forward on the grid rotations for other segment counts / ConditionLU")
         prog = _program(self, list(self.layers), self._perm_rows(), self.feature_dim, G_.device)
-        cond, B = None, 1
-        if prog.cond_floats:
-            if feature is None:
-                raise AssertionError("The input feature is needed in this module")
-            cond = prog.condition(feature.to(G_.device))
-            B = feature.shape[0]
-        A9 = c = None
-        if fisher_A is not None:
-            A9, c = fisher_constants(fisher_A.to(G_.device))
-            if A9.shape[0] != B:
-                raise ValueError("fisher_A must have one 3x3 matrix per image")
+        feature, B, _, _, A9, c = _per_image(prog.cond_floats != 0, feature, fisher_A, G_.device)
+        cond = prog.condition(feature) if feature is not None else None
         off = None if offset is None else offset.to(G_.device, torch.float32).contiguous()
         mode = mlp_mode or engine.default_mlp_mode()
         if gt_rotations is not None:

@@ -1,7 +1,6 @@
 """HEALPix SO(3) query grids generated on the device (utils/sd.py:11-82)."""
 from __future__ import annotations
 
-import ctypes as C
 import math
 
 import torch
@@ -24,16 +23,13 @@ def closest_grid_level(num_queries: int) -> int:
 
 def healpix_grid(level: int, begin: int = 0, end: int | None = None, device=None) -> torch.Tensor:
     """Rotations [begin,end) of the level-`level` grid as float32 [n,3,3] on `device` (rnf_healpix_grid)."""
-    lib = _cabi.load()
     total = 72 * 8 ** level
     end = total if end is None else end
     device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if device.type != "cuda":
         raise RuntimeError("healpix_grid generates the grid on a B200; there is no CPU path")
     out = torch.empty((max(end - begin, 0), 3, 3), device=device, dtype=torch.float32)
-    with torch.cuda.device(device):
-        st = C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
-        _cabi.check(lib.rnf_healpix_grid(int(level), int(begin), int(end), C.c_void_p(out.data_ptr()), st))
+    _cabi.launch("rnf_healpix_grid", device, int(level), int(begin), int(end), out)
     return out
 
 
@@ -95,11 +91,7 @@ def healpix_children(level: int, index: torch.Tensor, offset: torch.Tensor | Non
     child = torch.empty((n, 8), device=dev, dtype=torch.int64)
     rot = torch.empty((n, 8, 3, 3), device=dev, dtype=torch.float32)
     off = None if offset is None else offset.to(dev, torch.float32).reshape(3, 3).contiguous()
-    lib = _cabi.load()
-    with torch.cuda.device(dev):
-        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-        _cabi.check(lib.rnf_healpix_children(level, C.c_void_p(idx.data_ptr()), n, C.c_void_p(off.data_ptr()) if off is not None else None,
-                                             C.c_void_p(child.data_ptr()), C.c_void_p(rot.data_ptr()), st))
+    _cabi.launch("rnf_healpix_children", dev, level, idx, n, off, child, rot)
     return child, rot
 
 
@@ -124,14 +116,10 @@ def top_k(values: torch.Tensor, index: torch.Tensor | None, k: int):
     ix = None if index is None else (index[None] if squeeze else index).to(dev, torch.int64).contiguous()
     out_v = torch.empty((B, k), device=dev, dtype=torch.float32)
     out_i = torch.empty((B, k), device=dev, dtype=torch.int64)
-    lib = _cabi.load()
     if B > 0:
-        nbytes = int(lib.rnf_topk_workspace_bytes(B, Cn, k))
+        nbytes = int(_cabi.load().rnf_topk_workspace_bytes(B, Cn, k))
         ws = torch.empty((max(nbytes, 1),), device=dev, dtype=torch.uint8)
-        with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _cabi.check(lib.rnf_topk(C.c_void_p(v.data_ptr()), C.c_void_p(ix.data_ptr()) if ix is not None else None, B, Cn, k,
-                                     C.c_void_p(ws.data_ptr()), nbytes, C.c_void_p(out_v.data_ptr()), C.c_void_p(out_i.data_ptr()), st))
+        _cabi.launch("rnf_topk", dev, v, ix, B, Cn, k, ws, nbytes, out_v, out_i)
     if squeeze:
         return out_v[0], out_i[0]
     return out_v, out_i

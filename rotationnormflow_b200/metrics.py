@@ -1,8 +1,6 @@
 """Post-path metrics on the device (SURVEY.md 8f N2): utils/utils.py:208-209 (acc), :225-235 (geodesic distances)."""
 from __future__ import annotations
 
-import ctypes as C
-
 import torch
 
 from . import _cabi
@@ -12,16 +10,12 @@ def min_geodesic_distance_rotmats(r1s: torch.Tensor, r2s: torch.Tensor) -> torch
     """r1s [n,3,3] (estimates), r2s [n,k,3,3] (ground-truth sets) -> [n] angle to the closest one (utils/utils.py:231-235)."""
     if not r1s.is_cuda:
         raise RuntimeError("rotationnormflow_b200 runs on a B200 only: tensors must be CUDA tensors (there is no CPU fallback)")
-    lib = _cabi.load()
     n = r1s.shape[0]
     r2s = r2s.reshape(n, -1, 3, 3)
     est = r1s.reshape(n, 9).to(torch.float32).contiguous()
     gt = r2s.to(r1s.device, torch.float32).contiguous()
     out = torch.empty((n,), device=r1s.device, dtype=torch.float32)
-    with torch.cuda.device(r1s.device):
-        st = C.c_void_p(torch.cuda.current_stream(r1s.device).cuda_stream)
-        _cabi.check(lib.rnf_min_geodesic(C.c_void_p(est.data_ptr()), C.c_void_p(gt.data_ptr()), n, gt.shape[1],
-                                         C.c_void_p(out.data_ptr()), st))
+    _cabi.launch("rnf_min_geodesic", r1s.device, est, gt, n, gt.shape[1], out)
     return out
 
 

@@ -5,7 +5,6 @@ local maxima and how much of the probability each one carries: greedy non-maximu
 """
 from __future__ import annotations
 
-import ctypes as C
 import math
 
 import torch
@@ -16,7 +15,9 @@ MAX_MODES = 256
 RECORD_BYTES = 80          # RNF_MODES_RECORD_BYTES: one rank's per-image record of a sharded round
 
 
-def _check_args(values, rotations, num_modes, min_separation, neighbour_radius):
+def _inputs(values, rotations, num_modes, min_separation, neighbour_radius):
+    """The checked arguments of rotation_modes, values as float32 [B,G], rotations as float32 [G,3,3] on the values' device, and the
+    output dict: (M, theta, rho, squeeze, values, rotations, out)."""
     M = int(num_modes)
     theta, rho = float(min_separation), float(neighbour_radius)
     if not 1 <= M <= MAX_MODES:
@@ -29,7 +30,13 @@ def _check_args(values, rotations, num_modes, min_separation, neighbour_radius):
         raise ValueError(f"rotations must be [G,3,3] with G = values.shape[-1], got {tuple(rotations.shape)} for {tuple(values.shape)}")
     if not (values.is_cuda and rotations.is_cuda):
         raise RuntimeError("rotationnormflow_b200 runs on a B200 only: tensors must be CUDA tensors (there is no CPU fallback)")
-    return M, theta, rho
+    squeeze = values.dim() == 1
+    v = (values[None] if squeeze else values).to(torch.float32).contiguous()      # (a reshape to [-1, G] is ambiguous when G == 0)
+    B, dev = v.shape[0], v.device
+    out = dict(index=torch.empty((B, M), device=dev, dtype=torch.int64), value=torch.empty((B, M), device=dev, dtype=torch.float32),
+               local_max=torch.empty((B, M), device=dev, dtype=torch.bool), mass=torch.empty((B, M), device=dev, dtype=torch.float32),
+               count=torch.empty((B,), device=dev, dtype=torch.int32))
+    return M, theta, rho, squeeze, v, rotations.to(dev, torch.float32).contiguous(), out
 
 
 def rotation_modes(values: torch.Tensor, rotations: torch.Tensor, num_modes: int, min_separation: float, neighbour_radius: float,
@@ -52,33 +59,16 @@ def rotation_modes(values: torch.Tensor, rotations: torch.Tensor, num_modes: int
     A pick that is not a local maximum is a "shoulder": the rim of an earlier mode's ball.  On a continuous ridge of equal density
     (the cone and cylinder of SYMSOL) the picks sample the ridge about every ``min_separation``, and their ``local_max`` flags are
     decided by fp32 noise along it."""
-    M, theta, rho = _check_args(values, rotations, num_modes, min_separation, neighbour_radius)
-    squeeze = values.dim() == 1
-    v = (values[None] if squeeze else values).to(torch.float32).contiguous()      # (a reshape to [-1, G] is ambiguous when G == 0)
+    M, theta, rho, squeeze, v, rot, out = _inputs(values, rotations, num_modes, min_separation, neighbour_radius)
     B, G = v.shape
-    dev = v.device
-    rot = rotations.to(dev, torch.float32).contiguous()
-    lib = _cabi.load()
-    out = dict(index=torch.empty((B, M), device=dev, dtype=torch.int64), value=torch.empty((B, M), device=dev, dtype=torch.float32),
-               local_max=torch.empty((B, M), device=dev, dtype=torch.bool), mass=torch.empty((B, M), device=dev, dtype=torch.float32),
-               count=torch.empty((B,), device=dev, dtype=torch.int32))
     if B > 0:
-        nbytes = int(lib.rnf_rotation_modes_workspace_bytes(G, B, M))
-        ws = torch.empty((nbytes,), device=dev, dtype=torch.uint8)
-
-        def p(t):
-            return C.c_void_p(t.data_ptr())
-        with torch.cuda.device(dev):
-            st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _cabi.check(lib.rnf_rotation_modes(p(v), B, G, int(g_index0), p(rot), M, theta, rho, p(ws), nbytes, p(out["index"]),
-                                               p(out["value"]), p(out["local_max"]), p(out["mass"]), p(out["count"]), st))
+        nbytes = int(_cabi.load().rnf_rotation_modes_workspace_bytes(G, B, M))
+        ws = torch.empty((nbytes,), device=v.device, dtype=torch.uint8)
+        _cabi.launch("rnf_rotation_modes", v.device, v, B, G, int(g_index0), rot, M, theta, rho, ws, nbytes, out["index"], out["value"],
+                     out["local_max"], out["mass"], out["count"])
     if squeeze:
         out = {k: t[0] for k, t in out.items()}
     return out
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr())
 
 
 class RankModes:
@@ -94,34 +84,23 @@ class RankModes:
     def __init__(self, values, rotations, g_index0, num_modes, min_separation, neighbour_radius):
         if int(g_index0) < 0:
             raise ValueError(f"g_index0 must be >= 0, got {g_index0}")
-        M, self.theta, self.rho = _check_args(values, rotations, num_modes, min_separation, neighbour_radius)
-        self.M, self.g_index0, self.squeeze = M, int(g_index0), values.dim() == 1
-        v = (values[None] if self.squeeze else values).to(torch.float32).contiguous()
-        self.B, self.G = v.shape
-        dev = self.device = v.device
-        self.v, self.rot = v, rotations.to(dev, torch.float32).contiguous()
-        self.lib = _cabi.load()
-        B = self.B
-        self.out = dict(index=torch.empty((B, M), device=dev, dtype=torch.int64), value=torch.empty((B, M), device=dev, dtype=torch.float32),
-                        local_max=torch.empty((B, M), device=dev, dtype=torch.bool), mass=torch.empty((B, M), device=dev, dtype=torch.float32),
-                        count=torch.empty((B,), device=dev, dtype=torch.int32),
-                        rotations=torch.empty((B, M, 3, 3), device=dev, dtype=torch.float32))
+        M, self.theta, self.rho, self.squeeze, self.v, self.rot, self.out = _inputs(values, rotations, num_modes, min_separation,
+                                                                                    neighbour_radius)
+        self.M, self.g_index0 = M, int(g_index0)
+        self.B, self.G = self.v.shape
+        B, dev = self.B, self.v.device
+        self.device = dev
+        self.out["rotations"] = torch.empty((B, M, 3, 3), device=dev, dtype=torch.float32)
         self.record = torch.empty((B, RECORD_BYTES), device=dev, dtype=torch.uint8)
-        self.nbytes = int(self.lib.rnf_rotation_modes_shard_workspace_bytes(self.G, B))
+        self.nbytes = int(_cabi.load().rnf_rotation_modes_shard_workspace_bytes(self.G, B))
         self.ws = torch.empty((self.nbytes,), device=dev, dtype=torch.uint8)
-        with torch.cuda.device(dev):
-            _cabi.check(self.lib.rnf_rotation_modes_shard_setup(_ptr(self.rot), self.G, B, _ptr(self.ws), self.nbytes, self._stream()))
-
-    def _stream(self):
-        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        _cabi.launch("rnf_rotation_modes_shard_setup", dev, self.rot, self.G, B, self.ws, self.nbytes)
 
     def propose(self, r: int) -> torch.Tensor:
         """Round r on this rank's slice: labels mode r-1's points, tests it, proposes mode r.  Returns the record buffer (reused by
         the next round: gather it before proposing again)."""
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_rotation_modes_shard_round(_ptr(self.v), self.B, self.G, self.g_index0, _ptr(self.rot), int(r), self.M,
-                                                                self.theta, self.rho, _ptr(self.ws), self.nbytes, _ptr(self.record),
-                                                                self._stream()))
+        _cabi.launch("rnf_rotation_modes_shard_round", self.device, self.v, self.B, self.G, self.g_index0, self.rot, int(r), self.M, self.theta,
+                     self.rho, self.ws, self.nbytes, self.record)
         return self.record
 
     def merge(self, r: int, gathered: torch.Tensor) -> None:
@@ -130,10 +109,8 @@ class RankModes:
             raise ValueError(f"gathered records must be uint8 [W,{self.B},{RECORD_BYTES}], got {gathered.dtype} {tuple(gathered.shape)}")
         g = gathered.to(self.device).contiguous()
         o = self.out
-        with torch.cuda.device(self.device):
-            _cabi.check(self.lib.rnf_rotation_modes_shard_merge(_ptr(g), g.shape[0], self.B, int(r), self.M, _ptr(self.ws), self.nbytes,
-                                                                _ptr(o["index"]), _ptr(o["value"]), _ptr(o["local_max"]), _ptr(o["mass"]),
-                                                                _ptr(o["count"]), _ptr(o["rotations"]), self._stream()))
+        _cabi.launch("rnf_rotation_modes_shard_merge", self.device, g, g.shape[0], self.B, int(r), self.M, self.ws, self.nbytes, o["index"],
+                     o["value"], o["local_max"], o["mass"], o["count"], o["rotations"])
 
     def result(self) -> dict:
         """The outputs of ``rotation_modes`` plus ``rotations`` [B,M,3,3] (the owning rank's matrix of each mode, NaN padding) and

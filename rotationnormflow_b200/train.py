@@ -13,20 +13,10 @@ reference's; ``rotation.grad`` of the input is the tangential part of the refere
 a rotation matrix has no meaning on the manifold)."""
 from __future__ import annotations
 
-import ctypes as C
-
 import torch
 from torch.autograd.function import once_differentiable
 
 from . import _cabi, engine
-
-
-def _ptr(t):
-    return C.c_void_p(t.data_ptr())
-
-
-def _stream(dev):
-    return C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
 
 
 class MobiusMixture(torch.autograd.Function):
@@ -34,12 +24,10 @@ class MobiusMixture(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, R, out, perm: int, inverse: bool, K: int):
-        lib = _cabi.load()
         R, out = R.contiguous().float(), out.contiguous().float()
         N = R.shape[0]
         R_out, ldj, theta = torch.empty_like(R), R.new_empty(N), R.new_empty(N)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_mobius_forward(_ptr(R), _ptr(out), N, K, perm, int(inverse), _ptr(R_out), _ptr(ldj), _ptr(theta), _stream(R.device)))
+        _cabi.launch("rnf_train_mobius_forward", R.device, R, out, N, K, perm, int(inverse), R_out, ldj, theta)
         ctx.save_for_backward(R, out, theta, R_out)
         ctx.meta = (perm, inverse, K)
         return R_out, ldj
@@ -49,14 +37,11 @@ class MobiusMixture(torch.autograd.Function):
     def backward(ctx, G_Rout, g_ldj):
         R, out, theta, R_out = ctx.saved_tensors
         perm, inverse, K = ctx.meta
-        lib = _cabi.load()
         N = R.shape[0]
         G_Rout = torch.zeros_like(R) if G_Rout is None else G_Rout.contiguous().float()
         g_ldj = R.new_zeros(N) if g_ldj is None else g_ldj.contiguous().float()
         G_R, G_out = torch.empty_like(R), torch.empty_like(out)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_mobius_backward(_ptr(R), _ptr(out), N, K, perm, int(inverse), _ptr(theta), _ptr(R_out), _ptr(G_Rout), _ptr(g_ldj),
-                                                      _ptr(G_R), _ptr(G_out), _stream(R.device)))
+        _cabi.launch("rnf_train_mobius_backward", R.device, R, out, N, K, perm, int(inverse), theta, R_out, G_Rout, g_ldj, G_R, G_out)
         return G_R, G_out, None, None, None
 
 
@@ -65,12 +50,10 @@ class QuatAffine(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, R, W):
-        lib = _cabi.load()
         R, W = R.contiguous().float(), W.contiguous().float()
         N = R.shape[0]
         R_out, loglen = torch.empty_like(R), R.new_empty(N)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_affine_forward(_ptr(R), _ptr(W), N, _ptr(R_out), _ptr(loglen), _stream(R.device)))
+        _cabi.launch("rnf_train_affine_forward", R.device, R, W, N, R_out, loglen)
         ctx.save_for_backward(R, W, R_out)
         return R_out, loglen
 
@@ -78,13 +61,11 @@ class QuatAffine(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, G_Rout, g_loglen):
         R, W, R_out = ctx.saved_tensors
-        lib = _cabi.load()
         N = R.shape[0]
         G_Rout = torch.zeros_like(R) if G_Rout is None else G_Rout.contiguous().float()
         g_loglen = R.new_zeros(N) if g_loglen is None else g_loglen.contiguous().float()
         G_R, G_W = torch.empty_like(R), torch.empty_like(W)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_affine_backward(_ptr(R), _ptr(W), N, _ptr(R_out), _ptr(G_Rout), _ptr(g_loglen), _ptr(G_R), _ptr(G_W), _stream(R.device)))
+        _cabi.launch("rnf_train_affine_backward", R.device, R, W, N, R_out, G_Rout, g_loglen, G_R, G_W)
         return G_R, G_W
 
 
@@ -94,12 +75,10 @@ class AblationLayer(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, R, M, kind: int):
-        lib = _cabi.load()
         R, M = R.contiguous().float(), M.contiguous().float()
         N = R.shape[0]
         R_out, ldj = torch.empty_like(R), R.new_empty(N)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_ablation_forward(_ptr(R), _ptr(M), N, kind, _ptr(R_out), _ptr(ldj), _stream(R.device)))
+        _cabi.launch("rnf_train_ablation_forward", R.device, R, M, N, kind, R_out, ldj)
         ctx.save_for_backward(R, M, R_out)
         ctx.kind = kind
         return R_out, ldj
@@ -108,14 +87,11 @@ class AblationLayer(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, G_Rout, g_ldj):
         R, M, R_out = ctx.saved_tensors
-        lib = _cabi.load()
         N = R.shape[0]
         G_Rout = torch.zeros_like(R) if G_Rout is None else G_Rout.contiguous().float()
         g_ldj = R.new_zeros(N) if g_ldj is None else g_ldj.contiguous().float()
         G_R, G_M = torch.empty_like(R), torch.empty_like(M)
-        with torch.cuda.device(R.device):
-            _cabi.check(lib.rnf_train_ablation_backward(_ptr(R), _ptr(M), N, ctx.kind, _ptr(R_out), _ptr(G_Rout), _ptr(g_ldj), _ptr(G_R),
-                                                        _ptr(G_M), _stream(R.device)))
+        _cabi.launch("rnf_train_ablation_backward", R.device, R, M, N, ctx.kind, R_out, G_Rout, g_ldj, G_R, G_M)
         return G_R, G_M, None
 
 

@@ -24,7 +24,7 @@ import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import rotationnormflow_b200 as rnf  # noqa: E402
-from rotationnormflow_b200 import engine, flow as flow_mod  # noqa: E402
+from rotationnormflow_b200 import _cabi, engine, flow as flow_mod  # noqa: E402
 from rotationnormflow_b200.fisher import fisher_constants  # noqa: E402
 from oracle import rnf_oracle as orc  # noqa: E402
 
@@ -113,8 +113,8 @@ def run_config(name, fisher, N, dev, warmup, reps):
     def bwd_kernel():
         for s in range(0, N, chunk):
             n = min(chunk, N - s)
-            tp._call("rnf_flow_train_backward", weights, R[s:s + n], n, cond, N, idx32[s:s + n], 0, None, g_ldj[s:s + n],
-                     G_R[s:s + n], ws, int(ws.numel()))
+            _cabi.launch("rnf_flow_train_backward", dev, tp.prog.handle, weights, R[s:s + n], n, cond, N, idx32[s:s + n], 0, None, g_ldj[s:s + n],
+                         G_R[s:s + n], ws, int(ws.numel()))
 
     holder = {}
 
