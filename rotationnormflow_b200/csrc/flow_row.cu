@@ -33,23 +33,8 @@ namespace {
 #define TRACE(i) do { } while (0)
 #endif
 
-#ifndef RNF_ROW_SPLIT_PACKED
-#define RNF_ROW_SPLIT_PACKED 1
-#endif
 #ifndef RNF_INV_NEWTON
 #define RNF_INV_NEWTON 1         // inverse: locate the root with Newton steps, then replay the reference's 15 halvings (see below)
-#endif
-#ifndef RNF_INV_AMB_BAND
-#define RNF_INV_AMB_BAND 1e-6f    // replay: |predicted F(x0)| below which the sign is taken from an explicit evaluation
-#endif
-#ifndef RNF_INV_START_AVG
-#define RNF_INV_START_AVG 0       // inverse: Newton starts at the closed-form inverse of the Mobius map of the weighted mean centre
-#endif
-#ifndef RNF_INV_PREDICT
-#define RNF_INV_PREDICT 1         // inverse: stop the Newton iteration on the PREDICTED error of the next iterate (one evaluation less per layer)
-#endif
-#ifndef RNF_INV_DELTA
-#define RNF_INV_DELTA 1          // inverse: theta_k = t + 2 asin(sin delta_k) (no quadrant logic), see mobius_pair.cuh probe_delta_pairs
 #endif
 constexpr int kThreads = 256;
 constexpr int kRows = 128;                        // rows per tile = TMEM lanes = threads per tile
@@ -79,7 +64,6 @@ __device__ __forceinline__ void store_a32(uint8_t* a_hi, uint8_t* a_lo, int r, i
     uint32_t hi[4], lo[4];
 #pragma unroll
     for (int e = 0; e < 4; ++e) {
-#if RNF_ROW_SPLIT_PACKED
       // as in flow_t4.cu: truncation by mask + packed subtract (5 instructions per pair instead of 6 with two conversions back and
       // two scalar subtracts); this kernel runs at the per-warp issue cadence, so an instruction less is time less.  The masked
       // value converts exactly up to 65504 and to +Inf from 65536 on: overflow is loud, as in flow_t4.cu relu_split_pair.
@@ -89,9 +73,6 @@ __device__ __forceinline__ void store_a32(uint8_t* a_hi, uint8_t* a_lo, int r, i
       float d0, d1;
       upk(sub2(pk(x0, x1), pk(m0, m1)), d0, d1);
       asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo[e]) : "f"(d1), "f"(d0));
-#else
-      relu_split2(v[8 * c + 2 * e], v[8 * c + 2 * e + 1], hi[e], lo[e]);
-#endif
     }
     const int off = rbase + (((4 * h + c) ^ (r & 7)) << 4);
     *reinterpret_cast<uint4*>(a_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
@@ -412,26 +393,14 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
 #pragma unroll 1
           for (int j = 0; j < 4; ++j) {
             tmem_ld32_async(tm + 64 * j + 32, bufB);
-#if RNF_INV_DELTA
             probe_delta_pairs<4, RNF_INV_NEWTON != 0>(cs, sn, bufA, Fs2, Sf2);
-#else
-            probe_pairs<4, RNF_INV_NEWTON != 0>(cs, sn, bufA, Fs2, &Sf2);
-#endif
             tmem_ld_wait32(bufB);
             if (j < 3) tmem_ld32_async(tm + 64 * j + 64, bufA);
-#if RNF_INV_DELTA
             probe_delta_pairs<4, RNF_INV_NEWTON != 0>(cs, sn, bufB, Fs2, Sf2);
-#else
-            probe_pairs<4, RNF_INV_NEWTON != 0>(cs, sn, bufB, Fs2, &Sf2);
-#endif
             if (j < 3) tmem_ld_wait32(bufA);
           }
           dF = hsum(Sf2) / S_sp;
-#if RNF_INV_DELTA
           return fmaf(2.0f, hsum(Fs2) / S_sp, t) - ys;  // sum_k pi_k theta_k = t + 2 sum_k pi_k delta_k
-#else
-          return hsum(Fs2) / S_sp - ys;                // the reference's f(x0), same arithmetic for every use
-#endif
         };
         float lo = kPi / 2.0f, hi = 1.5f * kPi, x0 = 0.0f;
         int n_eval = 0;                               // evaluations of F by this warp in this layer (measurement hook)
@@ -444,24 +413,8 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
         // fp32 evaluation noise of F, a region where the reference's own decision is rounding noise too -- x0 is evaluated
         // explicitly with the reference's arithmetic, exactly as the plain bisection would.  At most one dyadic probe per row can be
         // that close (their spacing is pi / 2^15 = 9.6e-5 at the last level).
+        constexpr float kAmbBand = 1e-6f;             // replay: |predicted F(x0)| below which the sign is taken from an explicit evaluation
         float ts = kPi, dFs = 1.0f;                   // root estimate and slope there
-#if RNF_INV_START_AVG
-        // Starting point: the mixture with ALL components at the weighted mean centre w = sum_k pi_k w'_k is one Mobius map, whose
-        // inverse is closed form: z0 = (h + w) / (1 + conj(w) h) with h = e^{i ys}.  It agrees with the mixture map to first order in
-        // the centres (the iteration used to start at pi, i.e. at w = 0).  tools/proto/newton_stop_study.py: evaluations per warp
-        // 3.0 -> 2.1 on moderate mixtures, 5.3 -> 3.5 / 6.8 -> 4.4 on hard ones (|w'| up to 0.7, peaky weights).
-        {
-          const float inv_sp = 1.0f / S_sp;
-          const float wa = -hsum(S_th2) * inv_sp, wb = -hsum(S_f2) * inv_sp;      // in-plane mean centre (alpha, beta)
-          const float rn = rsqrtf(fmaf(zr, zr, zv * zv));
-          const float hx = zr * rn, hy = zv * rn;                                  // h = e^{i ys}
-          const float nx_ = hx + wa, ny_ = hy + wb;
-          const float dx = 1.0f + fmaf(wa, hx, wb * hy), dy = fmaf(wa, hy, -wb * hx);
-          float t0 = atan2f(fmaf(ny_, dx, -nx_ * dy), fmaf(nx_, dx, ny_ * dy));    // arg(n conj(d))
-          t0 = t0 >= 0.0f ? t0 : t0 + kTwoPi;
-          ts = fminf(fmaxf(t0, lo + 1e-3f), hi - 1e-3f);
-        }
-#endif
         bool newton_ok = false;
         {
           float a_ = lo, b_ = hi;
@@ -478,14 +431,12 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
               const float step = F / dF;
               const float as = fabsf(step);
               conv = as < 1e-5f;                        // quadratic convergence: the error after this step is ~step^2
-#if RNF_INV_PREDICT
               // ... and how far "~" is can be read off the last two steps: e_{k+1} = C e_k^2 with C = |F''/2F'| ~ |s_k| / s_{k-1}^2
               // once the iteration contracts (s_k = e_k up to the much smaller e_{k+1}).  Stop as soon as the error PREDICTED after
               // this step is below 5e-8 -- the fp32 evaluation noise of F keeps t* from being better than ~1e-7 anyway, and the
               // replay below evaluates explicitly whenever a midpoint is within 2e-6 / F' >= 3.5e-7 of t*.  Saves the evaluation
               // whose only result would be "the step is now below 1e-5" (typically the fourth).
               if (prev > 0.0f && as < 1e-2f) conv = conv || fmaxf(as / (prev * prev), 2.0f) * as * as < 5e-8f;
-#endif
               float tn = ts - step;
               prev = as;
               if (!conv && !(tn > a_ && tn < b_)) { tn = 0.5f * (a_ + b_); prev = 0.0f; }
@@ -499,7 +450,7 @@ __global__ void __launch_bounds__(kThreads, 1) flow_row_kernel(const FlowArgs a)
           for (int it = 0; it < 15; ++it) {
             x0 = (lo + hi) / 2.0f;
             const float d = x0 - ts;
-            const bool amb = fabsf(d) * dFs < RNF_INV_AMB_BAND;
+            const bool amb = fabsf(d) * dFs < kAmbBand;
             bool neg = d < 0.0f;
             if (__any_sync(0xffffffffu, amb)) {
               float dF;

@@ -18,8 +18,8 @@
 // One WORKER thread owns one rotation (512 threads = 4 tiles x 128 rows): nothing is computed twice, nothing is exchanged.
 //
 // Warp specialisation (round 2): a fifth warpgroup holds one SERVICE warp per tile that does nothing but wait for the tile's
-// hand-over (an mbarrier the four worker warps arrive on), issue the tile's MMAs, wake the workers when a dependent GEMM has
-// completed, and refill weight pieces.  Before, one of the tile's own worker warps issued: tcgen05.mma issue blocks at the pace
+// hand-over (an mbarrier the four worker warps arrive on), issue the tile's MMAs and refill weight pieces; the workers watch the
+// MMA mbarrier of a dependent GEMM themselves.  Before, one of the tile's own worker warps issued: tcgen05.mma issue blocks at the pace
 // of the tensor pipe (13 MMAs = ~450 cycles per GEMM, eight GEMMs per layer), so that warp ran ~30 % behind its three siblings
 // and every hand-over of the tile waited for it.  Registers: 640 threads launch with 96 each (the CTA's pool); the service warpgroup
 // drops to 32 (setmaxnreg.dec) and the four worker warpgroups take 112 (setmaxnreg.inc): 512 x 112 + 128 x 32 = 640 x 96.
@@ -42,33 +42,17 @@ namespace {
 #define TRACE(i) do { } while (0)
 #endif
 
-#ifndef RNF_T4_SPLIT_MASK
-#define RNF_T4_SPLIT_MASK 1
-#endif
-#ifndef RNF_T4_HALF_EPI
-#define RNF_T4_HALF_EPI 0        // 1: hand each half of an epilogue's A operand over on its own (first K steps of the next GEMM issue early)
-#endif
-#ifndef RNF_T4_SVC_HINT_NS
-#define RNF_T4_SVC_HINT_NS 0     // suspend-time hint of the service warps' mbarrier waits (0 = default try_wait)
-#endif
-#ifndef RNF_T4_DIRECT_WAIT_NS
-#define RNF_T4_DIRECT_WAIT_NS 2000  // > 0: workers wait for chain GEMMs on the MMA mbarrier themselves (try_wait with this hint) instead of the named barrier
-#endif
-#ifndef RNF_T4_SVC_NAP_NS
-#define RNF_T4_SVC_NAP_NS 0      // service warp: nanosleep between polls of waits that are NOT on a tile's critical path
-#endif
-#ifndef RNF_T4_WORKER_REGS
-#define RNF_T4_WORKER_REGS 112
-#endif
-#ifndef RNF_T4_SERVICE_REGS
-#define RNF_T4_SERVICE_REGS 32
-#endif
 constexpr int kTiles = 4;            // tiles in flight per SM (TMEM: 4 x 128 columns)
 constexpr int kWorkers = kTiles * 128;
 constexpr int kThreads = kWorkers + kTiles * 32;   // + one service warp per tile (warpgroup 4)
 constexpr int kRows = 128;
+constexpr int kWorkerRegs = 112, kServiceRegs = 32;   // setmaxnreg targets of the worker / service warpgroups
 // setmaxnreg moves registers inside the pool the CTA was LAUNCHED with (640 threads x 96, the largest multiple of 8 that fits the file)
-static_assert(kWorkers * RNF_T4_WORKER_REGS + kTiles * 32 * RNF_T4_SERVICE_REGS <= kThreads * 96, "register pool of the CTA");
+static_assert(kWorkers * kWorkerRegs + kTiles * 32 * kServiceRegs <= kThreads * 96, "register pool of the CTA");
+// Workers wait for a chain GEMM by polling its mbarrier with this suspend-time hint (ns).
+constexpr int kDirectWaitNs = 2000;
+// Variants that measured slower or equal (DESIGN.md section 8b, svc-x: half-epilogue hand-over, named-barrier wake-up of the
+// workers, suspend hints / naps in the service warps, the convert-back fp16 split) were removed; their code is in commit d73682a.
 
 // shared memory (bytes from a 1024-aligned base)
 constexpr int kOffW = 0;                                  // W1 | W2 | W3 pieces
@@ -84,10 +68,9 @@ constexpr int kSmemAlloc = kSmemBytes + 1024;
 static_assert(kOffLastW % 1024 == 0 && kW1Bytes % 1024 == 0, "UMMA SW128 tiles need 1024 B alignment");
 static_assert(kOffY % 16 == 0 && kOffC % 16 == 0 && kOffAux % 16 == 0, "no-swizzle blocks need 16 B alignment");
 
-// READY / READY2: hand-overs of a tile's workers to its service warp.  The second half of an epilogue has its own barrier: between
-// two phases of ONE barrier the workers always wait for a GEMM, i.e. for the service warp to have consumed the earlier phase, so a
-// parity wait can never be lapped (with a single barrier the two halves of an epilogue could both complete while the service warp
-// still waits for a weight piece, and a fast warp's second arrival would count towards the first phase).
+// READY: hand-overs of a tile's workers to its service warp.  Between two phases of it the workers always wait for a GEMM, i.e. for
+// the service warp to have consumed the earlier phase, so a parity wait can never be lapped.  Nothing reads the READY2 barriers
+// (they served the removed half-epilogue hand-over); they stay initialised because dropping them changes the kernel's code.
 enum { BAR_W_FULL = 0 /* W1,W2,W3,W4 */, BAR_AUX_FULL = 4 /* [2] */, BAR_MMA = 6 /* [tile] */, BAR_READY = 6 + kTiles /* [tile] */,
        BAR_READY2 = 6 + 2 * kTiles /* [tile] */, BAR_COUNT = 6 + 3 * kTiles };
 static_assert(BAR_COUNT <= 24, "mbarrier slots");
@@ -121,7 +104,8 @@ __device__ __forceinline__ void issue_split_ts(uint32_t d, uint32_t a_hi, uint32
   for (int k = 0; k < 4; ++k) umma_f16_ts(d, a_hi + 8 * k, b_hi + 2 * k, kDescHi, idesc, 1);
 }
 
-// ... the K steps k0, k0 + 1 of the three products: issued as soon as the HALF of the A operand they read has been handed over
+// ... the K steps k0, k0 + 1 of the three products.  The service warp issues a chain GEMM as two of these in separate elect blocks:
+// its first MMA then leaves sooner after the hand-over than from one block of all 13 (DESIGN.md section 8b, svc-x).
 __device__ __forceinline__ void issue_split_ts_half(uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t b_hi, uint32_t b_lo, uint32_t idesc, int k0) {
 #pragma unroll
   for (int k = k0; k < k0 + 2; ++k) umma_f16_ts(d, a_lo + 8 * k, b_hi + 2 * k, kDescHi, idesc, 1);
@@ -143,7 +127,6 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 // expires, instead of re-issuing the try_wait / branch pair every ~100 cycles
 template <int NS>
 __device__ __forceinline__ void mbar_wait_hint(uint32_t bar, uint32_t parity) {
-  if (NS <= 0) { mbar_wait(bar, parity); return; }
   uint32_t ok;
   do {
     asm volatile(
@@ -158,19 +141,10 @@ __device__ __forceinline__ void mbar_wait_hint(uint32_t bar, uint32_t parity) {
   } while (!ok);
 }
 
-// ReLU + error-compensated fp16 split of two activations (tc_common.cuh: relu_split2) with the residual taken packed.
+// ReLU + error-compensated fp16 split of two activations with the residual taken packed.
 // (The mixed-precision FHFMA form of the residual, fma.rn.f32.f16, issues one instruction less but runs at a quarter of the
 // FMA rate: tools/cvt_rate.cu.)
 __device__ __forceinline__ void relu_split_pair(float x0, float x1, uint32_t& hi, uint32_t& lo) {
-#if RNF_T4_SPLIT_MASK == 2
-  // mixed: one value by the mask (ALU pipe), the other by the conversion (FMA pipe) -- ncu r02: ALU 40 %, FMA 23 % with both on the ALU
-  asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(x1), "f"(x0));
-  const float m0 = __uint_as_float(__float_as_uint(x0) & 0xFFFFE000u);
-  const float m1 = __high2float(*reinterpret_cast<const __half2*>(&hi));
-  float d0, d1;
-  upk(sub2(pk(x0, x1), pk(m0, m1)), d0, d1);
-  asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(d1), "f"(d0));
-#elif RNF_T4_SPLIT_MASK
   // The fp16 truncation of x, back in fp32, is x with its low 13 mantissa bits cleared: two LOP3 on the (half idle) ALU pipe
   // instead of two HADD2.F32 on the FMA pipe, which is the busiest pipe of this kernel (tools/pipe_rate.cu: every one of these
   // instructions costs 2 cycles per warp on its pipe).  hi is that masked value converted exactly (cvt.rn without satfinite),
@@ -182,21 +156,12 @@ __device__ __forceinline__ void relu_split_pair(float x0, float x1, uint32_t& hi
   float d0, d1;
   upk(sub2(pk(x0, x1), pk(m0, m1)), d0, d1);
   asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(d1), "f"(d0));
-#else
-  asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(x1), "f"(x0));
-  const float2 back = __half22float2(*reinterpret_cast<const __half2*>(&hi));
-  float d0, d1;
-  upk(sub2(pk(x0, x1), pk(back.x, back.y)), d0, d1);
-  asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(d1), "f"(d0));
-#endif
 }
 
 // Epilogue of one GEMM: my row of the accumulator -> (+ c) -> ReLU -> fp16 hi / lo -> A operand in TMEM (K element 2e in the
-// low half of column e).  All four 16-column loads are in flight before the first wait.  The accumulator is in registers after
-// the loads, so each HALF of the A operand (K elements 0..31, then 32..63) is handed over on its own: the service warp issues the
-// next GEMM's first two K steps under the arithmetic of the second half.
-template <typename HandOver1, typename HandOver2>
-__device__ __forceinline__ void epilogue64(uint32_t tm, const float* cadd, HandOver1&& hand_over_first, HandOver2&& hand_over_second) {
+// low half of column e).  All four 16-column loads are in flight before the first wait; the whole A operand is handed over at once.
+template <typename HandOver>
+__device__ __forceinline__ void epilogue64(uint32_t tm, const float* cadd, HandOver&& hand_over) {
   float a0[16], a1[16], a2[16], a3[16];
   tmem_ld16_async(tm + kColD, a0);
   tmem_ld16_async(tm + kColD + 16, a1);
@@ -222,15 +187,9 @@ __device__ __forceinline__ void epilogue64(uint32_t tm, const float* cadd, HandO
     }
     tmem_st16_nowait(tm + kColAhi + 16 * h, hi);
     tmem_st16_nowait(tm + kColAlo + 16 * h, lo);
-#if RNF_T4_HALF_EPI
-    tmem_st_wait();
-    if (h == 0) hand_over_first(); else hand_over_second();
-#endif
   }
-#if !RNF_T4_HALF_EPI
   tmem_st_wait();
-  hand_over_first();
-#endif
+  hand_over();
 }
 
 template <int N>
@@ -277,42 +236,22 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
   const uint32_t w_hid_d = umma_desc_lo(smem_u32(smem + kOffW)), w_last_d = umma_desc_lo(smem_u32(smem + kOffLastW));
   const uint32_t bias_hid_d = umma_desc_lo_ns(smem_u32(smem + kOffW + 16384)), bias_last_d = umma_desc_lo_ns(smem_u32(smem + kOffLastW + 65536));
   const uint32_t aux_blk_d = umma_desc_lo_ns(smem_u32(smem + kOffAux + kAuxFirst));
-  const uint32_t bar_mma = bars + 8 * (BAR_MMA + tile), bar_ready = bars + 8 * (BAR_READY + tile), bar_ready2 = bars + 8 * (BAR_READY2 + tile);
-  const int bar_wait = 9 + tile;                     // named barrier the tile's workers sleep in during a GEMM round trip
+  const uint32_t bar_mma = bars + 8 * (BAR_MMA + tile), bar_ready = bars + 8 * (BAR_READY + tile);
   constexpr uint32_t kIdesc = umma_idesc(128, 64);
   const uint32_t d = tm_tile + kColD;
   const int n_active = sc.n_active;
-  uint32_t par_mma = 0, par_ready = 0, par_ready2 = 0, par_w = 0;
+  uint32_t par_mma = 0, par_ready = 0, par_w = 0;
   int step = 0;
   int mob_cur = 0;
 
   auto wait_ready = [&]() {                          // the tile's four worker warps have handed over (Y block / A operand / drained D)
-    mbar_wait_hint<RNF_T4_SVC_HINT_NS>(bar_ready, par_ready);
+    mbar_wait(bar_ready, par_ready);
     par_ready ^= 1;
     tc_fence_after();
   };
-  auto wait_relaxed = [&](uint32_t bar, uint32_t parity) {   // a wait with slack (chunks 1..3, refill bookkeeping): naps between polls
-#if RNF_T4_SVC_NAP_NS > 0
-    while (!mbar_try_wait(bar, parity)) __nanosleep(RNF_T4_SVC_NAP_NS);
-#else
-    mbar_wait(bar, parity);
-#endif
-  };
-  auto wait_ready_second = [&]() {                   // ... second half of an epilogue
-    mbar_wait_hint<RNF_T4_SVC_HINT_NS>(bar_ready2, par_ready2);
-    par_ready2 ^= 1;
-    tc_fence_after();
-  };
-  auto wake_workers = [&]() {                        // the GEMM the workers sleep on has completed
-#if RNF_T4_DIRECT_WAIT_NS == 0
-    mbar_wait_hint<RNF_T4_SVC_HINT_NS>(bar_mma, par_mma);
+  auto wait_gemm = [&]() {                           // the workers watch the mbarrier themselves; this wait only orders the refill bookkeeping
+    mbar_wait(bar_mma, par_mma);
     par_mma ^= 1;
-    tc_fence_before();
-    named_arrive(bar_wait, 128 + 32);
-#else
-    wait_relaxed(bar_mma, par_mma);                  // the workers watch the mbarrier themselves; this wait only orders the refill bookkeeping
-    par_mma ^= 1;
-#endif
   };
 
   for (int item = 0; item < sc.my_items; ++item) {
@@ -329,7 +268,7 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
       for (int l = 0; l < 4; ++l) {
         if (l == 0) mbar_wait(bars + 8 * (BAR_AUX_FULL + abuf), (uint32_t)((step >> 1) & 1));
         else mbar_wait(bars + 8 * (BAR_W_FULL + l - 1), (par_w >> (l - 1)) & 1u);
-        wait_ready();                                // l == 0: Y block written; l > 0: first half of the A operand (K 0..31)
+        wait_ready();                                // l == 0: Y block written; l > 0: the A operand
         if (l == 0) {
           if (elect_one_sync()) {
             umma_f16(d, y_d, aux_blk_d + abuf * (kAuxStride >> 4), kDescHiNS, kIdesc, 0);
@@ -344,9 +283,6 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
             issue_split_ts_half(d, tm_tile + kColAhi, tm_tile + kColAlo, wb, wb + (8192 >> 4), kIdesc, 0);
           }
           __syncwarp();
-#if RNF_T4_HALF_EPI
-          wait_ready_second();                       // second half (K 32..63)
-#endif
           if (elect_one_sync()) {
             issue_split_ts_half(d, tm_tile + kColAhi, tm_tile + kColAlo, wb, wb + (8192 >> 4), kIdesc, 2);
             if (c_by_mma && l == 3) umma_f16(d, y_d, c_d, kDescHiNS, kIdesc, 1);
@@ -354,7 +290,7 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
           }
           __syncwarp();
         }
-        wake_workers();
+        wait_gemm();
         // a piece is dead once ALL tiles' GEMM that reads it has completed: the last tile to get here refills it
         if (lane == 0) {
           if (l == 0) { if ((atomicAdd(&s_cnt[4 + abuf], 1) % n_active) == n_active - 1 && step + 2 < sc.total_steps) load_piece(mob_n2, 4, abuf); }
@@ -368,9 +304,9 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
       for (int c = 0; c < 4; ++c) {
         const uint32_t wb = w_last_d + c * (8192 >> 4);                    // rows 64c .. 64c+63 of the hi plane
         if (c == 0) {
-          wait_ready();                              // (first half of) the last hidden epilogue
+          wait_ready();                              // the last hidden epilogue
         } else {                                     // chunk c - 1 drained into registers; the workers have ~1.5 k cycles of arithmetic left
-          wait_relaxed(bar_ready, par_ready);
+          mbar_wait(bar_ready, par_ready);
           par_ready ^= 1;
           tc_fence_after();
         }
@@ -380,9 +316,6 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
             issue_split_ts_half(d, tm_tile + kColAhi, tm_tile + kColAlo, wb, wb + (32768 >> 4), kIdesc, 0);
           }
           __syncwarp();
-#if RNF_T4_HALF_EPI
-          wait_ready_second();                       // second half
-#endif
           if (elect_one_sync()) {
             issue_split_ts_half(d, tm_tile + kColAhi, tm_tile + kColAlo, wb, wb + (32768 >> 4), kIdesc, 2);
             umma_commit(bar_mma);
@@ -397,12 +330,11 @@ __device__ __forceinline__ void service_warp(const FlowArgs& a, uint8_t* smem, c
           __syncwarp();
         }
         if (c == 0) {
-          wake_workers();
+          wait_gemm();
         } else if (c == 3) {
           // W4 is dead the moment the last chunk's MMAs have completed (not after the arithmetic on it): the last tile to see
           // that refills it.
-          wait_relaxed(bar_mma, par_mma);
-          par_mma ^= 1;
+          wait_gemm();
           if (lane == 0 && (atomicAdd(&s_cnt[3], 1) % n_active) == n_active - 1 && step + 1 < sc.total_steps) load_piece(mob_n1, 3, 0);
           __syncwarp();
         } else {
@@ -465,15 +397,14 @@ __global__ void __launch_bounds__(kThreads, 1) flow_t4_kernel(const FlowArgs a) 
   sc.total_steps = sc.my_items * n_mob;
 
   if (service) {
-    set_max_regs_dec<RNF_T4_SERVICE_REGS>();
+    set_max_regs_dec<kServiceRegs>();
     service_warp<GRID>(a, smem, tmem_base, tile, lane, sc, n_mob, s_moff, s_cnt);
   } else {
-    set_max_regs_inc<RNF_T4_WORKER_REGS>();
+    set_max_regs_inc<kWorkerRegs>();
     const uint32_t tm = tmem_base + (uint32_t)tile * kColsPerTile + ((uint32_t)((warp & 3) * 32) << 16);   // my warp's lane quarter
     uint8_t* y_blk = smem + kOffY + tile * 4096;
     uint8_t* c_blk = smem + kOffC + tile * 2048;
-    const int bar_wait = 9 + tile;                     // named barrier: the tile's workers sleep here during a GEMM round trip
-    const uint32_t bar_mma = bars + 8 * (BAR_MMA + tile), bar_ready = bars + 8 * (BAR_READY + tile), bar_ready2 = bars + 8 * (BAR_READY2 + tile);
+    const uint32_t bar_mma = bars + 8 * (BAR_MMA + tile), bar_ready = bars + 8 * (BAR_READY + tile);
     uint32_t par_mma = 0;
 #if RNF_TC_TRACE
     int64_t step = 0;
@@ -486,21 +417,11 @@ __global__ void __launch_bounds__(kThreads, 1) flow_t4_kernel(const FlowArgs a) 
       __syncwarp();
       if (lane == 0) mbar_arrive(bar_ready);
     };
-    auto hand_over_second = [&]() {                    // second half of an epilogue (its own mbarrier, see BAR_READY2)
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(bar_ready2);
-    };
-    // Wait for a GEMM that the tile cannot overlap with anything (the dependent round trips of the chain).  Default: every worker
-    // warp watches the MMA's mbarrier itself (try_wait with a suspend hint).  Alternative (RNF_T4_DIRECT_WAIT_NS = 0): the workers
-    // sleep in a hardware named barrier that the service warp arrives on once its own poll of the mbarrier succeeds -- no polling
-    // by the workers, but a second wake-up hop on the critical path (measured ~1 % slower in cycles, tools/ab_ncu.sh).
+    // Wait for a GEMM that the tile cannot overlap with anything (the dependent round trips of the chain): every worker warp
+    // watches the MMA's mbarrier itself (try_wait with a suspend hint).  Sleeping in a named barrier that the service warp
+    // arrives on instead adds a second wake-up hop to the critical path (measured ~1 % slower in cycles, DESIGN.md svc-x).
     auto wait_mma_long = [&]() {
-#if RNF_T4_DIRECT_WAIT_NS > 0
-      mbar_wait_hint<RNF_T4_DIRECT_WAIT_NS>(bar_mma, par_mma);
-#else
-      named_bar(bar_wait, 128 + 32);
-#endif
+      mbar_wait_hint<kDirectWaitNs>(bar_mma, par_mma);
       par_mma ^= 1;
       tc_fence_after();
     };
@@ -608,7 +529,7 @@ __global__ void __launch_bounds__(kThreads, 1) flow_t4_kernel(const FlowArgs a) 
           wait_mma_long();
           TRACE(3 + 3 * l);
           const float* ca = (l == 0 || l == 3) ? cadd : nullptr;
-          epilogue64(tm, ca, hand_over, hand_over_second);
+          epilogue64(tm, ca, hand_over);
           TRACE(4 + 3 * l);
         }
         // ---- fc_last in four N = 64 chunks through the single accumulator; 16 mixture components per chunk ----

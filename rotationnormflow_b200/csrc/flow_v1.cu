@@ -24,23 +24,6 @@ constexpr int T = kV1Threads;                      // rotations per CTA
 constexpr int kSmemFloats = kMobFloats + kH * T;   // weights + private activation columns
 constexpr int kScratchPerCta = 4 * kK * T;         // inverse: (w.x, w.y, w.z, softplus) per component per thread
 
-__device__ __forceinline__ float sel3(int p, float a, float b, float c) { return p == 0 ? a : (p == 1 ? b : c); }
-
-__device__ __forceinline__ void get_col(const float R[9], int p, float o[3]) {
-  o[0] = sel3(p, R[0], R[1], R[2]);
-  o[1] = sel3(p, R[3], R[4], R[5]);
-  o[2] = sel3(p, R[6], R[7], R[8]);
-}
-
-__device__ __forceinline__ void set_col(float R[9], int p, const float c[3]) {
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    R[3 * i + 0] = p == 0 ? c[i] : R[3 * i + 0];
-    R[3 * i + 1] = p == 1 ? c[i] : R[3 * i + 1];
-    R[3 * i + 2] = p == 2 ? c[i] : R[3 * i + 2];
-  }
-}
-
 // first conditioner layer for output j: W0[j,:3].y + b0[j] (+ hoisted per-image W_f.feature)
 __device__ __forceinline__ float first_layer(const float4* sFirst, const float* cimg, int j, const float y[3]) {
   const float4 f = sFirst[j];

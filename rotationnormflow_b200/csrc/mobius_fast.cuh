@@ -1,15 +1,15 @@
-// mobius_fast.cuh -- the Mobius mixture arithmetic in the (r, v) plane with single-instruction SFU primitives.
+// mobius_fast.cuh -- single-instruction SFU primitives and the per-row frame of the tensor-core flow kernels.
 //
-// Same mathematics as mobius_math.cuh (flow/mobiusflow.py:17-24,62-72,94-125,196-245), restated so that one mixture
-// component costs ~70 instructions instead of ~190:
+// Same mathematics as mobius_math.cuh (flow/mobiusflow.py:17-24,62-72,94-125,196-245), restated for the Mobius layers of
+// flow_t4.cu and flow_row.cu, whose mixture arithmetic is in mobius_pair.cuh:
 //   * every w_k is projected onto the plane orthogonal to y (flow/mobiusflow.py:62-63) and r, v span that plane, so the
 //     projected centre is (alpha, beta) = (w.r, w.v): the projection, the 3-D norms and the two 3-D dot products of
 //     h with (r, v) collapse to 2-D arithmetic (the reference's own frame is orthonormal to ~1e-7, the same order as one
 //     fp32 rounding of these quantities);
 //   * 1/x, sqrt, 2^x, log2 use the SFU approximations (rcp/sqrt.approx: <= 1 ulp; ex2/lg2.approx: ~2^-22), whose errors
-//     enter theta' = sum_k pi_k theta_k and log sum_k pi_k f_k averaged over the 64 components;
-//   * atan2 + wrap to [0, 2 pi) is a branch-free min/max reduction with a degree-8 minimax polynomial in q^2
-//     (max error 7.6e-8 rad = 1.3 ulp on [0,1], fitted and verified against float64 in tests/test_fastmath.py).
+//     enter theta' = sum_k pi_k theta_k and log sum_k pi_k f_k averaged over the 64 components.
+// The scalar mixture that mobius_pair.cuh replaced (atan2 polynomial, softplus, four components stage by stage) was removed;
+// its code is in commit d73682a.
 // Accuracy against the float64 reference is asserted end-to-end by tests/test_gpu_parity.py in "tc" mode.
 #pragma once
 #include <cuda_runtime.h>
@@ -69,68 +69,6 @@ __device__ __forceinline__ void sincos_2pi(float t, float& sn, float& cs) {
   cs = ((q + 1) & 2) ? -b : b;
 }
 
-// Mixture weight of a component, in units of ln 2:  softplus(a) / ln 2 = log2(1 + 2^t),  t = a log2(e).
-// theta' = sum_k sp_k theta_k / sum_k sp_k and log sum_k sp_k f_k / sum_k sp_k are ratios, so the common factor ln 2
-// never has to be applied.  torch's softplus is the identity above a = 20 (threshold), i.e. t above 20 log2(e); for
-// 2^t < 2^-7 the series e (1 - e/2) / ln 2 replaces log2(1 + e), whose argument would round away e (absolute error of the
-// weight <= 2e-7 either way: what matters is the error relative to the sum of the 64 weights).
-__device__ __forceinline__ float softplus_log2(float a) {
-  const float t = a * 1.4426950408889634f;
-  const float e = ex2_approx(t);
-  const float big = lg2_approx(1.0f + e);
-  const float small = e * fmaf(e, -0.7213475204444817f, 1.4426950408889634f);
-  const float sp = e < 0.0078125f ? small : big;
-  return t > 28.853900817779268f ? t : sp;
-}
-
-// softplus(a) = log(1 + e^a) itself (same construction, natural units).
-__device__ __forceinline__ float softplus_fast(float a) { return 0.6931471805599453f * softplus_log2(a); }
-
-// atan2(y, x) wrapped to [0, 2 pi)  == torch.where(t >= 0, t, t + 2 pi) of flow/mobiusflow.py:94-99.
-__device__ __forceinline__ float atan2_wrapped_fast(float y, float x) {
-  const float ay = fabsf(y), ax = fabsf(x);
-  const float mx = fmaxf(ay, ax), mn = fminf(ay, ax);
-  const float q = mn * rcp_approx(mx);
-  const float s = q * q;
-  float p = -0.0024470302741974592f;                  // degree-8 minimax polynomial in s (Horner: fewest instructions;
-  p = fmaf(p, s, 0.013750280253589153f);              // an Estrin split measured 3 % slower -- the kernel is issue bound)
-  p = fmaf(p, s, -0.03627016767859459f);
-  p = fmaf(p, s, 0.06284360587596893f);
-  p = fmaf(p, s, -0.08673170208930969f);
-  p = fmaf(p, s, 0.11037994176149368f);
-  p = fmaf(p, s, -0.14279110729694366f);
-  p = fmaf(p, s, 0.1999976634979248f);
-  p = fmaf(p, s, -0.3333333134651184f);
-  p = p * s;
-  p = fmaf(p, q, q);                                  // atan(q), q in [0,1]
-  p = ay > ax ? 1.5707963267948966f - p : p;          // first octant pair
-  p = x < 0.0f ? kPi - p : p;                         // angle in [0, pi] of (|y|, x)
-  return y < 0.0f ? kTwoPi - p : p;
-}
-
-// Forward direction only: the evaluation point is the moving column itself, z = -|x| r, and |w| < 0.7 by construction
-// (flow/mobiusflow.py:72), so h_w(z) stays within +-2 asin(0.7) of the angle pi (SURVEY.md A.3 step 7): x < 0 always and the
-// wrapped angle is pi - atan(y / |x|).  One select fewer than the full-circle version.
-__device__ __forceinline__ float atan2_left_half_plane(float y, float x) {
-  const float ay = fabsf(y), ax = fabsf(x);
-  const float mx = fmaxf(ay, ax), mn = fminf(ay, ax);
-  const float q = mn * rcp_approx(mx);
-  const float s = q * q;
-  float p = -0.0024470302741974592f;
-  p = fmaf(p, s, 0.013750280253589153f);
-  p = fmaf(p, s, -0.03627016767859459f);
-  p = fmaf(p, s, 0.06284360587596893f);
-  p = fmaf(p, s, -0.08673170208930969f);
-  p = fmaf(p, s, 0.11037994176149368f);
-  p = fmaf(p, s, -0.14279110729694366f);
-  p = fmaf(p, s, 0.1999976634979248f);
-  p = fmaf(p, s, -0.3333333134651184f);
-  p = p * s;
-  p = fmaf(p, q, q);                                  // atan(q), q in [0,1]
-  p = ay > ax ? 1.5707963267948966f - p : p;          // atan(|y| / |x|)
-  return y < 0.0f ? kPi + p : kPi - p;
-}
-
 // point on the circle: z = r cos(t) + v sin(t), t in [0, 2 pi]            (flow/mobiusflow.py:102,169,231)
 __device__ __forceinline__ void circle_point_fast(const float r[3], const float v[3], float t, float z[3]) {
   float s, c;
@@ -152,167 +90,5 @@ __device__ __forceinline__ void make_frame_fast(const float x[3], const float y[
   cross3(y, P.r, P.v);
   normalize3_fast(P.v);
 }
-
-// raw conditioner output w (3-D) -> prepared in-plane centre (alpha', beta') with |.| < 0.7, and 1 - |w'|^2.
-__device__ __forceinline__ void comp_prep2(const Plane& P, float w0, float w1, float w2, float& al, float& be, float& omw) {
-  const float a = fmaf(w2, P.r[2], fmaf(w1, P.r[1], w0 * P.r[0]));
-  const float b = fmaf(w2, P.v[2], fmaf(w1, P.v[1], w0 * P.v[0]));
-  const float n2 = fmaf(b, b, a * a);
-  const float s = 0.7f * rcp_approx(1.0f + sqrt_approx(n2));
-  al = s * a;
-  be = s * b;
-  omw = fmaf(-be, be, fmaf(-al, al, 1.0f));
-}
-
-// Mobius map of the in-plane point (zr, zv): wrapped angle of h and f = |dh/dtheta| = (1 - |w|^2)/|z - w|^2.
-__device__ __forceinline__ void comp_eval2(float zr, float zv, float al, float be, float omw, float& theta, float& f) {
-  const float dr = zr - al, dv = zv - be;
-  const float dd = fmaf(dv, dv, dr * dr);
-  f = omw * rcp_approx(dd);
-  const float hr = fmaf(f, dr, -al), hv = fmaf(f, dv, -be);
-  theta = atan2_wrapped_fast(hv, hr);
-}
-
-// forward-direction variant of comp_eval2 (evaluation point = the moving column: h always in the left half plane)
-__device__ __forceinline__ void comp_eval2_fwd(float zr, float zv, float al, float be, float omw, float& theta, float& f) {
-  const float dr = zr - al, dv = zv - be;
-  const float dd = fmaf(dv, dv, dr * dr);
-  f = omw * rcp_approx(dd);
-  const float hr = fmaf(f, dr, -al), hv = fmaf(f, dv, -be);
-  theta = atan2_left_half_plane(hv, hr);
-}
-
-__device__ __forceinline__ float comp_f2(float zr, float zv, float al, float be, float omw) {
-  const float dr = zr - al, dv = zv - be;
-  return omw * rcp_approx(fmaf(dv, dv, dr * dr));
-}
-
-
-// Four mixture components at once, written stage by stage (structure-of-arrays) so that the four independent dependency
-// chains (~200 cycles deep each: EX2 -> LG2, SQRT -> RCP -> RCP -> RCP -> 9-term Horner) are issued interleaved; ptxas keeps
-// the component-by-component order of a plain loop and leaves a warp with an ILP of ~1.5.
-// raw[16] = (logit, w.x, w.y, w.z) x 4 as they come out of the fc_last GEMM.  FWD: accumulates the three mixture sums.
-// !FWD: overwrites raw with the prepared parameters (alpha', beta', 1 - |w'|^2, weight) for the bisection.
-template <int N, bool FWD>
-__device__ __forceinline__ void mixtureN(const Plane& P, float zr, float zv, float* raw, float& S_sp, float& S_th, float& S_f) {
-  float sp[N], al[N], be[N], omw[N];
-  {
-    float t[N], e[N], a[N], b[N], n2[N], rt[N], s[N];
-#pragma unroll
-    for (int k = 0; k < N; ++k) { t[k] = raw[4 * k] * 1.4426950408889634f; e[k] = ex2_approx(t[k]); }
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      a[k] = fmaf(raw[4 * k + 3], P.r[2], fmaf(raw[4 * k + 2], P.r[1], raw[4 * k + 1] * P.r[0]));
-      b[k] = fmaf(raw[4 * k + 3], P.v[2], fmaf(raw[4 * k + 2], P.v[1], raw[4 * k + 1] * P.v[0]));
-      n2[k] = fmaf(b[k], b[k], a[k] * a[k]);
-    }
-#pragma unroll
-    for (int k = 0; k < N; ++k) rt[k] = sqrt_approx(n2[k]);
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      const float big = lg2_approx(1.0f + e[k]);
-      const float small = e[k] * fmaf(e[k], -0.7213475204444817f, 1.4426950408889634f);
-      const float v = e[k] < 0.0078125f ? small : big;
-      sp[k] = t[k] > 28.853900817779268f ? t[k] : v;
-    }
-#pragma unroll
-    for (int k = 0; k < N; ++k) s[k] = 0.7f * rcp_approx(1.0f + rt[k]);
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      al[k] = s[k] * a[k];
-      be[k] = s[k] * b[k];
-      omw[k] = fmaf(-be[k], be[k], fmaf(-al[k], al[k], 1.0f));
-    }
-  }
-  if (FWD) {
-    float f[N], hr[N], hv[N], q[N], p[N], ay[N], ax[N];
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      const float dr = zr - al[k], dv = zv - be[k];
-      f[k] = omw[k] * rcp_approx(fmaf(dv, dv, dr * dr));
-      hr[k] = fmaf(f[k], dr, -al[k]);
-      hv[k] = fmaf(f[k], dv, -be[k]);
-      ay[k] = fabsf(hv[k]);
-      ax[k] = fabsf(hr[k]);
-    }
-#pragma unroll
-    for (int k = 0; k < N; ++k) q[k] = fminf(ay[k], ax[k]) * rcp_approx(fmaxf(ay[k], ax[k]));
-#pragma unroll
-    for (int k = 0; k < N; ++k) p[k] = -0.0024470302741974592f;
-    // Horner over the four components in lock step (same coefficients as atan2_wrapped_fast)
-#define RNF_HORNER(cf) _Pragma("unroll") for (int k = 0; k < N; ++k) p[k] = fmaf(p[k], q[k] * q[k], cf)
-    RNF_HORNER(0.013750280253589153f);
-    RNF_HORNER(-0.03627016767859459f);
-    RNF_HORNER(0.06284360587596893f);
-    RNF_HORNER(-0.08673170208930969f);
-    RNF_HORNER(0.11037994176149368f);
-    RNF_HORNER(-0.14279110729694366f);
-    RNF_HORNER(0.1999976634979248f);
-    RNF_HORNER(-0.3333333134651184f);
-#undef RNF_HORNER
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      float at = fmaf(p[k] * (q[k] * q[k]), q[k], q[k]);          // atan(q), q in [0,1]
-      at = ay[k] > ax[k] ? 1.5707963267948966f - at : at;          // atan(|hv| / |hr|); hr < 0 always in the forward direction
-      const float th = hv[k] < 0.0f ? kPi + at : kPi - at;
-      S_sp += sp[k];
-      S_th = fmaf(sp[k], th, S_th);
-      S_f = fmaf(sp[k], f[k], S_f);
-    }
-  } else {
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-      S_sp += sp[k];
-      raw[4 * k] = al[k]; raw[4 * k + 1] = be[k]; raw[4 * k + 2] = omw[k]; raw[4 * k + 3] = sp[k];
-    }
-  }
-}
-
-template <bool FWD>
-__device__ __forceinline__ void mixture4(const Plane& P, float zr, float zv, float raw[16], float& S_sp, float& S_th, float& S_f) {
-  mixtureN<4, FWD>(P, zr, zv, raw, S_sp, S_th, S_f);
-}
-
-// Bisection probe of four prepared components at the in-plane point (zr, zv) = (cos t, sin t): stage-wise like mixture4.
-// prm[16] = (alpha', beta', 1 - |w'|^2, weight) x 4; accumulates sum_k weight_k theta_k(z).  Full-circle atan2: during the
-// bisection z sweeps [pi/2, 3pi/2] and h may land anywhere (flow/mobiusflow.py:226-245).
-template <int N>
-__device__ __forceinline__ void probeN(float zr, float zv, const float* prm, float& Fs) {
-  float hr[N], hv[N], ay[N], ax[N], q[N], p[N];
-#pragma unroll
-  for (int k = 0; k < N; ++k) {
-    const float al = prm[4 * k], be = prm[4 * k + 1];
-    const float dr = zr - al, dv = zv - be;
-    const float f = prm[4 * k + 2] * rcp_approx(fmaf(dv, dv, dr * dr));
-    hr[k] = fmaf(f, dr, -al);
-    hv[k] = fmaf(f, dv, -be);
-    ay[k] = fabsf(hv[k]);
-    ax[k] = fabsf(hr[k]);
-  }
-#pragma unroll
-  for (int k = 0; k < N; ++k) q[k] = fminf(ay[k], ax[k]) * rcp_approx(fmaxf(ay[k], ax[k]));
-#pragma unroll
-  for (int k = 0; k < N; ++k) p[k] = -0.0024470302741974592f;
-#define RNF_HORNER(cf) _Pragma("unroll") for (int k = 0; k < N; ++k) p[k] = fmaf(p[k], q[k] * q[k], cf)
-  RNF_HORNER(0.013750280253589153f);
-  RNF_HORNER(-0.03627016767859459f);
-  RNF_HORNER(0.06284360587596893f);
-  RNF_HORNER(-0.08673170208930969f);
-  RNF_HORNER(0.11037994176149368f);
-  RNF_HORNER(-0.14279110729694366f);
-  RNF_HORNER(0.1999976634979248f);
-  RNF_HORNER(-0.3333333134651184f);
-#undef RNF_HORNER
-#pragma unroll
-  for (int k = 0; k < N; ++k) {
-    float at = fmaf(p[k] * (q[k] * q[k]), q[k], q[k]);
-    at = ay[k] > ax[k] ? 1.5707963267948966f - at : at;
-    at = hr[k] < 0.0f ? kPi - at : at;
-    const float th = hv[k] < 0.0f ? kTwoPi - at : at;
-    Fs = fmaf(prm[4 * k + 3], th, Fs);
-  }
-}
-
-__device__ __forceinline__ void probe4(float zr, float zv, const float prm[16], float& Fs) { probeN<4>(zr, zv, prm, Fs); }
 
 }  // namespace rnf

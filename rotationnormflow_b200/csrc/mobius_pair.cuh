@@ -9,23 +9,13 @@
 // Column layout of one pair (the host permutes the fc_last rows accordingly, engine._last_layer_perm_pairs): 8 consecutive
 // accumulator columns  (t_a, t_b, wx_a, wx_b, wy_a, wy_b, wz_a, wz_b)  with t = logit * log2(e) and w = 0.7 * centre (both factors are
 // folded into the weights), so that a tcgen05.ld vector delivers every packed operand as an aligned register pair.
-// Prepared parameters of a pair (inverse direction, kept in TMEM for the bisection):
+// Prepared parameters of a pair (inverse direction, kept in TMEM for the root search):
 //   (-alpha'_a, -alpha'_b, -beta'_a, -beta'_b, 1 - |w'_a|^2, 1 - |w'_b|^2, weight_a, weight_b).
+// The variants that lost or were superseded (logit clamp instead of the softplus select, degree-5 asin, two reciprocals + atan
+// in the forward mixture, the inverse's probes with the full-circle angle wrap; DESIGN.md section 8b) were removed; their code
+// is in commit d73682a.
 #pragma once
 #include "mobius_fast.cuh"
-
-#ifndef RNF_INV_MS_FROM_M
-#define RNF_INV_MS_FROM_M 1           // sin^2 delta as m * m (one multiply less per pair and evaluation: -1.5 % cycles of the inverse kernel)
-#endif
-#ifndef RNF_MIX_CLAMP
-#define RNF_MIX_CLAMP 0          // 1: logit clamped at 127 (log2 units) before ex2 instead of the  t > 28.85 ? t : ...  select
-#endif
-#ifndef RNF_ASIN_DEG
-#define RNF_ASIN_DEG 6           // degree of P in asin(m) = m + m s P(s): 6 -> 4.6e-8, 5 -> 8.9e-8 max abs error in fp32 Horner form
-#endif
-#ifndef RNF_MIX_RSQ
-#define RNF_MIX_RSQ 1            // forward mixture: rsqrt + asin (8 SFU operations per pair) instead of two reciprocals + atan (10)
-#endif
 
 namespace rnf {
 
@@ -58,8 +48,6 @@ __device__ __forceinline__ f32x2 sub2(f32x2 a, f32x2 b) {
   asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
-// sign flip of both halves: a bit operation that ptxas folds into the negate modifier of the consuming FFMA2 / FADD2
-__device__ __forceinline__ f32x2 neg2(f32x2 a) { return a ^ 0x8000000080000000ull; }
 __device__ __forceinline__ float hsum(f32x2 v) {
   float lo, hi;
   upk(v, lo, hi);
@@ -67,23 +55,11 @@ __device__ __forceinline__ float hsum(f32x2 v) {
 }
 #define RNF_MAP2(out, in, fn) do { float l_, h_; upk(in, l_, h_); out = pk(fn(l_), fn(h_)); } while (0)
 
-// Angle of a UNIT vector from its nearer axis, for a pair: asin(m) with m = min(|h.r|, |h.v|) in [0, 1/sqrt 2].  The Mobius map
-// sends the unit circle to itself, so |h| = 1 (to fp32 rounding) and atan(min / max) = asin(min): no reciprocal on the SFU --
-// the XU pipe (8 cycles per warp instruction, tools/mufu_rate.cu) is the tightest unit of the mixture -- and a shorter
-// polynomial: asin(m) = m + m s P(s), s = m^2, P of degree 6 (minimax fit, max abs error 4.4e-8 in fp32 Horner form,
-// tests/test_fastmath.py).
-__device__ __forceinline__ f32x2 asin_unit2_s(f32x2 m, f32x2 s);
-__device__ __forceinline__ f32x2 asin_unit2(f32x2 m) { return asin_unit2_s(m, mul2(m, m)); }
-// ... with s = m^2 supplied by the caller
+// asin(m) for a pair, |m| <= 1/sqrt 2, with s = m^2 supplied by the caller.  The angles of the mixture are asin of a sine
+// (|sin| <= 0.7, see mixture_pairs and probe_delta_pairs) instead of atan of a quotient: no reciprocal on the SFU -- the XU pipe
+// (8 cycles per warp instruction, tools/mufu_rate.cu) is the tightest unit of the mixture -- and a shorter polynomial:
+// asin(m) = m + m s P(s), P of degree 6 (minimax fit, max abs error 4.4e-8 in fp32 Horner form, tests/test_fastmath.py).
 __device__ __forceinline__ f32x2 asin_unit2_s(f32x2 m, f32x2 s) {
-#if RNF_ASIN_DEG == 5
-  f32x2 p = bc(0.11149732023477554f);
-  p = fma2(p, s, bc(-0.07131081074476242f));
-  p = fma2(p, s, bc(0.07036406546831131f));
-  p = fma2(p, s, bc(0.036296285688877106f));
-  p = fma2(p, s, bc(0.07581107318401337f));
-  p = fma2(p, s, bc(0.1666388362646103f));
-#else
   f32x2 p = bc(0.12371734529733658f);
   p = fma2(p, s, bc(-0.11529727280139923f));
   p = fma2(p, s, bc(0.09339626878499985f));
@@ -91,39 +67,27 @@ __device__ __forceinline__ f32x2 asin_unit2_s(f32x2 m, f32x2 s) {
   p = fma2(p, s, bc(0.04762402921915054f));
   p = fma2(p, s, bc(0.07478351145982742f));
   p = fma2(p, s, bc(0.16667234897613525f));
-#endif
   return fma2(mul2(p, s), m, m);
-}
-
-// atan on the half-angle range of the forward direction: |q| <= tan(asin 0.7) = 0.9802 (see mixture_pairs).
-// atan(q) = q + q s P(s), s = q^2, P of degree 7 (minimax fit of the absolute error, tools/fit_atan_half.py: 5.6e-9 exact,
-// 6.1e-8 in fp32 Horner form, tests/test_fastmath.py).
-__device__ __forceinline__ f32x2 atan_half2(f32x2 q) {
-  const f32x2 s = mul2(q, q);
-  f32x2 p = bc(0.0028766694f);
-  p = fma2(p, s, bc(-0.01609694f));
-  p = fma2(p, s, bc(0.04260853f));
-  p = fma2(p, s, bc(-0.07486252f));
-  p = fma2(p, s, bc(0.10627319f));
-  p = fma2(p, s, bc(-0.14198953f));
-  p = fma2(p, s, bc(0.1999194f));
-  p = fma2(p, s, bc(-0.33333054f));
-  return fma2(mul2(p, s), q, q);
 }
 
 // NP pairs of mixture components, stage by stage.  raw[8 NP]: accumulator columns in the pair layout above; the centre rows
 // arrive PRE-SCALED by 0.7 (engine.pack_mobius_tc), so with (a', b') = 0.7 (w.r, w.v) and u = 1 + |w| = 1 + |(a', b')| / 0.7
 // the squashed centre of flow/mobiusflow.py:72 is w' = (a', b') / u.
+// Mixture weight of a component, in units of ln 2:  softplus(a) / ln 2 = log2(1 + 2^t),  t = a log2(e).  theta' and
+// log sum_k w_k f_k / sum_k w_k are ratios, so the common factor ln 2 never has to be applied.  torch's softplus is the
+// identity above a = 20 (threshold), i.e. t above 20 log2(e) = 28.85; for 2^t < 2^-7 the series e (1 - e/2) / ln 2 replaces
+// log2(1 + e), whose argument would round away e (absolute error of the weight <= 2e-7 either way: what matters is the error
+// relative to the sum of the 64 weights).
 // FWD: the evaluation point is the moving column itself, z = (zr, 0) with zr = -|x|, a point of the unit circle, on which the
 // map of flow/mobiusflow.py:17-24 is the disk automorphism h = (z - w') / (1 - conj(w') z) (complex notation), so that
 //     arg h = 2 arg(z - w') - arg z = 2 arg(z - w') - pi.
 // Scaled by u (no reciprocal of u):  D = u (z - w') = (zr u - a', -b') =: (-Dn, -b'),  Dn > 0.3 u,  arg(z - w') = pi + atan(b' / Dn):
 //     theta = pi + 2 atan(q),  q = b' / Dn,  |q| < tan(asin 0.7);   sum_k w_k theta_k = pi sum_k w_k + 2 sum_k w_k atan(q_k)
-// -- one division, no octant selects, and the angle does not wait for f.  The log-det term needs
+// -- no octant selects, and the angle does not wait for f (atan(q) is taken as asin(b' / |D|), see below).  The log-det term needs
 //     f = (1 - |w'|^2) / |z - w'|^2 = (u^2 - |(a',b')|^2) / |D|^2,   |D|^2 = Dn^2 + b'^2.
 // Accumulates (sum w, sum w atan q, sum w f) as packed partial sums (a-components in the low, b in the high word).
-// !FWD: accumulates sum w (S_sp), sum w (-alpha') (S_at), sum w (-beta') (S_f) and overwrites raw with the prepared parameters
-// (-alpha', -beta', 1 - |w'|^2, weight).
+// !FWD: accumulates sum w (S_sp) and overwrites raw with the prepared parameters (-alpha', -beta', 1 - |w'|^2, weight);
+// S_at and S_f are left as they are.
 template <int NP, bool FWD>
 __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv, float* raw, f32x2& S_sp, f32x2& S_at, f32x2& S_f) {
   f32x2 sp[NP], ap[NP], bp[NP], bb[NP], n2[NP], u[NP], rt[NP];
@@ -131,13 +95,7 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
     f32x2 t[NP], e[NP], big[NP], small[NP];
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
-#if RNF_MIX_CLAMP
-      // lg2(1 + 2^t) = t to fp32 precision for t > 25, so the only job of the reference's  x > 20 ? x : log1p(exp(x))  branch
-      // (torch softplus threshold) is to avoid the overflow of 2^t: clamp t instead of selecting afterwards.
-      t[j] = pk(fminf(raw[8 * j], 127.0f), fminf(raw[8 * j + 1], 127.0f));
-#else
       t[j] = pk(raw[8 * j], raw[8 * j + 1]);
-#endif
       RNF_MAP2(e[j], t[j], ex2_approx);
     }
 #pragma unroll
@@ -161,18 +119,11 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
       float tl, th, el, eh, bl, bh, sl, sh;
       upk(t[j], tl, th); upk(e[j], el, eh); upk(big[j], bl, bh); upk(small[j], sl, sh);
       const float vl = el < 0.0078125f ? sl : bl, vh = eh < 0.0078125f ? sh : bh;
-#if RNF_MIX_CLAMP
-      sp[j] = pk(vl, vh);
-#else
       sp[j] = pk(tl > 28.853900817779268f ? tl : vl, th > 28.853900817779268f ? th : vh);
-#endif
     }
   }
   if (FWD) {
-    f32x2 f[NP], q[NP];
-#if RNF_MIX_RSQ
-    f32x2 qs[NP];
-#endif
+    f32x2 f[NP], q[NP], qs[NP];
     const f32x2 nzr = bc(-zr);
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
@@ -181,7 +132,6 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
       const f32x2 DD = fma2(Dn, Dn, bb[j]);
       // u^2 - |(a',b')|^2 with |(a',b')| = rt:  1 + (2 / 0.7) rt + (1 / 0.49 - 1) rt^2  -- all terms positive
       const f32x2 num = fma2(fma2(rt[j], bc(1.0408163265306123f), bc(2.857142857142857f)), rt[j], bc(1.0f));
-#if RNF_MIX_RSQ
       // ONE SFU operation per component instead of two reciprocals (the XU pipe, 8 cycles per warp instruction, is the tightest
       // unit of the mixture: 10 -> 8 MUFU per pair): with rs = 1 / |D|,  sin(arg) = b' rs  and  1 / |D|^2 = rs^2, and since
       // Dn > 0 the angle atan(b' / Dn) = asin(b' rs), |b' rs| <= 0.7 (the squashed centre stays inside the disk of radius 0.7).
@@ -191,21 +141,10 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
       f[j] = mul2(num, rs2);
       q[j] = mul2(bp[j], rs);
       qs[j] = mul2(bb[j], rs2);
-#else
-      f32x2 rc, rcd;
-      RNF_MAP2(rc, DD, rcp_approx);
-      RNF_MAP2(rcd, Dn, rcp_approx);
-      f[j] = mul2(num, rc);
-      q[j] = mul2(bp[j], rcd);
-#endif
     }
     f32x2 at[NP];
 #pragma unroll
-#if RNF_MIX_RSQ
     for (int j = 0; j < NP; ++j) at[j] = asin_unit2_s(q[j], qs[j]);
-#else
-    for (int j = 0; j < NP; ++j) at[j] = atan_half2(q[j]);
-#endif
 #pragma unroll
     for (int j = 0; j < NP; ++j) {
       S_sp = add2(S_sp, sp[j]);
@@ -222,8 +161,6 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
       const f32x2 nal = mul2(ap[j], nrc), nbe = mul2(bp[j], nrc);
       const f32x2 omw = fma2(fma2(nal, nal, mul2(nbe, nbe)), bc(-1.0f), bc(1.0f));      // 1 - |w'|^2
       S_sp = add2(S_sp, sp[j]);
-      S_at = fma2(sp[j], nal, S_at);                 // sum weight (-alpha'), sum weight (-beta'): the weighted mean centre, from which the
-      S_f = fma2(sp[j], nbe, S_f);                   // inverse direction takes the starting point of its root search (flow_row.cu)
       upk(nal, raw[8 * j], raw[8 * j + 1]);
       upk(nbe, raw[8 * j + 2], raw[8 * j + 3]);
       upk(omw, raw[8 * j + 4], raw[8 * j + 5]);
@@ -234,52 +171,6 @@ __device__ __forceinline__ void mixture_pairs(const Plane& P, float zr, float zv
 
 // wrapped mixture angle theta' = sum_k w_k theta_k / sum_k w_k from the forward sums of mixture_pairs
 __device__ __forceinline__ float mixture_angle(float S_at, float inv_sp) { return fmaf(2.0f * S_at, inv_sp, kPi); }
-
-// Bisection probe of NP prepared pairs at the in-plane point (zr, zv) = (cos t, sin t): accumulates sum_k weight_k theta_k(z).
-// Full-circle atan2: during the bisection z sweeps [pi/2, 3pi/2] and h may land anywhere (flow/mobiusflow.py:226-245).
-// DERIV: also accumulates sum_k weight_k f_k(z) = d/dt of the sum above (each component is a circle map with derivative f_k).
-template <int NP, bool DERIV = false>
-__device__ __forceinline__ void probe_pairs(float zr, float zv, const float* prm, f32x2& Fs, f32x2* Sf = nullptr) {
-  f32x2 mn[NP];
-  float hr_[2 * NP], hv_[2 * NP];
-#pragma unroll
-  for (int j = 0; j < NP; ++j) {
-    const f32x2 nal = pk(prm[8 * j], prm[8 * j + 1]), nbe = pk(prm[8 * j + 2], prm[8 * j + 3]), omw = pk(prm[8 * j + 4], prm[8 * j + 5]);
-    const f32x2 dr = add2(nal, bc(zr)), dv = add2(nbe, bc(zv));
-    const f32x2 dd = fma2(dv, dv, mul2(dr, dr));
-    f32x2 rc;
-    RNF_MAP2(rc, dd, rcp_approx);
-    const f32x2 f = mul2(omw, rc);
-    if (DERIV) *Sf = fma2(pk(prm[8 * j + 6], prm[8 * j + 7]), f, *Sf);
-    const f32x2 hr = fma2(f, dr, nal), hv = fma2(f, dv, nbe);
-    upk(hr, hr_[2 * j], hr_[2 * j + 1]);
-    upk(hv, hv_[2 * j], hv_[2 * j + 1]);
-    mn[j] = pk(fminf(fabsf(hv_[2 * j]), fabsf(hr_[2 * j])), fminf(fabsf(hv_[2 * j + 1]), fabsf(hr_[2 * j + 1])));
-  }
-  f32x2 at[NP];
-#pragma unroll
-  for (int j = 0; j < NP; ++j) at[j] = asin_unit2(mn[j]);
-#pragma unroll
-  for (int j = 0; j < NP; ++j) {
-    const f32x2 alt = fma2(at[j], bc(-1.0f), bc(1.5707963267948966f));
-    // Wrap to [0, 2 pi) with sign bits instead of two compare / select pairs.  phi = angle of (|hr|, |hv|) from the r axis;
-    // its complement c = pi/2 - phi is picked directly (asin or its complement), then
-    //   pi - theta_[0,pi] = pi/2 + copysign(c, hr)            (hr >= 0: pi - phi, hr < 0: phi)        =: v in [0, pi]
-    //   theta             = pi - copysign(v, hv)              (hv >= 0: pi - v,   hv < 0: pi + v)
-    // which is atan2(hv, hr) wrapped exactly (tests/test_fastmath.py).
-    float a_[2], b_[2], u_[2], v_[2];
-    upk(at[j], a_[0], a_[1]);
-    upk(alt, b_[0], b_[1]);
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-      const float c = fabsf(hv_[2 * j + i]) > fabsf(hr_[2 * j + i]) ? a_[i] : b_[i];
-      u_[i] = copysignf(c, hr_[2 * j + i]);
-    }
-    upk(add2(pk(u_[0], u_[1]), bc(1.5707963267948966f)), v_[0], v_[1]);
-    const f32x2 th = fma2(pk(copysignf(v_[0], hv_[2 * j]), copysignf(v_[1], hv_[2 * j + 1])), bc(-1.0f), bc(kPi));
-    Fs = fma2(pk(prm[8 * j + 6], prm[8 * j + 7]), th, Fs);
-  }
-}
 
 // The same evaluation without any quadrant logic.  On the unit circle the Mobius map is the disk automorphism
 // h = (z - w') / (1 - conj(w') z), so  theta_k = arg h = 2 arg(z - w') - t  with z = e^{it}; and because |w'| < 0.7 the direction of
@@ -300,11 +191,7 @@ __device__ __forceinline__ void probe_delta_pairs(float zr, float zv, const floa
     RNF_MAP2(rs, dd, rsqrt_approx);
     const f32x2 rs2 = mul2(rs, rs);
     m[j] = mul2(cr, rs);
-#if RNF_INV_MS_FROM_M
-    ms[j] = mul2(m[j], m[j]);                                           // one multiply less; one step longer dependency chain
-#else
-    ms[j] = mul2(mul2(cr, cr), rs2);
-#endif
+    ms[j] = mul2(m[j], m[j]);                                           // one multiply less than (cr^2) rs2; one step longer chain
     if (DERIV) Sf = fma2(pk(prm[8 * j + 6], prm[8 * j + 7]), mul2(pk(prm[8 * j + 4], prm[8 * j + 5]), rs2), Sf);
   }
 #pragma unroll

@@ -27,6 +27,56 @@ __device__ __forceinline__ void normalize3(float a[3]) {
   a[2] = a[2] / n;
 }
 
+// column p of R / write column p, by selects (a runtime index into a register array would put it in local memory)
+__device__ __forceinline__ float sel3(int p, float a, float b, float c) { return p == 0 ? a : (p == 1 ? b : c); }
+__device__ __forceinline__ void get_col(const float R[9], int p, float o[3]) {
+  o[0] = sel3(p, R[0], R[1], R[2]);
+  o[1] = sel3(p, R[3], R[4], R[5]);
+  o[2] = sel3(p, R[6], R[7], R[8]);
+}
+__device__ __forceinline__ void set_col(float R[9], int p, const float c[3]) {
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    R[3 * i + 0] = p == 0 ? c[i] : R[3 * i + 0];
+    R[3 * i + 1] = p == 1 ? c[i] : R[3 * i + 1];
+    R[3 * i + 2] = p == 2 ? c[i] : R[3 * i + 2];
+  }
+}
+
+// vee(R^T G): tangent (body frame) vector of a matrix gradient G at R, g_i = <G, R [e_i]x>
+__device__ __forceinline__ void tangent_of(const float R[9], const float G[9], float g[3]) {
+  float H[9];
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = 0; j < 3; ++j) H[3 * i + j] = R[i] * G[j] + R[3 + i] * G[3 + j] + R[6 + i] * G[6 + j];
+  g[0] = H[7] - H[5];
+  g[1] = H[2] - H[6];
+  g[2] = H[3] - H[1];
+}
+
+// G_R = R [g]x / 2
+__device__ __forceinline__ void gradient_from_tangent(const float R[9], const float g[3], float G[9]) {
+  const float h[9] = {0.0f, -g[2], g[1], g[2], 0.0f, -g[0], -g[1], g[0], 0.0f};
+#pragma unroll
+  for (int i = 0; i < 3; ++i)
+#pragma unroll
+    for (int j = 0; j < 3; ++j) G[3 * i + j] = 0.5f * (R[3 * i] * h[j] + R[3 * i + 1] * h[3 + j] + R[3 * i + 2] * h[6 + j]);
+}
+
+// E(q) omega = q (x) (0, omega): the 4x3 matrix of a body-frame perturbation of a unit quaternion (real first), and E(q)^T d
+__device__ __forceinline__ void E_mul(const float q[4], const float w[3], float o[4]) {
+  o[0] = -q[1] * w[0] - q[2] * w[1] - q[3] * w[2];
+  o[1] = q[0] * w[0] - q[3] * w[1] + q[2] * w[2];
+  o[2] = q[3] * w[0] + q[0] * w[1] - q[1] * w[2];
+  o[3] = -q[2] * w[0] + q[1] * w[1] + q[0] * w[2];
+}
+__device__ __forceinline__ void ET_mul(const float q[4], const float d[4], float o[3]) {
+  o[0] = -q[1] * d[0] + q[0] * d[1] + q[3] * d[2] - q[2] * d[3];
+  o[1] = -q[2] * d[0] - q[3] * d[1] + q[0] * d[2] + q[1] * d[3];
+  o[2] = -q[3] * d[0] + q[2] * d[1] - q[1] * d[2] + q[0] * d[3];
+}
+
 // R (row-major 3x3) -> quaternion (real first).  Only the winning candidate row of the public
 // algorithm is evaluated: argmax_i q_abs_i == argmax_i (q_abs_i^2) and that maximum is >= 1 because the
 // four radicands sum to 4, so the 0.1 floor of the public code can never be active on it.

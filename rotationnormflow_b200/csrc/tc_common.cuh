@@ -6,10 +6,6 @@
 #include "mobius_fast.cuh"
 #include "rnf_common.cuh"
 
-#ifndef RNF_TC_WAIT_HINT_NS
-#define RNF_TC_WAIT_HINT_NS 0
-#endif
-
 namespace rnf {
 
 // Packed global image of one Mobius conditioner (== the shared-memory pieces, one bulk copy each):
@@ -42,25 +38,7 @@ __device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
   asm volatile(
       "{\n"
       ".reg .pred p;\n"
-#if RNF_TC_WAIT_HINT_NS > 0
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n"
-#else
       "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n"
-#endif
-      "selp.u32 %0, 1, 0, p;\n"
-      "}\n"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"((uint32_t)RNF_TC_WAIT_HINT_NS)   // suspend-time hint: fewer polls stealing issue slots
-      : "memory");
-  return ok != 0;
-}
-// one non-blocking look at the barrier: true if the phase with this parity has completed
-__device__ __forceinline__ bool mbar_test(uint32_t bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n"
       "selp.u32 %0, 1, 0, p;\n"
       "}\n"
       : "=r"(ok)
@@ -157,17 +135,6 @@ __device__ __forceinline__ void tmem_ld_wait16(float v[16]) {
                :
                : "memory");
 }
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const float v[16]) {
-  const uint32_t* u = reinterpret_cast<const uint32_t*>(v);
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-      "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" ::"r"(taddr),
-      "r"(u[0]), "r"(u[1]), "r"(u[2]), "r"(u[3]), "r"(u[4]), "r"(u[5]), "r"(u[6]), "r"(u[7]), "r"(u[8]), "r"(u[9]),
-      "r"(u[10]), "r"(u[11]), "r"(u[12]), "r"(u[13]), "r"(u[14]), "r"(u[15])
-      : "memory");
-  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-}
-
 // stores without the wait (the caller issues one tmem_st_wait() for a batch)
 __device__ __forceinline__ void tmem_st16_nowait(uint32_t taddr, const uint32_t u[16]) {
   asm volatile(
@@ -195,20 +162,6 @@ __device__ __forceinline__ bool elect_one_sync() {
   return pred != 0;
 }
 
-// ReLU + error-compensated fp16 split of two activations in four instructions:
-//   hi = cvt.rz.relu.satfinite(t)          (round toward zero: the residual of a non-negative t is non-negative)
-//   lo = cvt.rn.relu.satfinite(t - hi)     (t < 0: hi = 0, residual = t < 0 -> 0)
-// so the ReLU of flow/condition.py:14-20 costs nothing, at one bit of the 22-bit split (hi 11 bits by truncation + lo 11).
-// Returns packed half2 words {x0 in the low half, x1 in the high half}.  Range (tests/test_weight_scales.py emulates it):
-// hi + lo = x to 22 bits only for x < 65536; above, hi saturates at 65504 and lo = x - 65504 keeps 11 bits (relative error up
-// to 2^-12.5), and from 131024 on lo saturates too: finite and clipped, never Inf.  The kernels compile the mask variants
-// (flow_t4.cu relu_split_pair, flow_row.cu store_a32) instead, which turn x >= 65536 into +Inf.
-__device__ __forceinline__ void relu_split2(float x0, float x1, uint32_t& hi, uint32_t& lo) {
-  asm("cvt.rz.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(x1), "f"(x0));
-  const float2 back = __half22float2(*reinterpret_cast<const __half2*>(&hi));
-  asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(x1 - back.y), "f"(x0 - back.x));
-}
-
 // UMMA shared-memory descriptor: K-major, SWIZZLE_128B, 8-row groups 1024 B apart (cute::UMMA::SmemDescriptor layout:
 // start>>4 [0,14) | LBO>>4 [16,30) | SBO>>4 [32,46) | version=1 [46,48) | layout_type=2 (SW128) [61,64)).
 constexpr uint32_t kDescHi = 64u | (1u << 14) | (2u << 29);          // bits [32,64): SBO = 1024 B, version 1, SW128
@@ -234,21 +187,6 @@ __device__ __forceinline__ void issue_split_gemm(uint32_t d_tmem, uint32_t a_hi,
   for (int k = 0; k < 4; ++k) umma_f16(d_tmem, a_hi + 2 * k, b_lo + 2 * k, kDescHi, idesc, 1);
 #pragma unroll
   for (int k = 0; k < 4; ++k) umma_f16(d_tmem, a_hi + 2 * k, b_hi + 2 * k, kDescHi, idesc, 1);
-}
-
-__device__ __forceinline__ float sel3(int p, float a, float b, float c) { return p == 0 ? a : (p == 1 ? b : c); }
-__device__ __forceinline__ void get_col(const float R[9], int p, float o[3]) {
-  o[0] = sel3(p, R[0], R[1], R[2]);
-  o[1] = sel3(p, R[3], R[4], R[5]);
-  o[2] = sel3(p, R[6], R[7], R[8]);
-}
-__device__ __forceinline__ void set_col(float R[9], int p, const float c[3]) {
-#pragma unroll
-  for (int i = 0; i < 3; ++i) {
-    R[3 * i + 0] = p == 0 ? c[i] : R[3 * i + 0];
-    R[3 * i + 1] = p == 1 ? c[i] : R[3 * i + 1];
-    R[3 * i + 2] = p == 2 ? c[i] : R[3 * i + 2];
-  }
 }
 
 }  // namespace rnf

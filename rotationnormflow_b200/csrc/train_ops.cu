@@ -147,27 +147,6 @@ __global__ void __launch_bounds__(128) mobius_mixture_fwd_kernel(const float* __
   theta_out[n] = theta;
 }
 
-// vee(R^T G): tangent (body frame) vector of a matrix gradient G at R, g_i = <G, R [e_i]x>
-__device__ __forceinline__ void tangent_of(const float R[9], const float* __restrict__ G, float g[3]) {
-  float H[9];
-#pragma unroll
-  for (int i = 0; i < 3; ++i)
-#pragma unroll
-    for (int j = 0; j < 3; ++j) H[3 * i + j] = R[i] * G[j] + R[3 + i] * G[3 + j] + R[6 + i] * G[6 + j];
-  g[0] = H[7] - H[5];
-  g[1] = H[2] - H[6];
-  g[2] = H[3] - H[1];
-}
-
-// G_R = R [g]x / 2
-__device__ __forceinline__ void gradient_from_tangent(const float R[9], const float g[3], float* __restrict__ G) {
-  const float h[9] = {0.0f, -g[2], g[1], g[2], 0.0f, -g[0], -g[1], g[0], 0.0f};
-#pragma unroll
-  for (int i = 0; i < 3; ++i)
-#pragma unroll
-    for (int j = 0; j < 3; ++j) G[3 * i + j] = 0.5f * (R[3 * i] * h[j] + R[3 * i + 1] * h[3 + j] + R[3 * i + 2] * h[6 + j]);
-}
-
 template <bool INV>
 __global__ void __launch_bounds__(128) mobius_mixture_bwd_kernel(const float* __restrict__ R, const float* __restrict__ out, int64_t N, int K,
                                                                  int p0, const float* __restrict__ theta_in, const float* __restrict__ R_out,
@@ -270,19 +249,6 @@ __global__ void __launch_bounds__(128) mobius_mixture_bwd_kernel(const float* __
     g[i] = m + c1[i] + c2[i];
   }
   gradient_from_tangent(Rm, g, G_R + n * 9);
-}
-
-// E(q) omega = q (x) (0, omega): the 4x3 matrix of a body-frame perturbation of a unit quaternion (real first)
-__device__ __forceinline__ void E_mul(const float q[4], const float w[3], float o[4]) {
-  o[0] = -q[1] * w[0] - q[2] * w[1] - q[3] * w[2];
-  o[1] = q[0] * w[0] - q[3] * w[1] + q[2] * w[2];
-  o[2] = q[3] * w[0] + q[0] * w[1] - q[1] * w[2];
-  o[3] = -q[2] * w[0] + q[1] * w[1] + q[0] * w[2];
-}
-__device__ __forceinline__ void ET_mul(const float q[4], const float d[4], float o[3]) {
-  o[0] = -q[1] * d[0] + q[0] * d[1] + q[3] * d[2] - q[2] * d[3];
-  o[1] = -q[2] * d[0] - q[3] * d[1] + q[0] * d[2] + q[1] * d[3];
-  o[2] = -q[3] * d[0] + q[2] * d[1] - q[1] * d[2] + q[0] * d[3];
 }
 
 __global__ void __launch_bounds__(128) quat_affine_fwd_kernel(const float* __restrict__ R, const float* __restrict__ W, int64_t N,

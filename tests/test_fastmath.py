@@ -1,4 +1,5 @@
-"""CPU checks of the constants baked into csrc/mobius_fast.cuh (fp32 emulation of the polynomial evaluation)."""
+"""CPU checks of the constants baked into csrc/mobius_fast.cuh and csrc/mobius_pair.cuh (fp32 emulation of the polynomial
+evaluation)."""
 import re
 import os
 
@@ -7,107 +8,51 @@ import numpy as np
 from conftest import ROOT
 
 
-def _coeffs():
-    """Coefficients c0..c8 (ascending powers of s = q^2) read back from the Horner evaluation in the header."""
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_fast.cuh")).read()
-    body = src[src.index("float atan2_wrapped_fast"):src.index("atan2_left_half_plane")]
-    first = re.search(r"float p = (-?[0-9.e-]+)f;", body).group(1)
-    rest = re.findall(r"p = fmaf\(p, s, (-?[0-9.e-]+)f\);", body)
-    return ([float(first)] + [float(v) for v in rest])[::-1]
-
-
-def test_both_atan_variants_share_the_polynomial():
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_fast.cuh")).read()
-    a = src[src.index("float atan2_wrapped_fast"):src.index("atan2_left_half_plane")]
-    b = src[src.index("float atan2_left_half_plane"):src.index("struct Plane")]
-    pat = r"fmaf\(p, s, (-?[0-9.e-]+)f\)"
-    assert re.findall(pat, a) == re.findall(pat, b) and len(re.findall(pat, a)) == 8
-
-
-def test_left_half_plane_identity():
-    """x < 0:  atan2(y, x) wrapped to [0, 2 pi)  ==  pi - atan(y / |x|)  (the forward-direction shortcut)."""
-    rng = np.random.default_rng(1)
-    y, x = rng.standard_normal(100000), -np.abs(rng.standard_normal(100000)) - 1e-3
-    ref = np.arctan2(y, x)
-    ref = np.where(ref >= 0, ref, ref + 2 * np.pi)
-    p = np.arctan(np.minimum(np.abs(y), -x) / np.maximum(np.abs(y), -x))
-    p = np.where(np.abs(y) > -x, np.pi / 2 - p, p)
-    got = np.where(y < 0, np.pi + p, np.pi - p)
-    assert np.abs(got - ref).max() < 1e-12
-
-
 def _fma32(a, b, c):
     return (a.astype(np.float64) * b.astype(np.float64) + np.float64(c)).astype(np.float32)
 
 
-def test_atan_polynomial_accuracy():
-    co = _coeffs()
-    assert len(co) == 9
-    q = np.linspace(0, 1, 1_000_001).astype(np.float32)
-    s = (q.astype(np.float64) * q).astype(np.float32)
-    p = np.full_like(s, np.float32(co[-1]))
-    for c in co[-2::-1]:
-        p = _fma32(p, s, np.float32(c))
-    p = (p.astype(np.float64) * s).astype(np.float32)
-    res = (p.astype(np.float64) * q + q).astype(np.float32)
-    err = np.abs(res.astype(np.float64) - np.arctan(q.astype(np.float64)))
-    assert err.max() < 1.0e-7                                   # 1.3 ulp at pi/4
+def _function_body(header, name):
+    """Source of the device function whose definition starts with `name` in csrc/<header>, up to its closing brace."""
+    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", header)).read()
+    start = src.index(name)
+    return src[start:src.index("\n}\n", start)]
 
 
-def test_octant_reduction_covers_the_circle():
-    """The min/max + three selects of atan2_wrapped_fast reproduce atan2 wrapped to [0, 2 pi) (float64 emulation)."""
-    rng = np.random.default_rng(0)
-    y, x = rng.standard_normal(100000), rng.standard_normal(100000)
-    ay, ax = np.abs(y), np.abs(x)
-    p = np.arctan(np.minimum(ay, ax) / np.maximum(ay, ax))
-    p = np.where(ay > ax, np.pi / 2 - p, p)
-    p = np.where(x < 0, np.pi - p, p)
-    p = np.where(y < 0, 2 * np.pi - p, p)
-    ref = np.arctan2(y, x)
-    ref = np.where(ref >= 0, ref, ref + 2 * np.pi)
-    assert np.abs(p - ref).max() < 1e-12
-
-
-def test_softplus_series_branch():
+def test_softplus_series_branch_of_mixture_pairs():
     """e (1 - e/2) against log1p(e) below the 2^-7 switch-over: relative error <= e^2/3, absolute <= 2e-7."""
     e = np.linspace(0, 0.0078125, 1001)[1:]
     series = e * (1 - e / 2)
     assert (np.abs(series - np.log1p(e)) / np.log1p(e)).max() < 2.1e-5
     assert np.abs(series - np.log1p(e)).max() < 2e-7
-    # constants in the header are the series coefficients divided by ln 2
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_fast.cuh")).read()
-    m = re.search(r"small = e \* fmaf\(e, (-?[0-9.]+)f, ([0-9.]+)f\)", src)
+    # constants in mixture_pairs are the series coefficients divided by ln 2
+    body = _function_body("mobius_pair.cuh", "void mixture_pairs")
+    m = re.search(r"small\[j\] = mul2\(e\[j\], fma2\(e\[j\], bc\((-?[0-9.]+)f\), bc\(([0-9.]+)f\)\)\)", body)
     assert abs(float(m.group(2)) - 1 / np.log(2)) < 1e-12 and abs(float(m.group(1)) + 0.5 / np.log(2)) < 1e-12
 
 
-def test_packed_asin_polynomial_accuracy():
-    """mobius_pair.cuh takes the angle of the unit vector h from its nearer axis as asin(min(|h.r|, |h.v|)) (no division):
-    float32 Horner emulation of the polynomial read back from the header, against asin on [0, 1/sqrt 2]."""
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_pair.cuh")).read()
-    body = src[src.index("f32x2 asin_unit2"):src.index("// atan on the half-angle range")]
-    # the shipped degree-6 polynomial (#else branch) and the degree-5 experiment (RNF_ASIN_DEG == 5), highest power first
-    deg5, deg6 = body[body.index("#if RNF_ASIN_DEG == 5"):body.index("#else")], body[body.index("#else"):body.index("#endif")]
-    assert "#define RNF_ASIN_DEG 6" in src
-    for part, n, bound in ((deg6, 7, 6e-8), (deg5, 6, 1e-7)):
-        co = [float(v) for v in re.findall(r"bc\((-?[0-9.e-]+)f\)", part)]
-        assert len(co) == n
-        m = np.linspace(0, 0.70711, 1_000_001).astype(np.float32)
-        s = (m.astype(np.float64) * m).astype(np.float32)
-        p = np.full_like(s, np.float32(co[0]))
-        for c in co[1:]:
-            p = _fma32(p, s, np.float32(c))
-        ps = (p.astype(np.float64) * s).astype(np.float32)
-        res = (ps.astype(np.float64) * m + m).astype(np.float32)
-        assert np.abs(res.astype(np.float64) - np.arcsin(m.astype(np.float64))).max() < bound
+def test_packed_asin_degree6_accuracy():
+    """mobius_pair.cuh takes the mixture angles as asin of a sine (no division): float32 Horner emulation of the degree-6
+    polynomial read back from the header, against asin on [0, 1/sqrt 2]."""
+    body = _function_body("mobius_pair.cuh", "f32x2 asin_unit2_s")
+    co = [float(v) for v in re.findall(r"bc\((-?[0-9.e-]+)f\)", body)]          # highest power first
+    assert len(co) == 7
+    m = np.linspace(0, 0.70711, 1_000_001).astype(np.float32)
+    s = (m.astype(np.float64) * m).astype(np.float32)
+    p = np.full_like(s, np.float32(co[0]))
+    for c in co[1:]:
+        p = _fma32(p, s, np.float32(c))
+    ps = (p.astype(np.float64) * s).astype(np.float32)
+    res = (ps.astype(np.float64) * m + m).astype(np.float32)
+    assert np.abs(res.astype(np.float64) - np.arcsin(m.astype(np.float64))).max() < 6e-8
     # unit vector: atan(min / max) == asin(min)
     t = np.linspace(0, np.pi / 4, 1001)
     assert np.abs(np.arctan(np.sin(t) / np.cos(t)) - np.arcsin(np.sin(t))).max() < 1e-15
 
 
-def test_sincos_2pi_accuracy():
+def test_sincos_2pi_polynomial_accuracy():
     """Float32 emulation of sincos_2pi (mobius_fast.cuh) over [0, 2 pi] with the constants read back from the header."""
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_fast.cuh")).read()
-    body = src[src.index("void sincos_2pi"):src.index("// Mixture weight of a component")]
+    body = _function_body("mobius_fast.cuh", "void sincos_2pi")
     num = r"(-?[0-9.]+(?:e-?[0-9]+)?)f"
     two_over_pi, magic = map(float, re.search(r"fmaf\(t, %s, %s\)" % (num, num), body).groups())
     hi = float(re.search(r"fmaf\(kf, %s, t\)" % num, body).group(1))
@@ -136,38 +81,11 @@ def test_sincos_2pi_accuracy():
     assert np.abs(C - np.cos(t.astype(np.float64))).max() < 1.2e-7
 
 
-def test_sign_bit_quadrant_logic_of_the_probe():
-    """probe_pairs wraps the angle with two copysigns: theta = pi - copysign(pi/2 + copysign(c, hr), hv), c = the complement of
-    the first-quadrant angle.  Float64 emulation against atan2 wrapped to [0, 2 pi) over the whole circle."""
-    t = np.random.default_rng(0).uniform(0, 2 * np.pi, 200000)
-    hr, hv = np.cos(t), np.sin(t)
-    ay, ax = np.abs(hv), np.abs(hr)
-    at = np.arcsin(np.minimum(ay, ax))
-    c = np.where(ay > ax, at, np.pi / 2 - at)
-    v = np.pi / 2 + np.copysign(c, hr)
-    th = np.pi - np.copysign(v, hv)
-    ref = np.arctan2(hv, hr)
-    ref = np.where(ref >= 0, ref, ref + 2 * np.pi)
-    assert np.abs(th - ref).max() < 1e-14
-
-
-def test_half_angle_atan_polynomial_and_identity():
+def test_half_angle_identity_of_the_forward_angle():
     """mixture_pairs (forward) takes theta = pi + 2 atan(q), q = -(tan of half the angle of h from the negative r axis) =
-    -h_v / (1 - h_r) (= b' / Dn in the kernel's variables), |q| <= tan(asin 0.7): float32 Horner emulation of atan_half2 read
-    back from the header, and the half-angle identity against atan2 wrapped to [0, 2 pi) over the left half plane."""
-    src = open(os.path.join(ROOT, "rotationnormflow_b200", "csrc", "mobius_pair.cuh")).read()
-    body = src[src.index("f32x2 atan_half2"):src.index("// NP pairs of mixture components")]
-    co = [float(v) for v in re.findall(r"bc\((-?[0-9.e-]+)f\)", body)]          # highest power first
-    assert len(co) == 8
+    -h_v / (1 - h_r) (= b' / Dn in the kernel's variables), |q| <= tan(asin 0.7), and evaluates atan(q) as asin(b' / |D|):
+    the half-angle identity against atan2 wrapped to [0, 2 pi) over the left half plane."""
     qmax = np.tan(np.arcsin(0.7))
-    q = np.linspace(-qmax, qmax, 2_000_001).astype(np.float32)
-    s = (q.astype(np.float64) * q).astype(np.float32)
-    p = np.full_like(s, np.float32(co[0]))
-    for c in co[1:]:
-        p = _fma32(p, s, np.float32(c))
-    ps = (p.astype(np.float64) * s).astype(np.float32)
-    res = (ps.astype(np.float64) * q + q).astype(np.float32)
-    assert np.abs(res.astype(np.float64) - np.arctan(q.astype(np.float64))).max() < 7e-8
     psi = np.linspace(-2 * np.arcsin(0.7), 2 * np.arcsin(0.7), 100001)
     hr, hv = -np.cos(psi), np.sin(psi)                                   # unit vector within +-2 asin(0.7) of the angle pi
     ref = np.arctan2(hv, hr)

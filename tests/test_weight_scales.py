@@ -4,7 +4,7 @@ Every other test runs random-initialisation weights: hidden activations of 0.01 
 the 0.7 disk.  Trained checkpoints leave that regime, and several fast paths are only right inside a numeric range:
   - the tensor-core GEMMs (modes tc, tc_row) split each activation into fp16 hi / lo planes (flow_t4.cu relu_split_pair,
     flow_row.cu store_a32): exact to 22 bits for 0.125 <= x < 65536, 2^-25 absolute below, +Inf from 65536 on;
-  - the fast-path mixture weights (mobius_fast.cuh softplus_log2, mobius_pair.cuh mixture_pairs) use ex2.approx.ftz and switch
+  - the fast-path mixture weights (mobius_pair.cuh mixture_pairs) use ex2.approx.ftz and switch
     branches at 2^t = 2^-7 (a = -4.852) and t = 28.85 (a = 20); a row whose logits are all below -87.3 has no weight left;
   - the inverse's Newton + replay root search was justified for F' in [0.17, 5.7].
 The stress models are transforms of golden weights whose effect is known exactly:
@@ -286,7 +286,8 @@ def split_emulation(x, variant):
     'mask':     the kernels' variant: m = x with its low 13 mantissa bits cleared, hi = cvt.rn(m) (no satfinite),
                 lo = cvt.rn.satfinite(x - m)
     'mask_sat': the same with hi = cvt.rz.satfinite(x) (the variant before overflow was made loud)
-    'convert':  hi = cvt.rz.satfinite(x), lo = cvt.rn.satfinite(x - float(hi))   (tc_common.cuh relu_split2)"""
+    'convert':  hi = cvt.rz.satfinite(x), lo = cvt.rn.satfinite(x - float(hi))   (the convert-back variant, removed from
+                tc_common.cuh; its code is in commit d73682a)"""
     x = np.asarray(x, dtype=np.float32)
     sat = lambda v: np.clip(v, -FP16_MAX, FP16_MAX)
     m = (x.view(np.uint32) & np.uint32(0xFFFFE000)).view(np.float32)

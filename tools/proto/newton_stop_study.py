@@ -1,7 +1,9 @@
-"""Offline check of the inverse kernel's Newton stopping rule (csrc/flow_row.cu, RNF_INV_PREDICT) on HARD synthetic mixtures:
-K = 64 components with |w'| up to 0.7 and peaky weights, evaluated in float32 like the kernel; the root it stops at is compared with
-the float64 root.  What has to hold: |t_stop - t_true| * F' stays far inside the 2e-6 band in which the replay of the reference's
-halvings evaluates explicitly instead of trusting sign(x0 - t*)."""
+"""Offline check of the inverse kernel's Newton stopping rule (csrc/flow_row.cu: stop on the predicted error of the next iterate)
+on HARD synthetic mixtures: K = 64 components with |w'| up to 0.7 and peaky weights, evaluated in float32 like the kernel; the root
+it stops at is compared with the float64 root.  What has to hold: |t_stop - t_true| * F' stays far inside the 2e-6 band in which
+the replay of the reference's halvings evaluates explicitly instead of trusting sign(x0 - t*).
+The "avg" rows start the iteration at the closed-form inverse of the Mobius map of the weighted mean centre.  The kernel starts
+at pi: that start was measured on the device (DESIGN.md section 4.1) and removed; its code is in commit d73682a."""
 import math
 import numpy as np
 
